@@ -2,6 +2,7 @@
 """bench.py — headline benchmark of the SpMM path (BASELINE.json metric) on N B200s of one node.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+                    [--dump-outputs DIR]
 
 A *step* is one pass of the hot path over the workload: SpMM forward C = A·B plus the A^T·dY
 backward (BASELINE.json configs[1]: "forward + A^T·dY backward").  Default workload = configs[1]
@@ -17,6 +18,10 @@ buffers, host<->device copies inside the timed region (max over ranks).  `roofli
 dominant kernel (spmm_merge_kernel, forward) under the gather model M2 of SURVEY.md §8d, with the
 ncu-measured DRAM and L2 bytes beside it; `cpu_baseline` is the oracle's OneFlow-style CPU loop on
 this box's host cores; `verified` says that sampled rows of the timed outputs matched the oracle.
+
+`--dump-outputs DIR` writes what the last timed step returned as DIR/<name>.npy, so that two builds
+can be compared output for output on identical (seeded) inputs.  Once build() has run (it compiles
+the CUDA library and the oracle), the benchmark writes nothing into the tree it runs from.
 """
 from __future__ import annotations
 
@@ -33,6 +38,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # no __pycache__ in the tree, which may be read-only
 
 METRIC = "SpMM GFLOP/s (2*nnz*N/t), fwd + A^T*dY"
 UNIT = "GFLOP/s"
@@ -42,6 +48,8 @@ L2_NOTE = ("inputs larger than L2 (CSR stream ~1 GB/step >> 126 MB); no flush be
 # L2 -> SM peak used for the second roofline entry: 184 L2 slices x 2 sectors/clk x 32 B x 1.964 GHz
 # (ncu: lts__lts2xbar_cycles_active peak_sustained = 2 per slice, 184 slices active, profiles/r2_ncu_*.md)
 L2_PEAK_GBS = 184 * 2 * 32 * 1.964
+# --dump-outputs: all files together stay under 64 MB; the budget is split evenly between the outputs
+DUMP_BYTES = 60 << 20
 
 WORKLOADS = {
     "cfg2_reddit_n128_fp32": dict(kind="reddit", scale_div=1, n=128, dtype="fp32"),
@@ -164,9 +172,11 @@ class CpuArm:
     def step(self, threads=None):
         th = threads or self.cores
         t0 = time.perf_counter()
-        self.O.spmm_f32(self.crow, self.col, self.val, self.B, self.cols, threads=th, native=self.native)
-        self.O.spmm_f32(self.t[0], self.t[1], self.t[2], self.dY, self.rows, threads=th, native=self.native)
-        return time.perf_counter() - t0
+        C = self.O.spmm_f32(self.crow, self.col, self.val, self.B, self.cols, threads=th, native=self.native)
+        dB = self.O.spmm_f32(self.t[0], self.t[1], self.t[2], self.dY, self.rows, threads=th, native=self.native)
+        secs = time.perf_counter() - t0
+        self.last = (C, dB)
+        return secs
 
     def single_thread_sample(self, frac=16):
         """The reference's default CPU_THREADING_RUNTIME is SEQ (CMakeLists.txt:54): the plain
@@ -203,27 +213,24 @@ def run_reference(args):
     B = ofs.graphs.dense_operand(A.cols, n, 11, dev)
     dY = ofs.graphs.upstream_grad(A.rows, n, 12, dev)
     arm = CpuArm(A, B, dY, n)
-    # bound the whole run to a few minutes whatever K and W the driver passes
-    budget, times = 150.0, []
-    t_first = arm.step()
-    warm = max(0, min(args.warmup, int(budget * 0.2 / max(t_first, 1e-3))) - 1)
-    for _ in range(warm):
+    for _ in range(args.warmup):
         arm.step()
-    steps = max(1, min(args.steps, int(budget * 0.8 / max(t_first, 1e-3))))
-    for _ in range(steps):
-        times.append(arm.step())
+    times = [arm.step() for _ in range(args.steps)]
+    if args.dump_outputs:
+        C, dB = (torch.from_numpy(a) for a in arm.last)
+        dump_outputs(args.dump_outputs, [("C", C, None, A.rows), ("dB", dB, None, A.cols)])
     secs = statistics.mean(times)
     flops = 2.0 * 2.0 * A.nnz * n
     v = flops / secs / 1e9
-    base = arm.describe(v, secs, steps)
+    base = arm.describe(v, secs, len(times))
     base["single_thread_value"] = arm.single_thread_sample()
     print(json.dumps({
-        "impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
+        "impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": len(times),
         "warmup": args.warmup, "ms_per_step": secs * 1e3, "higher_is_better": True, "scaling": "strong",
         "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": _config(args.workload, A, n),
-        "impl_detail": {"parallelism": f"{arm.cores} host threads", "timed_passes": steps,
-                        "note": "every timed step is the full workload; K is clipped so the run stays within minutes"},
+        "impl_detail": {"parallelism": f"{arm.cores} host threads", "timed_passes": len(times),
+                        "note": "every timed step is the full workload"},
         "cpu_baseline": base,
         "e2e": {"value": v, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }))
@@ -294,6 +301,50 @@ def verify_sample(A, B_full, dY_full, C_blk, r0, r1, dB_shard, shard_ids, dtype,
     res["dB_ok"] = bool((np.abs(got - want) <= tol + 1e-30).all())
     res["ok"] = res["C_ok"] and res["dB_ok"]
     return res
+
+
+def dump_outputs(path, outputs, rank=0, world=1):
+    """--dump-outputs: each output as <path>/<name>.npy (float64 stays float64, everything else is
+    written as float32).  ``outputs`` = [(name, tensor, where, rows)]: ``tensor`` holds rows of an
+    output of ``rows`` rows in all; ``where`` says which — None (all of them, the same on every rank),
+    an int (the global id of its first row, the rest follow contiguously) or a tensor of global row
+    ids.  An output larger than its share of DUMP_BYTES is a seeded sample of its rows in ascending
+    order, the same sample for every build and rank count.  Every rank calls this; rank 0 writes."""
+    import math
+
+    import numpy as np
+    import torch
+    share = DUMP_BYTES // len(outputs)
+    for name, t, where, rows in outputs:
+        dt = torch.float64 if t.dtype == torch.float64 else torch.float32
+        row_bytes = math.prod(t.shape[1:]) * (8 if dt == torch.float64 else 4)
+        sample = None
+        if t.dim() > 0 and rows * row_bytes > share:
+            g = torch.Generator().manual_seed(0)
+            sample = torch.unique(torch.randint(0, rows, (max(1, share // row_bytes),), generator=g))
+        if where is None:
+            part = t if sample is None else t[sample.to(t.device)]
+            part = part.detach().to(dt).cpu()
+        else:
+            if isinstance(where, int):
+                ids = torch.arange(where, where + t.shape[0]) if sample is None else \
+                    sample[(sample >= where) & (sample < where + t.shape[0])]
+                pos = ids - where
+            else:
+                ids_all = where.cpu().long()
+                pos = torch.arange(ids_all.numel()) if sample is None else torch.nonzero(torch.isin(ids_all, sample)).flatten()
+                ids = ids_all[pos]
+            pieces = [(ids, t[pos.to(t.device)].detach().to(dt).cpu())]
+            if world > 1:
+                import torch.distributed as dist
+                gathered = [None] * world
+                dist.all_gather_object(gathered, pieces[0])
+                pieces = gathered
+            ids = torch.cat([p[0] for p in pieces])
+            part = torch.cat([p[1] for p in pieces])[torch.argsort(ids)]
+        if rank == 0:
+            os.makedirs(path, exist_ok=True)
+            np.save(os.path.join(path, name + ".npy"), part.numpy())
 
 
 # ------------------------------------------------------------------------------------------------
@@ -580,7 +631,12 @@ def main():
                     help="N>1, pull: >0 runs the dB combine beside the last forward pass with that many CTAs")
     ap.add_argument("--layout", default="auto", choices=["auto", "block", "cyclic"],
                     help="N>1, pull: ownership of B / dB rows (auto = block-cyclic when contiguous blocks would skew the egress)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (a seeded row sample of outputs "
+                         "that would exceed 64 MB in all); bench_outputs/ in the tree is ignored by git")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(3, args.warmup)
     if args.impl == "reference":
         return run_reference(args)
@@ -696,6 +752,9 @@ def main():
     barrier()
     total_ms = ev[0].elapsed_time(ev[1])
     launches = ofs.launch_count() - launches0
+    if args.dump_outputs:
+        c_out, db_out = outputs()
+        dump_outputs(args.dump_outputs, [("C", c_out, r0, A.rows), ("dB", db_out, shard_ids, A.cols)], rank, world)
     # ---- the timed outputs are what gets verified (sampled rows vs the fp64 oracle)
     verified = None
     if not args.no_verify:

@@ -77,6 +77,11 @@ def main(args):
     total_ms = a.elapsed_time(b)
     launches = ofs.launch_count() - l0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:   # what train_step hands its caller: the loss and the gradients
+        g = model.grads
+        bench.dump_outputs(args.dump_outputs, [("loss", loss, None, 1), ("grad_W1", g["W1"], None, in_dim),
+                                               ("grad_W2", g["W2"], None, hidden),
+                                               ("grad_val", g["val"], int(A.crow[model.sh.r0]), A.nnz)], rank, world)
 
     # ---- the six sparse products alone, on layer-1 operands
     sh, m = model.sh, model.m

@@ -12,6 +12,7 @@ from __future__ import annotations
 import ctypes
 import os
 import subprocess
+import tempfile
 from typing import Optional, Tuple
 
 import numpy as np
@@ -25,25 +26,12 @@ _c_int = ctypes.c_int
 _vp = ctypes.c_void_p
 
 
-def _cpu_tag() -> str:
-    """Short hash of this host's CPU model + ISA flags: a -march=native build is only valid on the
-    machine type that built it (the repo snapshot, built files included, travels to other boxes)."""
-    import hashlib
-    try:
-        with open("/proc/cpuinfo") as f:
-            lines = [ln for ln in f if ln.startswith(("model name", "flags"))][:2]
-    except OSError:
-        lines = []
-    return hashlib.sha1("".join(lines).encode()).hexdigest()[:10]
-
-
-def build(native: bool = False, force: bool = False) -> str:
-    """Compile the oracle with gcc if the shared object is missing or older than its source."""
-    name = f"libofspmm_oracle_native_{_cpu_tag()}.so" if native else "libofspmm_oracle.so"
-    so = os.path.join(_OUT, name)
+def build(native: bool = False, force: bool = False, out: str = _OUT) -> str:
+    """Compile the oracle with gcc into ``out`` if the shared object is missing or older than its source."""
+    so = os.path.join(out, "libofspmm_oracle_native.so" if native else "libofspmm_oracle.so")
     if not force and os.path.exists(so) and os.path.getmtime(so) >= os.path.getmtime(_SRC):
         return so
-    os.makedirs(_OUT, exist_ok=True)
+    os.makedirs(out, exist_ok=True)
     march = "-march=native" if native else "-march=x86-64-v3"
     cmd = ["gcc", "-O3", "-fPIC", "-shared", "-pthread", "-std=c11", march, "-o", so, _SRC, "-lm"]
     subprocess.run(cmd, check=True, capture_output=True)
@@ -55,7 +43,15 @@ _LIBS = {}
 
 def lib(native: bool = False) -> ctypes.CDLL:
     if native not in _LIBS:
-        L = ctypes.CDLL(build(native=native))
+        if native:
+            # A -march=native build is only valid on the host that compiles it, and bench.py (the CPU
+            # baseline) must not write into the tree, which may be read-only.  So each process compiles
+            # it (about a second of gcc) in a temporary directory that is gone as soon as the library is
+            # loaded: nothing is left behind, however the process ends.
+            with tempfile.TemporaryDirectory(prefix="ofspmm_oracle_") as d:
+                L = ctypes.CDLL(build(native=True, out=d))
+        else:
+            L = ctypes.CDLL(build())
         for fn in ("oracle_spmm_f32", "oracle_spmm_f64", "oracle_spmm_absmax", "oracle_spmm_t_f32",
                    "oracle_spmm_t_f64", "oracle_sddmm_f32"):
             getattr(L, fn).argtypes = [_c_i64, _c_i64, _c_i64, _vp, _vp, _vp, _vp, _vp, _c_int]
