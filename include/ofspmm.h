@@ -66,14 +66,17 @@ enum {
   OFSPMM_ERR_UNSUPPORTED_DTYPE = 2, /* dtype combination without a kernel                      */
   OFSPMM_ERR_WORKSPACE = 3,         /* workspace null / misaligned / smaller than the query    */
   OFSPMM_ERR_CUDA = 4,              /* a CUDA runtime call or launch failed (cudaGetLastError) */
-  OFSPMM_ERR_TOO_LARGE = 5,         /* rows or nnz >= 2^31 (row offsets are kept in 32 bits)   */
+  OFSPMM_ERR_TOO_LARGE = 5,         /* rows >= 2^31-1, or nnz >= 2^31-1 with int32 indices      */
   OFSPMM_ERR_NO_DEVICE = 6          /* no sm_100 device current on this thread                 */
 };
 
 /* A (rows × cols) in CSR.  crow has rows+1 entries, col / val have nnz entries.
  * idx_dtype ∈ {INT32, INT64} applies to both crow and col (INDEX_DATA_TYPE_SEQ,
  * oneflow/core/common/data_type_seq.h:50-52).  val_dtype ∈ {FLOAT, BFLOAT16}; BFLOAT16 values are
- * only accepted together with a BFLOAT16 dense operand.  `val` may be NULL for ofspmm_sddmm. */
+ * only accepted together with a BFLOAT16 dense operand.  `val` may be NULL for ofspmm_sddmm.
+ * Ranges: rows < 2^31-1 for both index dtypes; nnz < 2^31-1 with INT32 indices, while INT64
+ * indices take any nnz whose (rows + nnz) / 256 merge-path tasks stay below 2^30
+ * (nnz below about 2.7e11). */
 typedef struct ofspmm_csr {
   int64_t rows;
   int64_t cols;

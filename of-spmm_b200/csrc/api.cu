@@ -36,7 +36,7 @@ FwdWorkspace fwd_workspace_layout(int64_t rows, int64_t nnz, int64_t n, int dens
   const size_t P = static_cast<size_t>(num_tasks(rows, nnz, items));
   L.counter_off = 0;  // task counter of the dynamic order (zeroed by a memset node before the launch)
   L.part_off = 256;
-  L.carry_off = L.part_off + align_up((P + 1) * sizeof(int2), 256);
+  L.carry_off = L.part_off + align_up((P + 1) * part_entry_bytes(nnz), 256);
   const size_t rowbuf = align_up(P * static_cast<size_t>(n) * sizeof(float), 256);
   L.head_off = L.carry_off + rowbuf;
   L.total = L.head_off + (dense_dtype == OFSPMM_DTYPE_FLOAT ? 0 : rowbuf);
@@ -51,12 +51,20 @@ bool idx_ok(int d) { return d == OFSPMM_DTYPE_INT32 || d == OFSPMM_DTYPE_INT64; 
 size_t dense_size(int d) { return d == OFSPMM_DTYPE_FLOAT ? 4 : 2; }
 size_t idx_size(int d) { return d == OFSPMM_DTYPE_INT64 ? 8 : 4; }
 
+// Sizes no kernel can address: rows that do not fit int, non-zeros that int32 row offsets cannot
+// count, or more 256-item tasks than the task index allows (kMaxTasks).  Wide int64 matrices are fine.
+bool too_large(int idx_dtype, int64_t rows, int64_t nnz) {
+  if (rows >= (int64_t{1} << 31) - 1) return true;
+  if (idx_dtype == OFSPMM_DTYPE_INT32 && wide_nnz(nnz)) return true;
+  return num_tasks(rows, nnz, kTaskItems) >= kMaxTasks;
+}
+
 int check_csr(const ofspmm_csr* A, bool need_val) {
   if (A == nullptr) return OFSPMM_ERR_INVALID_ARG;
   if (A->rows < 0 || A->cols < 0 || A->nnz < 0) return OFSPMM_ERR_INVALID_ARG;
   if (!idx_ok(A->idx_dtype)) return OFSPMM_ERR_UNSUPPORTED_DTYPE;
   if (A->val_dtype != OFSPMM_DTYPE_FLOAT && A->val_dtype != OFSPMM_DTYPE_BFLOAT16) return OFSPMM_ERR_UNSUPPORTED_DTYPE;
-  if (A->rows >= (int64_t{1} << 31) - 1 || A->nnz >= (int64_t{1} << 31) - 1) return OFSPMM_ERR_TOO_LARGE;
+  if (too_large(A->idx_dtype, A->rows, A->nnz)) return OFSPMM_ERR_TOO_LARGE;
   if (A->crow == nullptr) return OFSPMM_ERR_INVALID_ARG;
   if (A->nnz > 0 && (A->col == nullptr || (need_val && A->val == nullptr))) return OFSPMM_ERR_INVALID_ARG;
   return OFSPMM_OK;
@@ -82,7 +90,7 @@ size_t fwd_ws_auto(int64_t rows, int64_t nnz, int64_t n, int dense_dtype) {
 }
 
 size_t plan_bytes_for(int64_t rows, int64_t nnz, int items) {
-  return align_up((static_cast<size_t>(num_tasks(rows, nnz, items)) + 1) * sizeof(int2), 256);
+  return align_up((static_cast<size_t>(num_tasks(rows, nnz, items)) + 1) * part_entry_bytes(nnz), 256);
 }
 
 // Options of one call -> launch description.  `opts` may be NULL (all defaults).
@@ -94,6 +102,7 @@ FwdLaunch make_launch(const ofspmm_opts* opts, int64_t rows, int64_t nnz, int64_
   const uint32_t fl = opts ? opts->flags : 0u;
   // task order: dynamic (drawn from a counter) unless the caller pins the static interleave
   L.dynamic = OFSPMM_DEFAULT_DYNAMIC_ORDER ? (fl & OFSPMM_ORDER_STATIC) == 0 : (fl & OFSPMM_ORDER_DYNAMIC) != 0;
+  L.wide = wide_nnz(nnz);
   L.flags = fl & (OFSPMM_FWD_ACCUMULATE | OFSPMM_FWD_BIAS | OFSPMM_FWD_RELU | OFSPMM_FWD_ACC32_IN | OFSPMM_FWD_ACC32_OUT);
   L.bias = opts ? opts->bias : nullptr;
   L.acc32 = opts ? static_cast<float*>(opts->acc32) : nullptr;
@@ -180,7 +189,7 @@ int ofspmm_plan_build(const void* crow, int idx_dtype, int64_t rows, int64_t nnz
                       int variant, void* plan, size_t plan_bytes, ofspmm_stream_t stream) {
   if (crow == nullptr || plan == nullptr || rows < 0 || nnz < 0) return OFSPMM_ERR_INVALID_ARG;
   if (!idx_ok(idx_dtype)) return OFSPMM_ERR_UNSUPPORTED_DTYPE;
-  if (rows >= (int64_t{1} << 31) - 1 || nnz >= (int64_t{1} << 31) - 1) return OFSPMM_ERR_TOO_LARGE;
+  if (too_large(idx_dtype, rows, nnz)) return OFSPMM_ERR_TOO_LARGE;
   const int items = resolve_variant(variant, rows, nnz, n, dense_dtype).items;
   if (plan_bytes < plan_bytes_for(rows, nnz, items) || (reinterpret_cast<uintptr_t>(plan) & 15)) return OFSPMM_ERR_WORKSPACE;
   return launch_task_partition(crow, idx_dtype, rows, nnz, num_tasks(rows, nnz, items), items, plan,
@@ -272,7 +281,7 @@ int ofspmm_bwd_b(const ofspmm_csr* A, const ofspmm_csr* At, const void* dY, void
   if (int rc = check_ws(workspace, workspace_bytes, need)) return rc;
   unsigned char* w = static_cast<unsigned char*>(workspace);
   const int64_t P = num_tasks(A->rows, A->nnz);
-  const size_t part_bytes = align_up((static_cast<size_t>(P) + 1) * sizeof(int2), 256);
+  const size_t part_bytes = plan_bytes_for(A->rows, A->nnz, kTaskItems);
   if (int rc = launch_task_partition(A->crow, A->idx_dtype, A->rows, A->nnz, P, kTaskItems, w, stream)) return rc;
   if (dense_dtype == OFSPMM_DTYPE_FLOAT)
     return launch_bwd_atomic(A, dY, static_cast<float*>(dB), nullptr, n, dense_dtype, w, P, stream);
@@ -610,7 +619,7 @@ const char* ofspmm_strerror(int status) {
     case OFSPMM_ERR_UNSUPPORTED_DTYPE: return "unsupported dtype combination";
     case OFSPMM_ERR_WORKSPACE: return "workspace missing, misaligned or smaller than *_workspace_bytes()";
     case OFSPMM_ERR_CUDA: return "CUDA runtime call or kernel launch failed";
-    case OFSPMM_ERR_TOO_LARGE: return "rows or nnz >= 2^31-1";
+    case OFSPMM_ERR_TOO_LARGE: return "rows >= 2^31-1, or nnz >= 2^31-1 with int32 indices";
     case OFSPMM_ERR_NO_DEVICE: return "no sm_100 (B200) device current on this thread";
     default: return "unknown status";
   }

@@ -6,11 +6,11 @@ namespace ofspmm {
 
 namespace {
 
-template <typename DT, typename ValT, typename IdxT, int VEC, int LPR, int CH>
+template <typename DT, typename ValT, typename IdxT, typename PartT, int VEC, int LPR, int CH>
 int launch_one(const BwdAtomicParams& p, int panels, cudaStream_t stream) {
   constexpr int ITEMS = kTaskItems;
   constexpr int WARPS = kWarpsPerCta;
-  auto kern = bwd_atomic_kernel<DT, ValT, IdxT, VEC, LPR, CH, ITEMS, WARPS>;
+  auto kern = bwd_atomic_kernel<DT, ValT, IdxT, VEC, LPR, CH, ITEMS, WARPS, PartT>;
   const size_t smem = sizeof(TaskStage<IdxT, ValT, ITEMS>) * WARPS + sizeof(uint64_t) * WARPS;
   OFSPMM_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
   DevInfo dev;
@@ -28,31 +28,31 @@ int launch_one(const BwdAtomicParams& p, int panels, cudaStream_t stream) {
   return OFSPMM_OK;
 }
 
-template <typename DT, typename ValT, typename IdxT>
+template <typename DT, typename ValT, typename IdxT, typename PartT>
 int launch_typed(const BwdAtomicParams& p, bool aligned, cudaStream_t stream) {
   constexpr int VECW = 16 / sizeof(DT);
   const int n = p.n;
   if (aligned && n % VECW == 0) {
     const int nvec = n / VECW;
-    if (nvec <= 8) return launch_one<DT, ValT, IdxT, VECW, 8, 1>(p, 1, stream);
-    if (nvec <= 16) return launch_one<DT, ValT, IdxT, VECW, 16, 1>(p, 1, stream);
-    if (nvec <= 32) return launch_one<DT, ValT, IdxT, VECW, 32, 1>(p, 1, stream);
-    if (nvec <= 64) return launch_one<DT, ValT, IdxT, VECW, 32, 2>(p, 1, stream);
-    return launch_one<DT, ValT, IdxT, VECW, 32, 4>(p, (nvec + 127) / 128, stream);
+    if (nvec <= 8) return launch_one<DT, ValT, IdxT, PartT, VECW, 8, 1>(p, 1, stream);
+    if (nvec <= 16) return launch_one<DT, ValT, IdxT, PartT, VECW, 16, 1>(p, 1, stream);
+    if (nvec <= 32) return launch_one<DT, ValT, IdxT, PartT, VECW, 32, 1>(p, 1, stream);
+    if (nvec <= 64) return launch_one<DT, ValT, IdxT, PartT, VECW, 32, 2>(p, 1, stream);
+    return launch_one<DT, ValT, IdxT, PartT, VECW, 32, 4>(p, (nvec + 127) / 128, stream);
   }
-  if (n <= 32) return launch_one<DT, ValT, IdxT, 1, 32, 1>(p, 1, stream);
-  if (n <= 128) return launch_one<DT, ValT, IdxT, 1, 32, 4>(p, 1, stream);
-  return launch_one<DT, ValT, IdxT, 1, 32, 8>(p, (n + 255) / 256, stream);
+  if (n <= 32) return launch_one<DT, ValT, IdxT, PartT, 1, 32, 1>(p, 1, stream);
+  if (n <= 128) return launch_one<DT, ValT, IdxT, PartT, 1, 32, 4>(p, 1, stream);
+  return launch_one<DT, ValT, IdxT, PartT, 1, 32, 8>(p, (n + 255) / 256, stream);
 }
 
-template <typename IdxT>
+template <typename IdxT, typename PartT>
 int launch_idx(const BwdAtomicParams& p, int dense_dtype, int val_dtype, bool aligned, cudaStream_t stream) {
   if (dense_dtype == OFSPMM_DTYPE_FLOAT && val_dtype == OFSPMM_DTYPE_FLOAT)
-    return launch_typed<float, float, IdxT>(p, aligned, stream);
+    return launch_typed<float, float, IdxT, PartT>(p, aligned, stream);
   if (dense_dtype == OFSPMM_DTYPE_BFLOAT16 && val_dtype == OFSPMM_DTYPE_FLOAT)
-    return launch_typed<__nv_bfloat16, float, IdxT>(p, aligned, stream);
+    return launch_typed<__nv_bfloat16, float, IdxT, PartT>(p, aligned, stream);
   if (dense_dtype == OFSPMM_DTYPE_BFLOAT16 && val_dtype == OFSPMM_DTYPE_BFLOAT16)
-    return launch_typed<__nv_bfloat16, __nv_bfloat16, IdxT>(p, aligned, stream);
+    return launch_typed<__nv_bfloat16, __nv_bfloat16, IdxT, PartT>(p, aligned, stream);
   return OFSPMM_ERR_UNSUPPORTED_DTYPE;
 }
 
@@ -68,16 +68,18 @@ int launch_bwd_atomic(const ofspmm_csr* A, const void* dY, float* acc, void* dB_
   p.val = A->val;
   p.dY = dY;
   p.acc = acc;
-  p.part = static_cast<const int2*>(part);
+  p.part = part;
   p.cols = A->cols;
   p.rows = static_cast<int>(A->rows);
-  p.nnz = static_cast<int>(A->nnz);
   p.n = static_cast<int>(n);
   p.P = static_cast<int>(P);
   const bool aligned = ((reinterpret_cast<uintptr_t>(dY) | reinterpret_cast<uintptr_t>(acc)) & 15) == 0;
   int rc = OFSPMM_ERR_UNSUPPORTED_DTYPE;
-  if (A->idx_dtype == OFSPMM_DTYPE_INT32) rc = launch_idx<int32_t>(p, dense_dtype, A->val_dtype, aligned, stream);
-  if (A->idx_dtype == OFSPMM_DTYPE_INT64) rc = launch_idx<int64_t>(p, dense_dtype, A->val_dtype, aligned, stream);
+  if (A->idx_dtype == OFSPMM_DTYPE_INT32) rc = launch_idx<int32_t, int2>(p, dense_dtype, A->val_dtype, aligned, stream);
+  if (A->idx_dtype == OFSPMM_DTYPE_INT64 && !wide_nnz(A->nnz))
+    rc = launch_idx<int64_t, int2>(p, dense_dtype, A->val_dtype, aligned, stream);
+  if (A->idx_dtype == OFSPMM_DTYPE_INT64 && wide_nnz(A->nnz))
+    rc = launch_idx<int64_t, longlong2>(p, dense_dtype, A->val_dtype, aligned, stream);
   if (rc != OFSPMM_OK) return rc;
   if (dB_cast_out != nullptr) {  // bf16 output: cast the fp32 accumulator once
     DevInfo dev;

@@ -32,8 +32,15 @@ bool rows_supported(int64_t n, int dense_dtype) {
 // AUTO (no histogram available): decided from the host-known sizes only — fewer 256-item tasks
 // than resident warps -> 64-item tasks.  With the row-length histogram on the host,
 // ofspmm_choose_variant() may also pick the row-parallel layout (api.cu).
+// Wide matrices (wide_nnz) have 256-item merge-path kernels only: an explicit whole-row or
+// 64-item code falls back to them (AUTO never picks 64-item tasks at that size anyway).
 FwdVariant resolve_variant(int variant, int64_t rows, int64_t nnz, int64_t n, int dense_dtype) {
   FwdVariant v{kTaskItems, false, false};
+  if (wide_nnz(nnz)) {
+    v.row_parallel = (variant & OFSPMM_VARIANT_EXPLICIT) && (variant & OFSPMM_VARIANT_ROWPAR) &&
+                     !(variant & (OFSPMM_VARIANT_ROWS | OFSPMM_VARIANT_ITEMS64)) && rowpar_supported(n, dense_dtype);
+    return v;
+  }
   if (variant & OFSPMM_VARIANT_EXPLICIT) {
     if (variant & OFSPMM_VARIANT_ROWS) {
       // sized like the 64-item family, which is also what runs when a launch cannot use the
@@ -61,13 +68,17 @@ int launch_task_partition(const void* crow, int idx_dtype, int64_t rows, int64_t
   const int threads = 256;
   const unsigned blocks = static_cast<unsigned>((P + 1 + threads - 1) / threads);
   if (idx_dtype == OFSPMM_DTYPE_INT32) {
-    task_partition_kernel<int32_t><<<blocks, threads, 0, stream>>>(
+    task_partition_kernel<int32_t, int2><<<blocks, threads, 0, stream>>>(
         static_cast<const int32_t*>(crow), static_cast<int>(rows), static_cast<int>(nnz), items,
         static_cast<int>(P), static_cast<int2*>(part));
-  } else {
-    task_partition_kernel<int64_t><<<blocks, threads, 0, stream>>>(
+  } else if (!wide_nnz(nnz)) {
+    task_partition_kernel<int64_t, int2><<<blocks, threads, 0, stream>>>(
         static_cast<const int64_t*>(crow), static_cast<int>(rows), static_cast<int>(nnz), items,
         static_cast<int>(P), static_cast<int2*>(part));
+  } else {
+    task_partition_kernel<int64_t, longlong2><<<blocks, threads, 0, stream>>>(
+        static_cast<const int64_t*>(crow), static_cast<int>(rows), static_cast<long long>(nnz), items,
+        static_cast<int>(P), static_cast<longlong2*>(part));
   }
   count_launch();
   OFSPMM_CUDA_OK(cudaGetLastError());
@@ -75,7 +86,8 @@ int launch_task_partition(const void* crow, int idx_dtype, int64_t rows, int64_t
 }
 
 // The whole-row kernel needs what resolve_variant cannot see: the pointers' alignment, the
-// strides and the index dtype of THIS call.
+// strides and the index dtype of THIS call.  It never serves a wide matrix (resolve_variant
+// clears whole_rows for those; they have int64 indices besides).
 bool rows_kernel_applies(const ofspmm_csr* A, const void* B, int64_t ldb, const void* C, int64_t ldc, int64_t n,
                          int dense_dtype, const FwdLaunch& L) {
   if (!L.variant.whole_rows || A->idx_dtype != OFSPMM_DTYPE_INT32 || !rows_supported(n, dense_dtype)) return false;
@@ -96,12 +108,11 @@ int launch_fwd(const ofspmm_csr* A, const void* B, int64_t ldb, void* C, int64_t
   p.val = A->val;
   p.B = B;
   p.C = C;
-  p.part = static_cast<const int2*>(part);
+  p.part = part;
   p.carry = carry;
   p.head = head;
   p.cols = A->cols;
   p.rows = static_cast<int>(A->rows);
-  p.nnz = static_cast<int>(A->nnz);
   p.n = static_cast<int>(n);
   p.P = static_cast<int>(P);
   p.panels = 1;

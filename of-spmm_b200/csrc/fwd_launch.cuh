@@ -9,11 +9,12 @@
 
 namespace ofspmm {
 
-template <typename DT, typename ValT, typename IdxT, int VEC, int LPR, int CH, bool kFull, bool kRowPar, int ITEMS>
+template <typename DT, typename ValT, typename IdxT, typename PartT, int VEC, int LPR, int CH, bool kFull, bool kRowPar, int ITEMS>
 int launch_full(FwdParams p, int panels, const FwdLaunch& L, cudaStream_t stream) {
+  if (static_cast<int64_t>(p.P) * panels >= kMaxTasks) return OFSPMM_ERR_TOO_LARGE;
   p.panels = panels;
   constexpr int WARPS = kWarpsPerCta;
-  auto kern = spmm_merge_kernel<DT, ValT, IdxT, VEC, LPR, CH, kFull, kRowPar, ITEMS, WARPS>;
+  auto kern = spmm_merge_kernel<DT, ValT, IdxT, VEC, LPR, CH, kFull, kRowPar, ITEMS, WARPS, PartT>;
   const size_t smem = sizeof(TaskStage<IdxT, ValT, ITEMS>) * WARPS + sizeof(uint64_t) * WARPS;
   DevInfo dev;
   if (int rc = get_dev_info(&dev)) return rc;
@@ -53,7 +54,7 @@ int launch_full(FwdParams p, int panels, const FwdLaunch& L, cudaStream_t stream
   count_launch();
   OFSPMM_CUDA_OK(cudaGetLastError());
   if (p.P > 1) {  // stitch rows that span several tasks (a single task cannot split a row)
-    auto fix = spmm_fixup_kernel<DT, IdxT, VEC, WARPS>;
+    auto fix = spmm_fixup_kernel<DT, IdxT, VEC, WARPS, PartT>;
     fix<<<static_cast<unsigned>((ctas_needed + 31) / 32), WARPS * 32, 0, stream>>>(p);  // one lane per task
     count_launch();
     OFSPMM_CUDA_OK(cudaGetLastError());
@@ -62,59 +63,65 @@ int launch_full(FwdParams p, int panels, const FwdLaunch& L, cudaStream_t stream
 }
 
 // kFull (no masked lanes, immediate chunk offsets) when n is a whole number of register tiles.
-template <typename DT, typename ValT, typename IdxT, int VEC, int LPR, int CH, bool kRowPar, int ITEMS>
+template <typename DT, typename ValT, typename IdxT, typename PartT, int VEC, int LPR, int CH, bool kRowPar, int ITEMS>
 int launch_one(const FwdParams& p, int panels, const FwdLaunch& L, cudaStream_t stream) {
   if (p.n % (LPR * VEC * CH) == 0)
-    return launch_full<DT, ValT, IdxT, VEC, LPR, CH, true, kRowPar, ITEMS>(p, panels, L, stream);
-  return launch_full<DT, ValT, IdxT, VEC, LPR, CH, false, kRowPar, ITEMS>(p, panels, L, stream);
+    return launch_full<DT, ValT, IdxT, PartT, VEC, LPR, CH, true, kRowPar, ITEMS>(p, panels, L, stream);
+  return launch_full<DT, ValT, IdxT, PartT, VEC, LPR, CH, false, kRowPar, ITEMS>(p, panels, L, stream);
 }
 
 // Lane layout by dense width: 8 / 16 lanes per row (vector-per-row: 4 / 2 non-zero groups per
 // warp instruction) or 32 lanes x 1 / 2 / 4 16-byte chunks (warp-per-row); scalar lanes when the
 // rows are not 16-byte aligned.  The row-parallel family only exists for the sub-warp layouts
 // (fwd.cu checks rowpar_supported() first).
-template <typename DT, typename ValT, typename IdxT, bool kRowPar, int ITEMS>
+template <typename DT, typename ValT, typename IdxT, typename PartT, bool kRowPar, int ITEMS>
 int launch_typed(const FwdParams& p, bool aligned, const FwdLaunch& L, cudaStream_t stream) {
   constexpr int VECW = 16 / sizeof(DT);
   const int n = p.n;
   if (aligned && n % VECW == 0 && p.ldb % VECW == 0 && p.ldc % VECW == 0) {
     const int nvec = n / VECW;
-    if (nvec <= 8) return launch_one<DT, ValT, IdxT, VECW, 8, 1, kRowPar, ITEMS>(p, 1, L, stream);
-    if (nvec <= 16) return launch_one<DT, ValT, IdxT, VECW, 16, 1, kRowPar, ITEMS>(p, 1, L, stream);
+    if (nvec <= 8) return launch_one<DT, ValT, IdxT, PartT, VECW, 8, 1, kRowPar, ITEMS>(p, 1, L, stream);
+    if (nvec <= 16) return launch_one<DT, ValT, IdxT, PartT, VECW, 16, 1, kRowPar, ITEMS>(p, 1, L, stream);
     if constexpr (!kRowPar) {
-      if (nvec <= 32) return launch_one<DT, ValT, IdxT, VECW, 32, 1, false, ITEMS>(p, 1, L, stream);
-      if (nvec <= 64) return launch_one<DT, ValT, IdxT, VECW, 32, 2, false, ITEMS>(p, 1, L, stream);
-      return launch_one<DT, ValT, IdxT, VECW, 32, 4, false, ITEMS>(p, (nvec + 127) / 128, L, stream);
+      if (nvec <= 32) return launch_one<DT, ValT, IdxT, PartT, VECW, 32, 1, false, ITEMS>(p, 1, L, stream);
+      if (nvec <= 64) return launch_one<DT, ValT, IdxT, PartT, VECW, 32, 2, false, ITEMS>(p, 1, L, stream);
+      return launch_one<DT, ValT, IdxT, PartT, VECW, 32, 4, false, ITEMS>(p, (nvec + 127) / 128, L, stream);
     }
     return OFSPMM_ERR_INVALID_ARG;  // unreachable: rowpar_supported() guards it
   }
   if constexpr (!kRowPar) {
-    if (n <= 32) return launch_one<DT, ValT, IdxT, 1, 32, 1, false, ITEMS>(p, 1, L, stream);
-    if (n <= 64) return launch_one<DT, ValT, IdxT, 1, 32, 2, false, ITEMS>(p, 1, L, stream);
-    if (n <= 128) return launch_one<DT, ValT, IdxT, 1, 32, 4, false, ITEMS>(p, 1, L, stream);
-    return launch_one<DT, ValT, IdxT, 1, 32, 8, false, ITEMS>(p, (n + 255) / 256, L, stream);
+    if (n <= 32) return launch_one<DT, ValT, IdxT, PartT, 1, 32, 1, false, ITEMS>(p, 1, L, stream);
+    if (n <= 64) return launch_one<DT, ValT, IdxT, PartT, 1, 32, 2, false, ITEMS>(p, 1, L, stream);
+    if (n <= 128) return launch_one<DT, ValT, IdxT, PartT, 1, 32, 4, false, ITEMS>(p, 1, L, stream);
+    return launch_one<DT, ValT, IdxT, PartT, 1, 32, 8, false, ITEMS>(p, (n + 255) / 256, L, stream);
   }
   return OFSPMM_ERR_INVALID_ARG;
 }
 
-template <typename IdxT, bool kRowPar, int ITEMS>
+template <typename IdxT, typename PartT, bool kRowPar, int ITEMS>
 int launch_idx(const FwdParams& p, int dense_dtype, int val_dtype, bool aligned, const FwdLaunch& L,
                cudaStream_t stream) {
   if (dense_dtype == OFSPMM_DTYPE_FLOAT && val_dtype == OFSPMM_DTYPE_FLOAT)
-    return launch_typed<float, float, IdxT, kRowPar, ITEMS>(p, aligned, L, stream);
+    return launch_typed<float, float, IdxT, PartT, kRowPar, ITEMS>(p, aligned, L, stream);
   if (dense_dtype == OFSPMM_DTYPE_BFLOAT16 && val_dtype == OFSPMM_DTYPE_FLOAT)
-    return launch_typed<__nv_bfloat16, float, IdxT, kRowPar, ITEMS>(p, aligned, L, stream);
+    return launch_typed<__nv_bfloat16, float, IdxT, PartT, kRowPar, ITEMS>(p, aligned, L, stream);
   if (dense_dtype == OFSPMM_DTYPE_BFLOAT16 && val_dtype == OFSPMM_DTYPE_BFLOAT16)
-    return launch_typed<__nv_bfloat16, __nv_bfloat16, IdxT, kRowPar, ITEMS>(p, aligned, L, stream);
+    return launch_typed<__nv_bfloat16, __nv_bfloat16, IdxT, PartT, kRowPar, ITEMS>(p, aligned, L, stream);
   return OFSPMM_ERR_UNSUPPORTED_DTYPE;
 }
 
 template <bool kRowPar, int ITEMS>
 int launch_family(const FwdParams& p, int idx_dtype, int dense_dtype, int val_dtype, bool aligned,
                   const FwdLaunch& L, cudaStream_t stream) {
-  if (idx_dtype == OFSPMM_DTYPE_INT32) return launch_idx<int32_t, kRowPar, ITEMS>(p, dense_dtype, val_dtype, aligned, L, stream);
-  if (idx_dtype == OFSPMM_DTYPE_INT64) return launch_idx<int64_t, kRowPar, ITEMS>(p, dense_dtype, val_dtype, aligned, L, stream);
-  return OFSPMM_ERR_UNSUPPORTED_DTYPE;
+  if (idx_dtype == OFSPMM_DTYPE_INT32 && !L.wide)
+    return launch_idx<int32_t, int2, kRowPar, ITEMS>(p, dense_dtype, val_dtype, aligned, L, stream);
+  if (idx_dtype == OFSPMM_DTYPE_INT64 && !L.wide)
+    return launch_idx<int64_t, int2, kRowPar, ITEMS>(p, dense_dtype, val_dtype, aligned, L, stream);
+  // wide matrices: 256-item tasks only (resolve_variant never gives them 64-item tasks)
+  if constexpr (ITEMS == kTaskItems) {
+    if (idx_dtype == OFSPMM_DTYPE_INT64) return launch_idx<int64_t, longlong2, kRowPar, ITEMS>(p, dense_dtype, val_dtype, aligned, L, stream);
+  }
+  return L.wide ? OFSPMM_ERR_TOO_LARGE : OFSPMM_ERR_UNSUPPORTED_DTYPE;
 }
 
 }  // namespace ofspmm

@@ -32,6 +32,16 @@ inline int64_t num_tasks(int64_t rows, int64_t nnz, int items = kTaskItems) {
   return (total + items - 1) / items;
 }
 
+// Matrices with at least this many non-zeros ("wide"; int64 indices only, int32 row offsets cannot
+// hold them) keep 64-bit non-zero offsets in their task partition: 16-byte longlong2 entries
+// instead of int2 (spmm_kernels.cuh:PartOf).  Below it every kernel runs exactly as with int2.
+constexpr int64_t kWideNnz = (int64_t{1} << 31) - 1;
+inline bool wide_nnz(int64_t nnz) { return nnz >= kWideNnz; }
+inline size_t part_entry_bytes(int64_t nnz) { return wide_nnz(nnz) ? 16 : 8; }
+// Task indices (task count x column panels) are drawn from a 32-bit counter and held in int; 2^30
+// leaves room for the draws warps make past the last task.
+constexpr int64_t kMaxTasks = int64_t{1} << 30;
+
 // Resolved kernel family of a forward launch (public encoding: OFSPMM_VARIANT_*).
 struct FwdVariant {
   int items;          // merge items per warp task: kTaskItems or kSmallTaskItems
@@ -50,6 +60,7 @@ struct FwdLaunch {
   int tasks_per_warp;  // 0 = persistent grid
   int reserve_ctas;    // CTA slots per SM a persistent grid leaves free for overlapping exchange kernels
   bool dynamic;        // tasks drawn from a global counter (persistent grid only)
+  bool wide;           // 64-bit non-zero offsets in the task partition (wide_nnz)
   unsigned flags;      // kFwd* epilogue bits
   const void* bias;
   float* acc32;        // fp32 accumulator of multi-pass 16-bit products

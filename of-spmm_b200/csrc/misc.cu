@@ -45,14 +45,15 @@ __global__ void row_hist_kernel(const IdxT* __restrict__ crow, long long rows,
 // Sort keys of the transpose: the column index, or the sentinel `cols` for an index outside
 // [0, cols) — such entries are skipped by every kernel of the library (include/ofspmm.h), so they
 // must not alias into a valid column bucket; they sort behind every valid key.  pos[p] = p.
-template <typename IdxT>
+// KeyT is 32-bit whenever the sentinel fits (halves the key buffers of an int64 matrix).
+template <typename IdxT, typename KeyT>
 __global__ void transpose_keys_kernel(const IdxT* __restrict__ col, long long cols, long long count,
-                                      IdxT* __restrict__ keys, IdxT* __restrict__ pos) {
+                                      KeyT* __restrict__ keys, IdxT* __restrict__ pos) {
   const long long stride = static_cast<long long>(gridDim.x) * blockDim.x;
   for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < count; i += stride) {
     const IdxT c = col[i];
     const bool ok = static_cast<unsigned long long>(c) < static_cast<unsigned long long>(cols);
-    keys[i] = ok ? c : static_cast<IdxT>(cols);
+    keys[i] = ok ? static_cast<KeyT>(c) : static_cast<KeyT>(cols);
     pos[i] = static_cast<IdxT>(i);
   }
 }
@@ -60,8 +61,8 @@ __global__ void transpose_keys_kernel(const IdxT* __restrict__ col, long long co
 // t_crow[c] = first position in the column-sorted key array whose key is >= c.  t_crow[cols] is
 // pinned to nnz (crow[rows] == nnz is what the merge-path kernels rely on): the skipped entries
 // therefore trail the last row of A^T, where the fill kernel marks them with column -1.
-template <typename IdxT>
-__global__ void transpose_offsets_kernel(const IdxT* __restrict__ sorted_cols, long long nnz,
+template <typename IdxT, typename KeyT>
+__global__ void transpose_offsets_kernel(const KeyT* __restrict__ sorted_cols, long long nnz,
                                          long long cols, IdxT* __restrict__ t_crow) {
   const long long c = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (c > cols) return;
@@ -78,10 +79,10 @@ __global__ void transpose_offsets_kernel(const IdxT* __restrict__ sorted_cols, l
 }
 
 // For transposed position q with source position p = perm[q]: row(p) by binary search in crow.
-template <typename IdxT, typename ValT>
+template <typename IdxT, typename KeyT, typename ValT>
 __global__ void transpose_fill_kernel(const IdxT* __restrict__ crow, long long rows,
                                       const ValT* __restrict__ val, const IdxT* __restrict__ perm,
-                                      const IdxT* __restrict__ sorted_keys, long long cols,
+                                      const KeyT* __restrict__ sorted_keys, long long cols,
                                       long long nnz, IdxT* __restrict__ t_col, ValT* __restrict__ t_val) {
   const long long stride = static_cast<long long>(gridDim.x) * blockDim.x;
   for (long long q = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; q < nnz; q += stride) {
@@ -107,71 +108,85 @@ int bits_for(int64_t cols) {
   return b;
 }
 
-template <typename IdxT>
+template <typename KeyT, typename IdxT>
 size_t cub_sort_temp_bytes(int64_t nnz, int end_bit) {
   size_t bytes = 0;
-  cub::DeviceRadixSort::SortPairs(nullptr, bytes, static_cast<const IdxT*>(nullptr),
-                                  static_cast<IdxT*>(nullptr), static_cast<const IdxT*>(nullptr),
-                                  static_cast<IdxT*>(nullptr), static_cast<long long>(nnz), 0, end_bit);
+  cub::DoubleBuffer<KeyT> keys(nullptr, nullptr);
+  cub::DoubleBuffer<IdxT> vals(nullptr, nullptr);
+  cub::DeviceRadixSort::SortPairs(nullptr, bytes, keys, vals, static_cast<long long>(nnz), 0, end_bit);
   return bytes;
 }
 
+// Workspace of the transpose: two key buffers and one position buffer for the ping-pong radix
+// sort (the other position buffer is t_perm, or t_col when the caller keeps no t_perm: both are
+// nnz-long IdxT outputs) and cub's scratch.
 struct TransposeLayout {
-  size_t keys_in, keys_out, pos_in, pos_out, cub_tmp, cub_bytes, total;
+  size_t keys_a, keys_b, pos, cub_tmp, cub_bytes, total;
 };
 
-template <typename IdxT>
+// Column keys are 32-bit when the sentinel `cols` fits an int32 (every int32 matrix does).
+bool narrow_keys(int64_t cols) { return cols < (int64_t{1} << 31) - 1; }
+
+template <typename IdxT, typename KeyT>
 TransposeLayout transpose_layout(int64_t cols, int64_t nnz) {
   TransposeLayout L;
-  const size_t arr = align_up(static_cast<size_t>(nnz > 0 ? nnz : 1) * sizeof(IdxT), 256);
-  L.keys_in = 0;
-  L.keys_out = arr;
-  L.pos_in = 2 * arr;
-  L.pos_out = 3 * arr;
-  L.cub_tmp = 4 * arr;
-  L.cub_bytes = cub_sort_temp_bytes<IdxT>(nnz, bits_for(cols + 1));
+  const size_t n = static_cast<size_t>(nnz > 0 ? nnz : 1);
+  const size_t karr = align_up(n * sizeof(KeyT), 256);
+  L.keys_a = 0;
+  L.keys_b = karr;
+  L.pos = 2 * karr;
+  L.cub_tmp = L.pos + align_up(n * sizeof(IdxT), 256);
+  L.cub_bytes = cub_sort_temp_bytes<KeyT, IdxT>(nnz, bits_for(cols + 1));
   L.total = L.cub_tmp + align_up(L.cub_bytes, 256);
   return L;
 }
 
-template <typename IdxT>
+template <typename IdxT, typename KeyT>
 int transpose_impl(const ofspmm_csr* A, void* t_crow, void* t_col, void* t_val, void* t_perm,
                    void* ws, size_t ws_bytes, cudaStream_t stream) {
   const int64_t nnz = A->nnz, rows = A->rows, cols = A->cols;
-  const TransposeLayout L = transpose_layout<IdxT>(cols, nnz);
+  const TransposeLayout L = transpose_layout<IdxT, KeyT>(cols, nnz);
   if (ws == nullptr || ws_bytes < L.total) return OFSPMM_ERR_WORKSPACE;
   unsigned char* w = static_cast<unsigned char*>(ws);
-  IdxT* keys_in = reinterpret_cast<IdxT*>(w + L.keys_in);
-  IdxT* keys_out = reinterpret_cast<IdxT*>(w + L.keys_out);
-  IdxT* pos_in = reinterpret_cast<IdxT*>(w + L.pos_in);
-  IdxT* pos_out = t_perm != nullptr ? static_cast<IdxT*>(t_perm) : reinterpret_cast<IdxT*>(w + L.pos_out);
+  cub::DoubleBuffer<KeyT> keys(reinterpret_cast<KeyT*>(w + L.keys_a), reinterpret_cast<KeyT*>(w + L.keys_b));
+  IdxT* pos_ws = reinterpret_cast<IdxT*>(w + L.pos);
+  cub::DoubleBuffer<IdxT> pos(pos_ws, static_cast<IdxT*>(t_perm != nullptr ? t_perm : t_col));
+  // where the sorted positions must end up: t_perm when the caller keeps them, else the workspace
+  // buffer; never t_col, which the fill kernel overwrites with rows
+  IdxT* perm = t_perm != nullptr ? static_cast<IdxT*>(t_perm) : pos_ws;
   DevInfo dev;
   if (int rc = get_dev_info(&dev)) return rc;
   const int grid = dev.sms * 8;
   if (nnz > 0) {
-    transpose_keys_kernel<IdxT><<<grid, 256, 0, stream>>>(static_cast<const IdxT*>(A->col), cols, nnz, keys_in, pos_in);
+    transpose_keys_kernel<IdxT, KeyT><<<grid, 256, 0, stream>>>(static_cast<const IdxT*>(A->col), cols, nnz,
+                                                                keys.Current(), pos.Current());
     count_launch();
     size_t cub_bytes = L.cub_bytes;
     // stable LSD radix sort by column: entries of one column keep ascending source position,
-    // i.e. ascending row — the transposed CSR is deterministic and row-sorted.
-    OFSPMM_CUDA_OK(cub::DeviceRadixSort::SortPairs(w + L.cub_tmp, cub_bytes, static_cast<const IdxT*>(keys_in),
-                                                   keys_out, static_cast<const IdxT*>(pos_in), pos_out,
-                                                   static_cast<long long>(nnz), 0, bits_for(cols + 1), stream));
+    // i.e. ascending row — the transposed CSR is deterministic and row-sorted.  The ping-pong
+    // overload needs no nnz-long scratch of its own.
+    OFSPMM_CUDA_OK(cub::DeviceRadixSort::SortPairs(w + L.cub_tmp, cub_bytes, keys, pos, static_cast<long long>(nnz),
+                                                   0, bits_for(cols + 1), stream));
     count_launch(4);
+    if (pos.Current() != perm)
+      OFSPMM_CUDA_OK(cudaMemcpyAsync(perm, pos.Current(), static_cast<size_t>(nnz) * sizeof(IdxT),
+                                     cudaMemcpyDeviceToDevice, stream));
   }
-  transpose_offsets_kernel<IdxT><<<static_cast<unsigned>((cols + 1 + 255) / 256), 256, 0, stream>>>(
+  const KeyT* keys_out = keys.Current();
+  IdxT* pos_out = perm;
+  transpose_offsets_kernel<IdxT, KeyT><<<static_cast<unsigned>((cols + 1 + 255) / 256), 256, 0, stream>>>(
       keys_out, nnz, cols, static_cast<IdxT*>(t_crow));
   count_launch();
   if (nnz > 0) {
     if (A->val == nullptr || t_val == nullptr) {
-      transpose_fill_kernel<IdxT, float><<<grid, 256, 0, stream>>>(
+      transpose_fill_kernel<IdxT, KeyT, float><<<grid, 256, 0, stream>>>(
           static_cast<const IdxT*>(A->crow), rows, nullptr, pos_out, keys_out, cols, nnz, static_cast<IdxT*>(t_col), nullptr);
     } else if (A->val_dtype == OFSPMM_DTYPE_FLOAT) {
-      transpose_fill_kernel<IdxT, float><<<grid, 256, 0, stream>>>(
+      transpose_fill_kernel<IdxT, KeyT, float><<<grid, 256, 0, stream>>>(
           static_cast<const IdxT*>(A->crow), rows, static_cast<const float*>(A->val), pos_out, keys_out, cols, nnz,
           static_cast<IdxT*>(t_col), static_cast<float*>(t_val));
     } else if (A->val_dtype == OFSPMM_DTYPE_BFLOAT16) {
-      transpose_fill_kernel<IdxT, __nv_bfloat16><<<grid, 256, 0, stream>>>(
+      transpose_fill_kernel<IdxT, KeyT, __nv_bfloat16><<<grid, 256, 0, stream>>>(
           static_cast<const IdxT*>(A->crow), rows, static_cast<const __nv_bfloat16*>(A->val), pos_out, keys_out, cols, nnz,
           static_cast<IdxT*>(t_col), static_cast<__nv_bfloat16*>(t_val));
     } else {
@@ -227,14 +242,17 @@ int launch_row_hist(const void* crow, int idx_dtype, int64_t rows, int64_t* hist
 
 size_t transpose_workspace_bytes(int64_t rows, int64_t cols, int64_t nnz, int idx_dtype) {
   (void)rows;
-  if (idx_dtype == OFSPMM_DTYPE_INT64) return transpose_layout<int64_t>(cols, nnz).total;
-  return transpose_layout<int32_t>(cols, nnz).total;
+  if (idx_dtype == OFSPMM_DTYPE_INT32) return transpose_layout<int32_t, int32_t>(cols, nnz).total;
+  if (narrow_keys(cols)) return transpose_layout<int64_t, int32_t>(cols, nnz).total;
+  return transpose_layout<int64_t, int64_t>(cols, nnz).total;
 }
 
 int launch_transpose(const ofspmm_csr* A, void* t_crow, void* t_col, void* t_val, void* t_perm,
                      void* ws, size_t ws_bytes, cudaStream_t stream) {
-  if (A->idx_dtype == OFSPMM_DTYPE_INT32) return transpose_impl<int32_t>(A, t_crow, t_col, t_val, t_perm, ws, ws_bytes, stream);
-  if (A->idx_dtype == OFSPMM_DTYPE_INT64) return transpose_impl<int64_t>(A, t_crow, t_col, t_val, t_perm, ws, ws_bytes, stream);
+  if (A->idx_dtype == OFSPMM_DTYPE_INT32) return transpose_impl<int32_t, int32_t>(A, t_crow, t_col, t_val, t_perm, ws, ws_bytes, stream);
+  if (A->idx_dtype == OFSPMM_DTYPE_INT64 && narrow_keys(A->cols))
+    return transpose_impl<int64_t, int32_t>(A, t_crow, t_col, t_val, t_perm, ws, ws_bytes, stream);
+  if (A->idx_dtype == OFSPMM_DTYPE_INT64) return transpose_impl<int64_t, int64_t>(A, t_crow, t_col, t_val, t_perm, ws, ws_bytes, stream);
   return OFSPMM_ERR_UNSUPPORTED_DTYPE;
 }
 

@@ -29,52 +29,52 @@ int launch_persistent(Kern kern, SddmmParams p, size_t smem, bool dynamic_ok, Ke
   return OFSPMM_OK;
 }
 
-template <typename DT, typename ValT, typename IdxT, int VEC, int LPR, int CH>
+template <typename DT, typename ValT, typename IdxT, typename PartT, int VEC, int LPR, int CH>
 int launch_one(const SddmmParams& p, cudaStream_t stream) {
   constexpr int ITEMS = kTaskItems;
   constexpr int WARPS = kWarpsPerCta;
   const size_t smem = sizeof(TaskStage<IdxT, float, ITEMS>) * WARPS + sizeof(uint64_t) * WARPS;
   static KernelLaunchCache cache_full, cache_masked;
   if (p.n % (LPR * VEC * CH) == 0)
-    return launch_persistent(sddmm_merge_kernel<DT, ValT, IdxT, VEC, LPR, CH, true, ITEMS, WARPS>, p, smem, true, cache_full, stream);
-  return launch_persistent(sddmm_merge_kernel<DT, ValT, IdxT, VEC, LPR, CH, false, ITEMS, WARPS>, p, smem, true, cache_masked, stream);
+    return launch_persistent(sddmm_merge_kernel<DT, ValT, IdxT, VEC, LPR, CH, true, ITEMS, WARPS, PartT>, p, smem, true, cache_full, stream);
+  return launch_persistent(sddmm_merge_kernel<DT, ValT, IdxT, VEC, LPR, CH, false, ITEMS, WARPS, PartT>, p, smem, true, cache_masked, stream);
 }
 
-template <typename DT, typename ValT, typename IdxT, int VEC>
+template <typename DT, typename ValT, typename IdxT, typename PartT, int VEC>
 int launch_wide(const SddmmParams& p, cudaStream_t stream) {
   constexpr int ITEMS = kTaskItems;
   constexpr int WARPS = kWarpsPerCta;
   const size_t smem = sizeof(TaskStage<IdxT, float, ITEMS>) * WARPS + sizeof(uint64_t) * WARPS;
   static KernelLaunchCache cache;
-  return launch_persistent(sddmm_wide_kernel<DT, ValT, IdxT, VEC, ITEMS, WARPS>, p, smem, false, cache, stream);
+  return launch_persistent(sddmm_wide_kernel<DT, ValT, IdxT, VEC, ITEMS, WARPS, PartT>, p, smem, false, cache, stream);
 }
 
-template <typename DT, typename ValT, typename IdxT>
+template <typename DT, typename ValT, typename IdxT, typename PartT>
 int launch_typed(const SddmmParams& p, bool aligned, cudaStream_t stream) {
   constexpr int VECW = 16 / sizeof(DT);
   const int n = p.n;
   if (aligned && n % VECW == 0) {
     const int nvec = n / VECW;
-    if (nvec <= 8) return launch_one<DT, ValT, IdxT, VECW, 8, 1>(p, stream);
-    if (nvec <= 16) return launch_one<DT, ValT, IdxT, VECW, 16, 1>(p, stream);
-    if (nvec <= 32) return launch_one<DT, ValT, IdxT, VECW, 32, 1>(p, stream);
-    if (nvec <= 64) return launch_one<DT, ValT, IdxT, VECW, 32, 2>(p, stream);
-    if (nvec <= 128) return launch_one<DT, ValT, IdxT, VECW, 32, 4>(p, stream);
-    return launch_wide<DT, ValT, IdxT, VECW>(p, stream);
+    if (nvec <= 8) return launch_one<DT, ValT, IdxT, PartT, VECW, 8, 1>(p, stream);
+    if (nvec <= 16) return launch_one<DT, ValT, IdxT, PartT, VECW, 16, 1>(p, stream);
+    if (nvec <= 32) return launch_one<DT, ValT, IdxT, PartT, VECW, 32, 1>(p, stream);
+    if (nvec <= 64) return launch_one<DT, ValT, IdxT, PartT, VECW, 32, 2>(p, stream);
+    if (nvec <= 128) return launch_one<DT, ValT, IdxT, PartT, VECW, 32, 4>(p, stream);
+    return launch_wide<DT, ValT, IdxT, PartT, VECW>(p, stream);
   }
-  if (n <= 32) return launch_one<DT, ValT, IdxT, 1, 32, 1>(p, stream);
-  if (n <= 128) return launch_one<DT, ValT, IdxT, 1, 32, 4>(p, stream);
-  return launch_wide<DT, ValT, IdxT, 1>(p, stream);
+  if (n <= 32) return launch_one<DT, ValT, IdxT, PartT, 1, 32, 1>(p, stream);
+  if (n <= 128) return launch_one<DT, ValT, IdxT, PartT, 1, 32, 4>(p, stream);
+  return launch_wide<DT, ValT, IdxT, PartT, 1>(p, stream);
 }
 
-template <typename IdxT>
+template <typename IdxT, typename PartT>
 int launch_idx(const SddmmParams& p, int dense_dtype, int val_dtype, bool aligned, cudaStream_t stream) {
   if (dense_dtype == OFSPMM_DTYPE_FLOAT && val_dtype == OFSPMM_DTYPE_FLOAT)
-    return launch_typed<float, float, IdxT>(p, aligned, stream);
+    return launch_typed<float, float, IdxT, PartT>(p, aligned, stream);
   if (dense_dtype == OFSPMM_DTYPE_BFLOAT16 && val_dtype == OFSPMM_DTYPE_FLOAT)
-    return launch_typed<__nv_bfloat16, float, IdxT>(p, aligned, stream);
+    return launch_typed<__nv_bfloat16, float, IdxT, PartT>(p, aligned, stream);
   if (dense_dtype == OFSPMM_DTYPE_BFLOAT16 && val_dtype == OFSPMM_DTYPE_BFLOAT16)
-    return launch_typed<__nv_bfloat16, __nv_bfloat16, IdxT>(p, aligned, stream);
+    return launch_typed<__nv_bfloat16, __nv_bfloat16, IdxT, PartT>(p, aligned, stream);
   return OFSPMM_ERR_UNSUPPORTED_DTYPE;
 }
 
@@ -89,15 +89,16 @@ int launch_sddmm(const ofspmm_csr* A, const void* dY, const void* B, void* dval,
   p.dY = dY;
   p.B = B;
   p.dval = dval;
-  p.part = static_cast<const int2*>(part);
+  p.part = part;
   p.cols = A->cols;
   p.rows = static_cast<int>(A->rows);
-  p.nnz = static_cast<int>(A->nnz);
   p.n = static_cast<int>(n);
   p.P = static_cast<int>(P);
   const bool aligned = ((reinterpret_cast<uintptr_t>(B) | reinterpret_cast<uintptr_t>(dY)) & 15) == 0;
-  if (A->idx_dtype == OFSPMM_DTYPE_INT32) return launch_idx<int32_t>(p, dense_dtype, A->val_dtype, aligned, stream);
-  if (A->idx_dtype == OFSPMM_DTYPE_INT64) return launch_idx<int64_t>(p, dense_dtype, A->val_dtype, aligned, stream);
+  if (A->idx_dtype == OFSPMM_DTYPE_INT32) return launch_idx<int32_t, int2>(p, dense_dtype, A->val_dtype, aligned, stream);
+  if (A->idx_dtype == OFSPMM_DTYPE_INT64 && !wide_nnz(A->nnz))
+    return launch_idx<int64_t, int2>(p, dense_dtype, A->val_dtype, aligned, stream);
+  if (A->idx_dtype == OFSPMM_DTYPE_INT64) return launch_idx<int64_t, longlong2>(p, dense_dtype, A->val_dtype, aligned, stream);
   return OFSPMM_ERR_UNSUPPORTED_DTYPE;
 }
 

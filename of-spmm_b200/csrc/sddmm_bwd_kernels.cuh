@@ -11,11 +11,11 @@ struct SddmmParams {
   const void* dY;   // rows x n
   const void* B;    // cols x n
   void* dval;       // nnz
-  const int2* part;
+  const void* part;  // int2 or longlong2 entries (PartOf in spmm_kernels.cuh)
   unsigned int* counter;  // dynamic task order (see spmm_merge_kernel); nullptr = static
   long long cols;
   int rows;
-  int nnz;
+  int reserved = 0;  // not read; keeps the parameter layout the narrow kernels were tuned with
   int n;
   int P;
 };
@@ -34,9 +34,11 @@ __device__ __forceinline__ unsigned group_mask(int grp) {
 // transpose-reduce across the LPR lanes (log2(LPR)+1 shuffles for the 4 results instead of
 // 4·log2(LPR)).  Results are staged in shared memory (the stage's unused value array) and written
 // back coalesced; out-of-range columns produce 0 (the oracle's convention).
-template <typename DT, typename ValT, typename IdxT, int VEC, int LPR, int CH, bool kFull, int ITEMS, int WARPS>
+template <typename DT, typename ValT, typename IdxT, int VEC, int LPR, int CH, bool kFull, int ITEMS, int WARPS, typename PartT>
 __global__ void __launch_bounds__(WARPS * 32, min_ctas_per_sm<DT, CH>())
 sddmm_merge_kernel(const SddmmParams p) {
+  using NzT = typename PartOf<PartT>::Nz;
+  const PartT* part = static_cast<const PartT*>(p.part);
   constexpr int G = 32 / LPR;
   constexpr bool kVecIdx = sizeof(IdxT) == 4;
   constexpr uint32_t kChunkBytes = LPR * VEC * sizeof(DT);
@@ -98,11 +100,12 @@ sddmm_merge_kernel(const SddmmParams p) {
   for (; k < p.P; k = k1, k1 = dynamic ? static_cast<int>(__shfl_sync(0xffffffffu, pending, 0)) : k1 + total_warps) {
     pending = 0;
     if (dynamic && lane == 0) pending = atomicAdd(p.counter, 1u);
-    if (k1 < p.P && lane == 0) asm volatile("prefetch.global.L2 [%0];" ::"l"(&p.part[k1]));
-    const int2 ps = __ldg(&p.part[k]);
-    const int2 pe = __ldg(&p.part[k + 1]);
-    const int rs = ps.x, ns = ps.y, re = pe.x, ne = pe.y;
-    const int cnt_nz = ne - ns;
+    if (k1 < p.P && lane == 0) asm volatile("prefetch.global.L2 [%0];" ::"l"(&part[k1]));
+    const PartT ps = PartOf<PartT>::load(&part[k]);
+    const PartT pe = PartOf<PartT>::load(&part[k + 1]);
+    const int rs = static_cast<int>(ps.x), re = static_cast<int>(pe.x);
+    const NzT ns = ps.y;
+    const int cnt_nz = static_cast<int>(pe.y - ns);
     if (cnt_nz == 0) continue;
     const StagedTask<IdxT, float> tk = stage_task<false>(st, bar, phase, crow, col, static_cast<const float*>(nullptr),
                                                         rs, ns, re - rs + 1, cnt_nz, p.cols, lane, pol_stream);
@@ -110,7 +113,7 @@ sddmm_merge_kernel(const SddmmParams p) {
 
     int e = 0;
     for (int r = rs; r <= re; ++r) {
-      const int e_end = r < re ? static_cast<int>(tk.srow[r - rs + 1]) - ns : cnt_nz;
+      const int e_end = r < re ? task_rel(tk.srow[r - rs + 1], ns) : cnt_nz;
       if (e_end <= e) continue;
       // dY row chunk → registers
       float y[CH][VEC];
@@ -229,8 +232,10 @@ sddmm_merge_kernel(const SddmmParams p) {
 
 // Very wide dense rows (n beyond the register tile): loop over the row in LPR*VEC-column steps,
 // re-reading the dY chunk from L1 each time.
-template <typename DT, typename ValT, typename IdxT, int VEC, int ITEMS, int WARPS>
+template <typename DT, typename ValT, typename IdxT, int VEC, int ITEMS, int WARPS, typename PartT>
 __global__ void __launch_bounds__(WARPS * 32) sddmm_wide_kernel(const SddmmParams p) {
+  using NzT = typename PartOf<PartT>::Nz;
+  const PartT* part = static_cast<const PartT*>(p.part);
   using Stage = TaskStage<IdxT, float, ITEMS>;
   using RV = RowVec<DT, VEC>;
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -253,17 +258,18 @@ __global__ void __launch_bounds__(WARPS * 32) sddmm_wide_kernel(const SddmmParam
   const int total_warps = gridDim.x * WARPS;
   uint32_t phase = 0;
   for (int k = blockIdx.x * WARPS + warp; k < p.P; k += total_warps) {
-    const int2 ps = __ldg(&p.part[k]);
-    const int2 pe = __ldg(&p.part[k + 1]);
-    const int rs = ps.x, ns = ps.y, re = pe.x, ne = pe.y;
-    const int cnt_nz = ne - ns;
+    const PartT ps = PartOf<PartT>::load(&part[k]);
+    const PartT pe = PartOf<PartT>::load(&part[k + 1]);
+    const int rs = static_cast<int>(ps.x), re = static_cast<int>(pe.x);
+    const NzT ns = ps.y;
+    const int cnt_nz = static_cast<int>(pe.y - ns);
     if (cnt_nz == 0) continue;
     const StagedTask<IdxT, float> tk = stage_task<false>(st, bar, phase, crow, col, static_cast<const float*>(nullptr),
                                                         rs, ns, re - rs + 1, cnt_nz, p.cols, lane, pol_stream);
     float* sout = st.val;
     int e = 0;
     for (int r = rs; r <= re; ++r) {
-      const int e_end = r < re ? static_cast<int>(tk.srow[r - rs + 1]) - ns : cnt_nz;
+      const int e_end = r < re ? task_rel(tk.srow[r - rs + 1], ns) : cnt_nz;
       const DT* yrow = dY + static_cast<size_t>(r) * n;
       for (int q = e; q < e_end; ++q) {
         const IdxT cq = tk.scol[q];
@@ -296,10 +302,10 @@ struct BwdAtomicParams {
   const void* val;
   const void* dY;  // rows x n
   float* acc;      // cols x n fp32 accumulator (zeroed by the caller)
-  const int2* part;
+  const void* part;  // int2 or longlong2 entries (PartOf in spmm_kernels.cuh)
   long long cols;
   int rows;
-  int nnz;
+  int reserved = 0;  // not read; keeps the parameter layout the narrow kernels were tuned with
   int n;
   int P;
 };
@@ -320,8 +326,10 @@ __device__ __forceinline__ void red_add_f32(float* p, const float (&v)[8]) {
 // acc[col[p], :] += val[p] * dY[i, :] with 16-byte vector reductions (red.global.add.v4.f32).
 // Route (2) of ofspmm_bwd_b: needs no transposed copy of A, order-nondeterministic like the
 // reference's atomic scatter (oneflow/user/kernels/unsorted_segment_sum_kernel_util.cu:96-117).
-template <typename DT, typename ValT, typename IdxT, int VEC, int LPR, int CH, int ITEMS, int WARPS>
+template <typename DT, typename ValT, typename IdxT, int VEC, int LPR, int CH, int ITEMS, int WARPS, typename PartT>
 __global__ void __launch_bounds__(WARPS * 32) bwd_atomic_kernel(const BwdAtomicParams p) {
+  using NzT = typename PartOf<PartT>::Nz;
+  const PartT* part = static_cast<const PartT*>(p.part);
   constexpr int G = 32 / LPR;
   using Stage = TaskStage<IdxT, ValT, ITEMS>;
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -353,16 +361,17 @@ __global__ void __launch_bounds__(WARPS * 32) bwd_atomic_kernel(const BwdAtomicP
   const int total_warps = gridDim.x * WARPS;
   uint32_t phase = 0;
   for (int k = blockIdx.x * WARPS + warp; k < p.P; k += total_warps) {
-    const int2 ps = __ldg(&p.part[k]);
-    const int2 pe = __ldg(&p.part[k + 1]);
-    const int rs = ps.x, ns = ps.y, re = pe.x, ne = pe.y;
-    const int cnt_nz = ne - ns;
+    const PartT ps = PartOf<PartT>::load(&part[k]);
+    const PartT pe = PartOf<PartT>::load(&part[k + 1]);
+    const int rs = static_cast<int>(ps.x), re = static_cast<int>(pe.x);
+    const NzT ns = ps.y;
+    const int cnt_nz = static_cast<int>(pe.y - ns);
     if (cnt_nz == 0) continue;
     const StagedTask<IdxT, ValT> tk = stage_task<true>(st, bar, phase, crow, col, val, rs, ns, re - rs + 1,
                                                        cnt_nz, p.cols, lane, pol_stream);
     int e = 0;
     for (int r = rs; r <= re; ++r) {
-      const int e_end = r < re ? static_cast<int>(tk.srow[r - rs + 1]) - ns : cnt_nz;
+      const int e_end = r < re ? task_rel(tk.srow[r - rs + 1], ns) : cnt_nz;
       if (e_end <= e) continue;
       float y[CH][VEC];
 #pragma unroll

@@ -51,12 +51,12 @@ struct FwdParams {
   const void* val;
   const void* B;
   void* C;
-  const int2* part;  // P+1 split points (row, nz)
+  const void* part;  // P+1 split points (row, nz): int2, or longlong2 for wide matrices (PartOf below)
   float* carry;      // P x n fp32
   float* head;       // P x n fp32 (only for non-fp32 outputs)
   long long cols;    // K
   int rows;          // M
-  int nnz;
+  int reserved = 0;  // not read; keeps the parameter layout the narrow kernels were tuned with
   int n;             // dense width
   int P;             // number of tasks
   int panels;        // column panels of LPR*VEC*CH columns each
@@ -80,6 +80,27 @@ constexpr unsigned kFwdRelu = 4u;        // max(., 0)
 // to bf16 exactly once, like a single-pass product.
 constexpr unsigned kFwdAcc32In = 32u;    // add the fp32 row of acc32 to this pass's sum
 constexpr unsigned kFwdAcc32Out = 64u;   // store the fp32 sum into acc32 instead of C (no epilogue)
+
+// Task partition entry: (first row, first non-zero) of a task.  Matrices with fewer than 2^31-1
+// non-zeros use 8-byte int2 entries; wider ones ("wide", int64 indices only) 16-byte longlong2
+// entries whose .y is the 64-bit non-zero offset (.x still holds a row < 2^31-1).  Only the task
+// start is 64-bit: everything inside a task (e0, e1, cnt_nz, crow[r] - ns) is bounded by ITEMS.
+template <typename PartT> struct PartOf;
+template <> struct PartOf<int2> {
+  using Nz = int;
+  __device__ __forceinline__ static int2 load(const int2* p) { return __ldg(p); }
+};
+template <> struct PartOf<longlong2> {
+  using Nz = long long;
+  __device__ __forceinline__ static longlong2 load(const longlong2* p) { return __ldg(p); }
+};
+
+// Position of a non-zero (a crow value) relative to the task start ns; the result is < ITEMS.
+template <typename IdxT, typename NzT>
+__device__ __forceinline__ int task_rel(IdxT v, NzT ns) {
+  if constexpr (sizeof(NzT) == 4) return static_cast<int>(v) - ns;
+  else return static_cast<int>(static_cast<long long>(v) - ns);
+}
 
 // acc (+ old C) (+ bias) (relu) for VEC consecutive columns starting at column `c0` of row `crow_ptr`.
 template <typename DT, int VEC>
@@ -153,10 +174,10 @@ struct StagedTask {
 // scans the column indices once: a task whose indices are all inside [0, cols) runs the check-free
 // vector loop; a task with an out-of-range index is flagged `dirty` and runs a per-element checked
 // loop that issues no load for such an element (so NaN / Inf in unrelated B rows cannot leak in).
-template <bool kWithVal, typename IdxT, typename ValT, int ITEMS>
+template <bool kWithVal, typename IdxT, typename ValT, int ITEMS, typename NzT>
 __device__ __forceinline__ StagedTask<IdxT, ValT> stage_task(
     TaskStage<IdxT, ValT, ITEMS>& st, uint64_t* bar, uint32_t& phase, const IdxT* __restrict__ crow,
-    const IdxT* __restrict__ col, const ValT* __restrict__ val, int rs, int ns, int cnt_row,
+    const IdxT* __restrict__ col, const ValT* __restrict__ val, int rs, NzT ns, int cnt_row,
     int cnt_nz, long long cols, int lane, uint64_t pol_stream) {
   int pre_c, head_c, body_c, pre_v = 0, head_v = 0, body_v = 0, pre_r, head_r, body_r;
   seg_plan(col + ns, cnt_nz, pre_c, head_c, body_c);
@@ -261,9 +282,11 @@ __device__ __forceinline__ uint2 lds64(uint32_t addr) {
 // kFull: n is a whole number of LPR*VEC*CH-column tiles, so no lane is ever masked and the chunk
 // offsets are immediates.  Otherwise masked chunks are pointed at column 0 (a valid address:
 // their loads are harmless duplicates) and only the stores are predicated.
-template <typename DT, typename ValT, typename IdxT, int VEC, int LPR, int CH, bool kFull, bool kRowPar, int ITEMS, int WARPS>
+template <typename DT, typename ValT, typename IdxT, int VEC, int LPR, int CH, bool kFull, bool kRowPar, int ITEMS, int WARPS,
+          typename PartT>
 __global__ void __launch_bounds__(WARPS * 32, min_ctas_per_sm<DT, CH>())
 spmm_merge_kernel(const FwdParams p) {
+  using NzT = typename PartOf<PartT>::Nz;
   constexpr int G = 32 / LPR;  // groups of lanes working on different non-zeros
   constexpr bool kF32Out = sizeof(DT) == 4;
   constexpr bool kVecIdx = sizeof(IdxT) == 4;  // 16-byte LDS path needs 4-byte indices
@@ -329,7 +352,7 @@ spmm_merge_kernel(const FwdParams p) {
     const bool more = done + 2 < max_tasks;
     if (dynamic && more && lane == 0) pending = atomicAdd(p.counter, 1u);   // read at the end of the task
     if (t1 < total && lane == 0)
-      asm volatile("prefetch.global.L2 [%0];" ::"l"(&p.part[t1 % p.P]));
+      asm volatile("prefetch.global.L2 [%0];" ::"l"(&static_cast<const PartT*>(p.part)[t1 % p.P]));
     // panel-major: all tasks of column panel 0, then panel 1, ... (keeps the B panel in L2)
     const int panel = t / p.P;
     const int k = t - panel * p.P;
@@ -349,17 +372,20 @@ spmm_merge_kernel(const FwdParams p) {
     asm volatile("" : "+l"(bl_bits));
     const char* __restrict__ Bl = reinterpret_cast<const char*>(bl_bits);
 
-    const int2 ps = __ldg(&p.part[k]);
-    const int2 pe = __ldg(&p.part[k + 1]);
-    const int rs = ps.x, ns = ps.y, re = pe.x, ne = pe.y;
-    const int cnt_nz = ne - ns;
+    const PartT ps = PartOf<PartT>::load(&static_cast<const PartT*>(p.part)[k]);
+    const PartT pe = PartOf<PartT>::load(&static_cast<const PartT*>(p.part)[k + 1]);
+    const int rs = static_cast<int>(ps.x);
+    const NzT ns = ps.y;
+    const int re = static_cast<int>(pe.x);
+    const NzT ne = pe.y;
+    const int cnt_nz = static_cast<int>(ne - ns);
     const StagedTask<IdxT, ValT> tk = stage_task<true>(st, bar, phase, crow, col, val, rs, ns, re - rs + 1,
                                                        cnt_nz, p.cols, lane, pol_stream);
     // 16-byte LDS path: index chunk and value chunk must share their alignment phase
     const bool vec_ok = kVecIdx && !tk.dirty && (((tk.pre_v - tk.pre_c) & 3) == 0);
     // value byte address of the slot that pairs with index slot 0
     const uint32_t val_s0 = val_sa + static_cast<uint32_t>((tk.pre_v - tk.pre_c) * static_cast<int>(sizeof(ValT)));
-    const bool started_earlier = static_cast<int>(tk.srow[0]) < ns;
+    const bool started_earlier = static_cast<NzT>(tk.srow[0]) < ns;
 
     // nnz-parallel (kRowPar == false): every group walks every row, chunk q of a row goes to group
     // q % G and the groups' partial rows are combined with __shfl_xor at the row end.
@@ -369,8 +395,9 @@ spmm_merge_kernel(const FwdParams p) {
     const int chunk_first = kRowPar ? 0 : grp;
     for (int r = kRowPar ? rs + grp : rs; r <= re; r += (kRowPar ? G : 1)) {
       // rows rs..re-1 end in this task; r == re is the trailing partial row (if it has elements)
-      const int e0 = r == rs ? 0 : static_cast<int>(tk.srow[r - rs]) - ns;
-      const int e1 = r < re ? static_cast<int>(tk.srow[r - rs + 1]) - ns : cnt_nz;
+      // = task_rel(), written out: the int2 instantiations then compile to the code they always had
+      const int e0 = r == rs ? 0 : static_cast<int>(static_cast<NzT>(tk.srow[r - rs]) - ns);
+      const int e1 = r < re ? static_cast<int>(static_cast<NzT>(tk.srow[r - rs + 1]) - ns) : cnt_nz;
       if (r == re && e1 <= e0) break;
 
       float acc[CH][VEC];
@@ -545,30 +572,33 @@ spmm_merge_kernel(const FwdParams p) {
 // row's final segment (a deterministic segmented reduction).  Each LANE inspects one task k: if k
 // ends a row that started in an earlier task, the lane finds the first task j of that row; the
 // warp then stitches the flagged rows one after another, all 32 lanes across the dense width.
-template <typename DT, typename IdxT, int VEC, int WARPS>
+template <typename DT, typename IdxT, int VEC, int WARPS, typename PartT>
 __global__ void __launch_bounds__(WARPS * 32) spmm_fixup_kernel(const FwdParams p) {
+  using NzT = typename PartOf<PartT>::Nz;
+  using Part = PartOf<PartT>;
+  const PartT* part = static_cast<const PartT*>(p.part);
   constexpr bool kF32Out = sizeof(DT) == 4;
   const int lane = threadIdx.x & 31;
   const int k = (blockIdx.x * WARPS + (threadIdx.x >> 5)) * 32 + lane;
   bool need = false;
   int j = 0, rs = 0;
   if (k >= 1 && k < p.P) {
-    const int2 ps = __ldg(&p.part[k]);
-    const int re = __ldg(&p.part[k + 1]).x;
+    const PartT ps = Part::load(&part[k]);
+    const int re = static_cast<int>(Part::load(&part[k + 1]).x);
     if (re > ps.x) {  // a row ends in task k
-      const int cr = static_cast<int>(static_cast<const IdxT*>(p.crow)[ps.x]);
+      const NzT cr = static_cast<NzT>(static_cast<const IdxT*>(p.crow)[ps.x]);
       if (cr < ps.y) {  // ... and it started before task k
         need = true;
-        rs = ps.x;
+        rs = static_cast<int>(ps.x);
         // first task holding a non-zero of the row = smallest j with part[j+1].y > cr
         j = k - 1;
         int steps = 0;
-        while (j > 0 && steps < 4 && __ldg(&p.part[j]).y > cr) { --j; ++steps; }
-        if (j > 0 && __ldg(&p.part[j]).y > cr) {  // hub row: finish with a binary search
+        while (j > 0 && steps < 4 && Part::load(&part[j]).y > cr) { --j; ++steps; }
+        if (j > 0 && Part::load(&part[j]).y > cr) {  // hub row: finish with a binary search
           int lo = 0, hi = j;                    // invariant: part[hi].y > cr, answer in [lo, hi)
           while (lo < hi) {
             const int mid = (lo + hi) >> 1;
-            if (__ldg(&p.part[mid + 1]).y > cr) hi = mid; else lo = mid + 1;
+            if (Part::load(&part[mid + 1]).y > cr) hi = mid; else lo = mid + 1;
           }
           j = lo;
         }
@@ -625,16 +655,17 @@ __global__ void __launch_bounds__(WARPS * 32) spmm_fixup_kernel(const FwdParams 
 }
 
 // part[k] = merge-path split of diagonal min(k*items, rows+nnz), k = 0..P.
-template <typename IdxT>
-__global__ void task_partition_kernel(const IdxT* __restrict__ crow, int rows, int nnz, int items,
-                                      int P, int2* __restrict__ part) {
+template <typename IdxT, typename PartT>
+__global__ void task_partition_kernel(const IdxT* __restrict__ crow, int rows, typename PartOf<PartT>::Nz nnz,
+                                      int items, int P, PartT* __restrict__ part) {
   const int k = blockIdx.x * blockDim.x + threadIdx.x;
   if (k > P) return;
   const long long total = static_cast<long long>(rows) + nnz;
   long long d = static_cast<long long>(k) * items;
   if (d > total) d = total;
   const long long r = merge_path_search<IdxT>(crow, rows, nnz, d);
-  part[k] = make_int2(static_cast<int>(r), static_cast<int>(d - r));
+  if constexpr (sizeof(PartT) == 8) part[k] = make_int2(static_cast<int>(r), static_cast<int>(d - r));
+  else part[k] = make_longlong2(r, d - r);
 }
 
 }  // namespace ofspmm

@@ -248,6 +248,63 @@ def upstream_grad(M: int, N: int, seed: int, device="cpu", dtype=torch.float32) 
     return torch.rand(M, N, generator=g, device=device, dtype=torch.float32).to(dtype)
 
 
+# A matrix with more non-zeros than int32 offsets can count (2^31 + 2^25, int64 indices; 26 GB on
+# the device).  Row WIDE_HUB holds 2^25 entries straddling non-zero 2^31; the rows before it are
+# ~2000 long, the rows after it ~16; every 97th row is empty and every 89th has one entry.
+WIDE_M, WIDE_K, WIDE_NNZ = 1 << 21, 1 << 20, (1 << 31) + (1 << 25)
+WIDE_HUB, WIDE_HUB_START, WIDE_HUB_LEN = 1 << 20, (1 << 31) - (1 << 24), 1 << 25
+# (position, column) of the entries outside [0, K), which every kernel skips: on both sides of 2^31
+WIDE_BAD = ((1000, -1), ((1 << 31) - 5, -1), ((1 << 31) - 3, WIDE_K), ((1 << 31) + 7, -1),
+            ((1 << 31) + 11, WIDE_K), (WIDE_NNZ - 2, WIDE_K))
+
+
+def _wide_lengths(g: torch.Generator, n: int, total: int) -> torch.Tensor:
+    idx = torch.arange(n)
+    w = torch.rand(n, generator=g, dtype=torch.float64) + 0.5
+    ones = idx % 89 == 5
+    w[(idx % 97 == 3) | ones] = 0
+    target = total - int(ones.sum())
+    lens = torch.floor(w / w.sum() * target).to(torch.int64)
+    lens[torch.nonzero(w > 0).flatten()[:target - int(lens.sum())]] += 1
+    lens[ones] = 1
+    return lens
+
+
+def _mix64_(x: torch.Tensor) -> torch.Tensor:
+    """In-place splitmix64 finaliser on int64 (wrapping products, logical shifts)."""
+    x.mul_(-7046029254386353131)
+    x.bitwise_xor_((x >> 30) & ((1 << 34) - 1))
+    x.mul_(-4658895280553007687)
+    x.bitwise_xor_((x >> 27) & ((1 << 37) - 1))
+    x.mul_(-7723592293110705685)
+    x.bitwise_xor_((x >> 31) & ((1 << 33) - 1))
+    return x
+
+
+def wide_csr(device="cuda", seed: int = 9, chunk: int = 1 << 26) -> CsrMatrix:
+    """The WIDE_* matrix built on ``device`` in chunks: column and fp32 value of non-zero p are a
+    hash of (seed, p), values k / 2^15 in [-1, 1)."""
+    g = torch.Generator().manual_seed(seed)
+    lens = torch.empty(WIDE_M, dtype=torch.int64)
+    lens[:WIDE_HUB] = _wide_lengths(g, WIDE_HUB, WIDE_HUB_START)
+    lens[WIDE_HUB] = WIDE_HUB_LEN
+    lens[WIDE_HUB + 1:] = _wide_lengths(g, WIDE_M - WIDE_HUB - 1, WIDE_NNZ - WIDE_HUB_START - WIDE_HUB_LEN)
+    crow = torch.zeros(WIDE_M + 1, dtype=torch.int64)
+    crow[1:] = torch.cumsum(lens, 0)
+    assert int(crow[-1]) == WIDE_NNZ and int(crow[WIDE_HUB]) == WIDE_HUB_START
+    col = torch.empty(WIDE_NNZ, dtype=torch.int64, device=device)
+    val = torch.empty(WIDE_NNZ, dtype=torch.float32, device=device)
+    for p0 in range(0, WIDE_NNZ, chunk):
+        p1 = min(WIDE_NNZ, p0 + chunk)
+        x = _mix64_(torch.arange(p0, p1, dtype=torch.int64, device=device).add_(seed << 48))
+        col[p0:p1] = (x >> 24) & (WIDE_K - 1)
+        val[p0:p1] = ((x & 0xFFFF) - 32768).to(torch.float32).div_(32768.0)
+        del x
+    for p, c in WIDE_BAD:
+        col[p] = c
+    return CsrMatrix(crow.to(device), col, val, WIDE_M, WIDE_K)
+
+
 def expected_alg_bytes(M: int, K: int, nnz: int, N: int, s_dense: int, s_val: int = 4,
                        s_idx: int = 4) -> dict:
     """SURVEY.md §8d: gather-model (M2) and compulsory (M1) byte counts for one SpMM."""
