@@ -14,6 +14,8 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "lib", "libofspmm_b200.so")
 
 DTYPE_FLOAT, DTYPE_INT32, DTYPE_INT64, DTYPE_BFLOAT16 = 2, 5, 6, 11
+# value dtype of a pattern matrix: every stored entry is 1.0, no values array (val must be NULL)
+VAL_UNIT = 0x100
 
 EXPORTS = (
     "ofspmm_fwd_workspace_bytes", "ofspmm_fwd", "ofspmm_fwd_strided", "ofspmm_bwd_b_workspace_bytes", "ofspmm_bwd_b",
@@ -31,6 +33,7 @@ EXPORTS = (
 
 # ofspmm_opts.flags / variant codes (include/ofspmm.h)
 FWD_ACCUMULATE, FWD_BIAS, FWD_RELU, ORDER_DYNAMIC, ORDER_STATIC, FWD_ACC32_IN, FWD_ACC32_OUT = 1, 2, 4, 8, 16, 32, 64
+FWD_MEAN = 128
 VARIANT_AUTO, VARIANT_ITEMS64, VARIANT_ROWPAR, VARIANT_ROWS, VARIANT_EXPLICIT = 0, 1, 2, 4, 0x100
 
 

@@ -50,6 +50,9 @@ bool dense_ok(int d) { return d == OFSPMM_DTYPE_FLOAT || d == OFSPMM_DTYPE_BFLOA
 bool idx_ok(int d) { return d == OFSPMM_DTYPE_INT32 || d == OFSPMM_DTYPE_INT64; }
 size_t dense_size(int d) { return d == OFSPMM_DTYPE_FLOAT ? 4 : 2; }
 size_t idx_size(int d) { return d == OFSPMM_DTYPE_INT64 ? 8 : 4; }
+// Bytes per stored value: a pattern matrix (OFSPMM_VAL_UNIT) stores none.
+size_t val_size(int d) { return d == OFSPMM_DTYPE_FLOAT ? 4 : (d == OFSPMM_VAL_UNIT ? 0 : 2); }
+bool unit(const ofspmm_csr* A) { return A->val_dtype == OFSPMM_VAL_UNIT; }
 
 // Sizes no kernel can address: rows that do not fit int, non-zeros that int32 row offsets cannot
 // count, or more 256-item tasks than the task index allows (kMaxTasks).  Wide int64 matrices are fine.
@@ -63,10 +66,12 @@ int check_csr(const ofspmm_csr* A, bool need_val) {
   if (A == nullptr) return OFSPMM_ERR_INVALID_ARG;
   if (A->rows < 0 || A->cols < 0 || A->nnz < 0) return OFSPMM_ERR_INVALID_ARG;
   if (!idx_ok(A->idx_dtype)) return OFSPMM_ERR_UNSUPPORTED_DTYPE;
-  if (A->val_dtype != OFSPMM_DTYPE_FLOAT && A->val_dtype != OFSPMM_DTYPE_BFLOAT16) return OFSPMM_ERR_UNSUPPORTED_DTYPE;
+  if (A->val_dtype != OFSPMM_DTYPE_FLOAT && A->val_dtype != OFSPMM_DTYPE_BFLOAT16 && !unit(A))
+    return OFSPMM_ERR_UNSUPPORTED_DTYPE;
   if (too_large(A->idx_dtype, A->rows, A->nnz)) return OFSPMM_ERR_TOO_LARGE;
   if (A->crow == nullptr) return OFSPMM_ERR_INVALID_ARG;
-  if (A->nnz > 0 && (A->col == nullptr || (need_val && A->val == nullptr))) return OFSPMM_ERR_INVALID_ARG;
+  if (unit(A) && A->val != nullptr) return OFSPMM_ERR_INVALID_ARG;  // a values array with the pattern dtype
+  if (A->nnz > 0 && (A->col == nullptr || (need_val && !unit(A) && A->val == nullptr))) return OFSPMM_ERR_INVALID_ARG;
   return OFSPMM_OK;
 }
 
@@ -103,7 +108,8 @@ FwdLaunch make_launch(const ofspmm_opts* opts, int64_t rows, int64_t nnz, int64_
   // task order: dynamic (drawn from a counter) unless the caller pins the static interleave
   L.dynamic = OFSPMM_DEFAULT_DYNAMIC_ORDER ? (fl & OFSPMM_ORDER_STATIC) == 0 : (fl & OFSPMM_ORDER_DYNAMIC) != 0;
   L.wide = wide_nnz(nnz);
-  L.flags = fl & (OFSPMM_FWD_ACCUMULATE | OFSPMM_FWD_BIAS | OFSPMM_FWD_RELU | OFSPMM_FWD_ACC32_IN | OFSPMM_FWD_ACC32_OUT);
+  L.flags = fl & (OFSPMM_FWD_ACCUMULATE | OFSPMM_FWD_BIAS | OFSPMM_FWD_RELU | OFSPMM_FWD_ACC32_IN | OFSPMM_FWD_ACC32_OUT |
+                 OFSPMM_FWD_MEAN);
   L.bias = opts ? opts->bias : nullptr;
   L.acc32 = opts ? static_cast<float*>(opts->acc32) : nullptr;
   return L;
@@ -112,6 +118,11 @@ FwdLaunch make_launch(const ofspmm_opts* opts, int64_t rows, int64_t nnz, int64_
 // C = A·B through the merge-path kernels; shared by every forward-shaped entry point.
 int run_fwd(const ofspmm_csr* A, const void* B, int64_t ldb, void* C, int64_t ldc, int64_t n,
             int dense_dtype, const ofspmm_opts* opts, void* ws, size_t ws_bytes, cudaStream_t stream) {
+  // the mean divides this call's complete row sum: with an accumulated C (or fp32 row sums carried
+  // between passes) the division would also apply to what earlier passes added
+  if (opts != nullptr && (opts->flags & OFSPMM_FWD_MEAN) &&
+      (opts->flags & (OFSPMM_FWD_ACCUMULATE | OFSPMM_FWD_ACC32_IN | OFSPMM_FWD_ACC32_OUT)))
+    return OFSPMM_ERR_INVALID_ARG;
   if (A->rows == 0 || n == 0) return OFSPMM_OK;
   if (ldb < n || ldc < n || ldb >= (int64_t{1} << 30)) return OFSPMM_ERR_INVALID_ARG;
   FwdLaunch L = make_launch(opts, A->rows, A->nnz, n, dense_dtype);
@@ -123,8 +134,10 @@ int run_fwd(const ofspmm_csr* A, const void* B, int64_t ldb, void* C, int64_t ld
       return OFSPMM_ERR_INVALID_ARG;
   }
   if (A->nnz == 0 || A->cols == 0) {
-    if (L.flags == OFSPMM_FWD_ACCUMULATE || L.flags == (OFSPMM_FWD_ACC32_IN | OFSPMM_FWD_ACC32_OUT)) return OFSPMM_OK;  // += 0
-    if (L.flags == 0) {
+    // every row sum is 0, and so is its mean: MEAN changes nothing here
+    const unsigned fl = L.flags & ~static_cast<unsigned>(OFSPMM_FWD_MEAN);
+    if (fl == OFSPMM_FWD_ACCUMULATE || fl == (OFSPMM_FWD_ACC32_IN | OFSPMM_FWD_ACC32_OUT)) return OFSPMM_OK;  // += 0
+    if (fl == 0) {
       OFSPMM_CUDA_OK(cudaMemset2DAsync(C, static_cast<size_t>(ldc) * dense_size(dense_dtype), 0,
                                        static_cast<size_t>(n) * dense_size(dense_dtype),
                                        static_cast<size_t>(A->rows), stream));
@@ -296,11 +309,11 @@ struct TransientLayout {
 TransientLayout transient_layout(int64_t rows, int64_t cols, int64_t nnz, int64_t n, int dense_dtype,
                                  int idx_dtype, int val_dtype) {
   TransientLayout L;
-  const size_t is = idx_size(idx_dtype), vs = val_dtype == OFSPMM_DTYPE_FLOAT ? 4 : 2;
+  const size_t is = idx_size(idx_dtype), vs = val_size(val_dtype);
   size_t off = 0;
   L.t_crow = off; off += align_up(static_cast<size_t>(cols + 1) * is, 256);
   L.t_col = off;  off += align_up(static_cast<size_t>(nnz > 0 ? nnz : 1) * is, 256);
-  L.t_val = off;  off += align_up(static_cast<size_t>(nnz > 0 ? nnz : 1) * vs, 256);
+  L.t_val = off;  off += align_up(static_cast<size_t>(nnz > 0 ? nnz : 1) * vs, 256);  // 0 for a pattern matrix
   L.tws = off;    L.tws_bytes = transpose_workspace_bytes(rows, cols, nnz, idx_dtype);
   off += align_up(L.tws_bytes, 256);
   L.fws = off;    off += fwd_ws_auto(cols, nnz, n, dense_dtype);
@@ -330,20 +343,21 @@ int ofspmm_bwd_b_transient(const ofspmm_csr* A, const void* dY, void* dB, int64_
   const TransientLayout L = transient_layout(A->rows, A->cols, A->nnz, n, dense_dtype, A->idx_dtype, A->val_dtype);
   if (int rc = check_ws(workspace, workspace_bytes, L.total)) return rc;
   unsigned char* w = static_cast<unsigned char*>(workspace);
-  if (int rc = launch_transpose(A, w + L.t_crow, w + L.t_col, w + L.t_val, nullptr, w + L.tws, L.tws_bytes, stream)) return rc;
+  void* t_val = unit(A) ? nullptr : w + L.t_val;  // a pattern A^T has no values to build
+  if (int rc = launch_transpose(A, w + L.t_crow, w + L.t_col, t_val, nullptr, w + L.tws, L.tws_bytes, stream)) return rc;
   ofspmm_csr At = *A;
   At.rows = A->cols;
   At.cols = A->rows;
   At.crow = w + L.t_crow;
   At.col = w + L.t_col;
-  At.val = w + L.t_val;
+  At.val = t_val;
   return run_fwd(&At, dY, n, dB, n, n, dense_dtype, nullptr, w + L.fws, workspace_bytes - L.fws, stream);
 }
 
 size_t ofspmm_bwd_b_cached_workspace_bytes(int64_t rows, int64_t cols, int64_t nnz, int64_t n, int dense_dtype,
                                           int val_dtype) {
   if (rows < 0 || cols < 0 || nnz < 0 || n < 0) return 0;
-  const size_t vs = val_dtype == OFSPMM_DTYPE_FLOAT ? 4 : 2;
+  const size_t vs = val_size(val_dtype);
   return align_up(static_cast<size_t>(nnz > 0 ? nnz : 1) * vs, 256) + fwd_ws_auto(cols, nnz, n, dense_dtype);
 }
 
@@ -357,20 +371,21 @@ int ofspmm_bwd_b_cached(const ofspmm_csr* A, const void* t_crow, const void* t_c
   if (A->cols == 0 || n == 0) return OFSPMM_OK;
   if (dB == nullptr || t_crow == nullptr || (A->nnz > 0 && (dY == nullptr || t_col == nullptr || t_perm == nullptr)))
     return OFSPMM_ERR_INVALID_ARG;
-  const size_t vs = A->val_dtype == OFSPMM_DTYPE_FLOAT ? 4 : 2;
-  const size_t tv_bytes = align_up(static_cast<size_t>(A->nnz > 0 ? A->nnz : 1) * vs, 256);
+  const size_t tv_bytes = align_up(static_cast<size_t>(A->nnz > 0 ? A->nnz : 1) * val_size(A->val_dtype), 256);
   const size_t need = ofspmm_bwd_b_cached_workspace_bytes(A->rows, A->cols, A->nnz, n, dense_dtype, A->val_dtype);
   if (int rc = check_ws(workspace, workspace_bytes, need)) return rc;
   unsigned char* w = static_cast<unsigned char*>(workspace);
   // the STRUCTURE of A^T is cached by the caller; the values are re-gathered from A on every call,
-  // so in-place updates of a_val (learnable edge weights) are always seen
-  if (int rc = launch_gather_vals(A->val, A->val_dtype, t_perm, A->idx_dtype, A->nnz, w, stream)) return rc;
+  // so in-place updates of a_val (learnable edge weights) are always seen.  A pattern matrix has
+  // nothing to gather.
+  if (!unit(A))
+    if (int rc = launch_gather_vals(A->val, A->val_dtype, t_perm, A->idx_dtype, A->nnz, w, stream)) return rc;
   ofspmm_csr At = *A;
   At.rows = A->cols;
   At.cols = A->rows;
   At.crow = t_crow;
   At.col = t_col;
-  At.val = w;
+  At.val = unit(A) ? nullptr : w;
   return run_fwd(&At, dY, n, dB, n, n, dense_dtype, opts, w + tv_bytes, workspace_bytes - tv_bytes, stream);
 }
 
@@ -489,6 +504,8 @@ int ofspmm_sddmm(const ofspmm_csr* A, const void* dY, const void* B, void* dval,
 int ofspmm_sddmm_ex(const ofspmm_csr* A, const void* dY, const void* B, void* dval, int64_t n, int dense_dtype,
                     const ofspmm_opts* opts, void* workspace, size_t workspace_bytes, ofspmm_stream_t stream_) {
   cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+  // val_dtype is the dtype of the output dval here: a pattern matrix has no values to differentiate
+  if (A != nullptr && unit(A)) return OFSPMM_ERR_UNSUPPORTED_DTYPE;
   if (int rc = check_csr(A, false)) return rc;
   if (int rc = check_dtypes(A, dense_dtype)) return rc;
   if (n < 0 || n >= (int64_t{1} << 31)) return OFSPMM_ERR_INVALID_ARG;
@@ -557,6 +574,7 @@ int ofspmm_csr_transpose(const ofspmm_csr* A, void* t_crow, void* t_col, void* t
                          void* workspace, size_t workspace_bytes, ofspmm_stream_t stream) {
   if (int rc = check_csr(A, false)) return rc;
   if (t_crow == nullptr || (A->nnz > 0 && t_col == nullptr)) return OFSPMM_ERR_INVALID_ARG;
+  if (unit(A) && t_val != nullptr) return OFSPMM_ERR_INVALID_ARG;  // a pattern A^T has no values
   return launch_transpose(A, t_crow, t_col, t_val, t_perm, workspace, workspace_bytes,
                           reinterpret_cast<cudaStream_t>(stream));
 }
@@ -564,7 +582,7 @@ int ofspmm_csr_transpose(const ofspmm_csr* A, void* t_crow, void* t_col, void* t
 size_t ofspmm_fwd_host_workspace_bytes(int64_t rows, int64_t cols, int64_t nnz, int64_t n, int dense_dtype,
                                        int idx_dtype, int val_dtype) {
   if (rows < 0 || cols < 0 || nnz < 0 || n < 0) return 0;
-  const size_t vs = val_dtype == OFSPMM_DTYPE_FLOAT ? 4 : 2;
+  const size_t vs = val_size(val_dtype);
   size_t total = 0;
   total += align_up(static_cast<size_t>(rows + 1) * idx_size(idx_dtype), 256);
   total += align_up(static_cast<size_t>(nnz) * idx_size(idx_dtype), 256);
@@ -586,7 +604,7 @@ int ofspmm_fwd_host(const ofspmm_csr* Ah, const void* B_host, void* C_host, int6
   const size_t need = ofspmm_fwd_host_workspace_bytes(Ah->rows, Ah->cols, Ah->nnz, n, dense_dtype,
                                                       Ah->idx_dtype, Ah->val_dtype);
   if (int rc = check_ws(workspace, workspace_bytes, need)) return rc;
-  const size_t is = idx_size(Ah->idx_dtype), vs = Ah->val_dtype == OFSPMM_DTYPE_FLOAT ? 4 : 2;
+  const size_t is = idx_size(Ah->idx_dtype), vs = val_size(Ah->val_dtype);
   const size_t ds = dense_size(dense_dtype);
   unsigned char* w = static_cast<unsigned char*>(workspace);
   size_t off = 0;
@@ -599,14 +617,15 @@ int ofspmm_fwd_host(const ofspmm_csr* Ah, const void* B_host, void* C_host, int6
   OFSPMM_CUDA_OK(cudaMemcpyAsync(d_crow, Ah->crow, static_cast<size_t>(Ah->rows + 1) * is, cudaMemcpyHostToDevice, stream));
   if (Ah->nnz > 0) {
     OFSPMM_CUDA_OK(cudaMemcpyAsync(d_col, Ah->col, static_cast<size_t>(Ah->nnz) * is, cudaMemcpyHostToDevice, stream));
-    OFSPMM_CUDA_OK(cudaMemcpyAsync(d_val, Ah->val, static_cast<size_t>(Ah->nnz) * vs, cudaMemcpyHostToDevice, stream));
+    if (!unit(Ah))
+      OFSPMM_CUDA_OK(cudaMemcpyAsync(d_val, Ah->val, static_cast<size_t>(Ah->nnz) * vs, cudaMemcpyHostToDevice, stream));
   }
   if (Ah->cols > 0 && B_host != nullptr)
     OFSPMM_CUDA_OK(cudaMemcpyAsync(d_B, B_host, static_cast<size_t>(Ah->cols) * n * ds, cudaMemcpyHostToDevice, stream));
   ofspmm_csr Ad = *Ah;
   Ad.crow = d_crow;
   Ad.col = d_col;
-  Ad.val = d_val;
+  Ad.val = unit(Ah) ? nullptr : d_val;
   if (int rc = run_fwd(&Ad, d_B, n, d_C, n, n, dense_dtype, nullptr, w + off, workspace_bytes - off, stream)) return rc;
   OFSPMM_CUDA_OK(cudaMemcpyAsync(C_host, d_C, static_cast<size_t>(Ah->rows) * n * ds, cudaMemcpyDeviceToHost, stream));
   return OFSPMM_OK;

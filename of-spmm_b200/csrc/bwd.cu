@@ -53,6 +53,10 @@ int launch_idx(const BwdAtomicParams& p, int dense_dtype, int val_dtype, bool al
     return launch_typed<__nv_bfloat16, float, IdxT, PartT>(p, aligned, stream);
   if (dense_dtype == OFSPMM_DTYPE_BFLOAT16 && val_dtype == OFSPMM_DTYPE_BFLOAT16)
     return launch_typed<__nv_bfloat16, __nv_bfloat16, IdxT, PartT>(p, aligned, stream);
+  if (dense_dtype == OFSPMM_DTYPE_FLOAT && val_dtype == OFSPMM_VAL_UNIT)
+    return launch_typed<float, UnitVal, IdxT, PartT>(p, aligned, stream);
+  if (dense_dtype == OFSPMM_DTYPE_BFLOAT16 && val_dtype == OFSPMM_VAL_UNIT)
+    return launch_typed<__nv_bfloat16, UnitVal, IdxT, PartT>(p, aligned, stream);
   return OFSPMM_ERR_UNSUPPORTED_DTYPE;
 }
 

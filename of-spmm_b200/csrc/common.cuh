@@ -5,6 +5,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <type_traits>
+
 namespace ofspmm {
 
 // ---------------------------------------------------------------- shared-memory / mbarrier / TMA
@@ -70,6 +72,18 @@ __device__ __forceinline__ void tma_bulk_g2s(void* dst_smem, const void* src_gme
 
 __device__ __forceinline__ float to_float(float v) { return v; }
 __device__ __forceinline__ float to_float(__nv_bfloat16 v) { return __bfloat162float(v); }
+
+// Value type of a pattern matrix (OFSPMM_VAL_UNIT): every stored entry is 1.0 and nothing is
+// stored, staged or loaded for it.  One more ValT of the product kernels, beside float and bf16.
+struct UnitVal {};
+template <typename ValT> constexpr bool kIsUnit = std::is_same<ValT, UnitVal>::value;
+
+// Value i of a value array as fp32 (1.0 for a pattern matrix, whose array pointer is null).
+template <typename ValT, typename I>
+__device__ __forceinline__ float val_at(const ValT* v, I i) {
+  if constexpr (kIsUnit<ValT>) return 1.f;
+  else return to_float(v[i]);
+}
 
 template <typename T> __device__ __forceinline__ T from_float(float v);
 template <> __device__ __forceinline__ float from_float<float>(float v) { return v; }

@@ -107,6 +107,10 @@ int launch_idx(const FwdParams& p, int dense_dtype, int val_dtype, bool aligned,
     return launch_typed<__nv_bfloat16, float, IdxT, PartT, kRowPar, ITEMS>(p, aligned, L, stream);
   if (dense_dtype == OFSPMM_DTYPE_BFLOAT16 && val_dtype == OFSPMM_DTYPE_BFLOAT16)
     return launch_typed<__nv_bfloat16, __nv_bfloat16, IdxT, PartT, kRowPar, ITEMS>(p, aligned, L, stream);
+  if (dense_dtype == OFSPMM_DTYPE_FLOAT && val_dtype == OFSPMM_VAL_UNIT)
+    return launch_typed<float, UnitVal, IdxT, PartT, kRowPar, ITEMS>(p, aligned, L, stream);
+  if (dense_dtype == OFSPMM_DTYPE_BFLOAT16 && val_dtype == OFSPMM_VAL_UNIT)
+    return launch_typed<__nv_bfloat16, UnitVal, IdxT, PartT, kRowPar, ITEMS>(p, aligned, L, stream);
   return OFSPMM_ERR_UNSUPPORTED_DTYPE;
 }
 

@@ -35,6 +35,8 @@ int launch_family_rows(const FwdParams& p, int dense_dtype, int val_dtype, cudaS
   if (dense_dtype == OFSPMM_DTYPE_BFLOAT16 && val_dtype == OFSPMM_DTYPE_FLOAT) return launch_rows_typed<__nv_bfloat16, float>(p, stream);
   if (dense_dtype == OFSPMM_DTYPE_BFLOAT16 && val_dtype == OFSPMM_DTYPE_BFLOAT16)
     return launch_rows_typed<__nv_bfloat16, __nv_bfloat16>(p, stream);
+  if (dense_dtype == OFSPMM_DTYPE_FLOAT && val_dtype == OFSPMM_VAL_UNIT) return launch_rows_typed<float, UnitVal>(p, stream);
+  if (dense_dtype == OFSPMM_DTYPE_BFLOAT16 && val_dtype == OFSPMM_VAL_UNIT) return launch_rows_typed<__nv_bfloat16, UnitVal>(p, stream);
   return OFSPMM_ERR_UNSUPPORTED_DTYPE;
 }
 

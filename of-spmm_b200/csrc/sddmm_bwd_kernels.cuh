@@ -367,8 +367,8 @@ __global__ void __launch_bounds__(WARPS * 32) bwd_atomic_kernel(const BwdAtomicP
     const NzT ns = ps.y;
     const int cnt_nz = static_cast<int>(pe.y - ns);
     if (cnt_nz == 0) continue;
-    const StagedTask<IdxT, ValT> tk = stage_task<true>(st, bar, phase, crow, col, val, rs, ns, re - rs + 1,
-                                                       cnt_nz, p.cols, lane, pol_stream);
+    const StagedTask<IdxT, ValT> tk = stage_task<!kIsUnit<ValT>>(st, bar, phase, crow, col, val, rs, ns, re - rs + 1,
+                                                                 cnt_nz, p.cols, lane, pol_stream);
     int e = 0;
     for (int r = rs; r <= re; ++r) {
       const int e_end = r < re ? task_rel(tk.srow[r - rs + 1], ns) : cnt_nz;
@@ -380,7 +380,7 @@ __global__ void __launch_bounds__(WARPS * 32) bwd_atomic_kernel(const BwdAtomicP
       for (int q = e + grp; q < e_end; q += G) {
         const IdxT c = tk.scol[q];
         if (static_cast<unsigned long long>(c) >= static_cast<unsigned long long>(p.cols)) continue;  // skipped
-        const float v = to_float(tk.sval[q]);
+        const float v = val_at(tk.sval, q);
         float* dst = accl + static_cast<size_t>(c) * n;
 #pragma unroll
         for (int ch = 0; ch < CH; ++ch)

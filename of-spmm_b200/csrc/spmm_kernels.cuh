@@ -80,6 +80,11 @@ constexpr unsigned kFwdRelu = 4u;        // max(., 0)
 // to bf16 exactly once, like a single-pass product.
 constexpr unsigned kFwdAcc32In = 32u;    // add the fp32 row of acc32 to this pass's sum
 constexpr unsigned kFwdAcc32Out = 64u;   // store the fp32 sum into acc32 instead of C (no epilogue)
+// Mean aggregation: the complete row sum is divided by the row's stored-entry count, first thing in
+// the epilogue.  Never combined with kFwdAccumulate / kFwdAcc32* (rejected in api.cu): for fp32
+// rows stitched from several tasks the merge kernel folds the old C into the final segment before
+// the fix-up adds the carries, so a division in the fix-up would divide the old C as well.
+constexpr unsigned kFwdMean = 128u;
 
 // Task partition entry: (first row, first non-zero) of a task.  Matrices with fewer than 2^31-1
 // non-zeros use 8-byte int2 entries; wider ones ("wide", int64 indices only) 16-byte longlong2
@@ -102,10 +107,26 @@ __device__ __forceinline__ int task_rel(IdxT v, NzT ns) {
   else return static_cast<int>(static_cast<long long>(v) - ns);
 }
 
-// acc (+ old C) (+ bias) (relu) for VEC consecutive columns starting at column `c0` of row `crow_ptr`.
+// 1 / d for a row count d >= 1 without the slow-path subroutine call of the IEEE division (that
+// call site costs registers, and spills, in every kernel carrying the epilogue, mean or not):
+// reciprocal estimate refined by one Newton step.  The mean is sum * (1/d): within 1.5 ulp of the
+// correctly rounded quotient.
+__device__ __forceinline__ float recip_count(float d) {
+  float r;
+  asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(d));
+  return fmaf(fmaf(-d, r, 1.f), r, r);
+}
+
+// acc (/ len) (+ old C) (+ bias) (relu) for VEC consecutive columns starting at column `c0` of a
+// row with `len` stored entries (read only for kFwdMean; an empty row keeps its sum of 0).
 template <typename DT, int VEC>
 __device__ __forceinline__ void row_epilogue(float (&acc)[VEC], const DT* c_old, const void* bias, int c0,
-                                             unsigned flags, bool add_old) {
+                                             unsigned flags, bool add_old, float len) {
+  if ((flags & kFwdMean) && len > 0.f) {
+    const float inv = recip_count(len);
+#pragma unroll
+    for (int i = 0; i < VEC; ++i) acc[i] *= inv;
+  }
   if (add_old) {
     float o[VEC];
     RowVec<DT, VEC>::load(c_old, o);
@@ -132,6 +153,20 @@ struct alignas(16) TaskStage {
   IdxT crow[ITEMS + 2 * kPadI];
   ValT val[ITEMS + kPadV];
 };
+// A pattern matrix stages no values.
+template <typename IdxT, int ITEMS>
+struct alignas(16) TaskStage<IdxT, UnitVal, ITEMS> {
+  static constexpr int kPadI = 2 * (16 / sizeof(IdxT));
+  IdxT col[ITEMS + kPadI];
+  IdxT crow[ITEMS + 2 * kPadI];
+};
+
+// Shared-memory address of the staged values (0 for a pattern matrix, which stages none).
+template <typename IdxT, typename ValT, int ITEMS>
+__device__ __forceinline__ uint32_t staged_val_addr(TaskStage<IdxT, ValT, ITEMS>& st) {
+  if constexpr (kIsUnit<ValT>) return 0u;
+  else return smem_u32(st.val);
+}
 
 // Where element e of a `count`-element global slice starting at `src` lands in the staging array
 // (dst[pre + e]) and which part of it is a 16-byte aligned body a TMA bulk copy can move.
@@ -193,7 +228,9 @@ __device__ __forceinline__ StagedTask<IdxT, ValT> stage_task(
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     mbar_arrive_expect_tx(bar, tx);
     if (body_c) tma_bulk_g2s(st.col + pre_c + head_c, col + ns + head_c, body_c * sizeof(IdxT), bar, pol_stream);
-    if (kWithVal && body_v) tma_bulk_g2s(st.val + pre_v + head_v, val + ns + head_v, body_v * sizeof(ValT), bar, pol_stream);
+    if constexpr (kWithVal) {
+      if (body_v) tma_bulk_g2s(st.val + pre_v + head_v, val + ns + head_v, body_v * sizeof(ValT), bar, pol_stream);
+    }
     if (body_r) tma_bulk_g2s(st.crow + pre_r + head_r, crow + rs + head_r, body_r * sizeof(IdxT), bar, pol_stream);
   }
   seg_copy_edges(st.col, col + ns, cnt_nz, pre_c, head_c, body_c, lane);
@@ -222,7 +259,8 @@ __device__ __forceinline__ StagedTask<IdxT, ValT> stage_task(
   t.badmask = badmask;
   t.dirty = dirty;
   t.scol = st.col + pre_c;
-  t.sval = st.val + pre_v;
+  if constexpr (kIsUnit<ValT>) t.sval = nullptr;
+  else t.sval = st.val + pre_v;
   t.srow = st.crow + pre_r;
   t.pre_c = pre_c;
   t.pre_v = pre_v;
@@ -291,6 +329,7 @@ spmm_merge_kernel(const FwdParams p) {
   constexpr bool kF32Out = sizeof(DT) == 4;
   constexpr bool kVecIdx = sizeof(IdxT) == 4;  // 16-byte LDS path needs 4-byte indices
   constexpr uint32_t kChunkBytes = LPR * VEC * sizeof(DT);
+  constexpr bool kUnit = kIsUnit<ValT>;  // pattern matrix: no value stream, every value is 1
   using Stage = TaskStage<IdxT, ValT, ITEMS>;
   using RV = RowVec<DT, VEC>;
 
@@ -305,7 +344,7 @@ spmm_merge_kernel(const FwdParams p) {
   Stage& st = stages[warp];
   uint64_t* bar = &bars[warp];
   const uint32_t col_sa = smem_u32(st.col);
-  const uint32_t val_sa = smem_u32(st.val);
+  const uint32_t val_sa = staged_val_addr(st);
 
   if (lane == 0) mbar_init(bar, 1);
   fence_mbar_init();
@@ -379,10 +418,10 @@ spmm_merge_kernel(const FwdParams p) {
     const int re = static_cast<int>(pe.x);
     const NzT ne = pe.y;
     const int cnt_nz = static_cast<int>(ne - ns);
-    const StagedTask<IdxT, ValT> tk = stage_task<true>(st, bar, phase, crow, col, val, rs, ns, re - rs + 1,
-                                                       cnt_nz, p.cols, lane, pol_stream);
+    const StagedTask<IdxT, ValT> tk = stage_task<!kUnit>(st, bar, phase, crow, col, val, rs, ns, re - rs + 1,
+                                                         cnt_nz, p.cols, lane, pol_stream);
     // 16-byte LDS path: index chunk and value chunk must share their alignment phase
-    const bool vec_ok = kVecIdx && !tk.dirty && (((tk.pre_v - tk.pre_c) & 3) == 0);
+    const bool vec_ok = kVecIdx && !tk.dirty && (kUnit || (((tk.pre_v - tk.pre_c) & 3) == 0));
     // value byte address of the slot that pairs with index slot 0
     const uint32_t val_s0 = val_sa + static_cast<uint32_t>((tk.pre_v - tk.pre_c) * static_cast<int>(sizeof(ValT)));
     const bool started_earlier = static_cast<NzT>(tk.srow[0]) < ns;
@@ -409,13 +448,17 @@ spmm_merge_kernel(const FwdParams p) {
       if (vec_ok) {
         // slots s = pre_c + e.  The row's elements are read as 16-byte chunks of 4 slots; the
         // first / last chunk may contain slots of neighbouring rows (or staging padding), which
-        // are masked: no load is issued and the value is forced to 0.
+        // are masked: no load is issued and the value is forced to 0 (also for a pattern matrix,
+        // whose value is otherwise 1).
         const int s0 = tk.pre_c + e0, s1 = tk.pre_c + e1;
         const int cbase = s0 & ~3;
         const int nchunks = s1 > s0 ? ((s1 + 3) >> 2) - (s0 >> 2) : 0;
         auto load_vals = [&](int sa, float (&v4)[4]) {
           const uint32_t va = val_s0 + static_cast<uint32_t>(sa) * static_cast<uint32_t>(sizeof(ValT));
-          if constexpr (sizeof(ValT) == 4) {
+          if constexpr (kUnit) {
+            (void)va;
+            v4[0] = v4[1] = v4[2] = v4[3] = 1.f;
+          } else if constexpr (sizeof(ValT) == 4) {
             const uint4 w = lds128(va);
             v4[0] = __uint_as_float(w.x); v4[1] = __uint_as_float(w.y);
             v4[2] = __uint_as_float(w.z); v4[3] = __uint_as_float(w.w);
@@ -476,7 +519,10 @@ spmm_merge_kernel(const FwdParams p) {
               ca += 16u * kChunkStride;
               if (ca < cend) cn = lds128(ca);  // next chunk's indices, while the gathers fly
               float v4[4];
-              if constexpr (sizeof(ValT) == 4) {
+              if constexpr (kUnit) {
+                (void)va;
+                v4[0] = v4[1] = v4[2] = v4[3] = 1.f;
+              } else if constexpr (sizeof(ValT) == 4) {
                 const uint4 w = lds128(va);
                 v4[0] = __uint_as_float(w.x); v4[1] = __uint_as_float(w.y);
                 v4[2] = __uint_as_float(w.z); v4[3] = __uint_as_float(w.w);
@@ -497,7 +543,7 @@ spmm_merge_kernel(const FwdParams p) {
         for (int el = e0 + chunk_first; el < e1; el += kChunkStride) {
           const IdxT c = tk.scol[el];
           if (static_cast<unsigned long long>(c) >= static_cast<unsigned long long>(p.cols)) continue;
-          const float v = to_float(tk.sval[el]);
+          const float v = val_at(tk.sval, el);
           const char* brow = Bl + row_offset(c, row_bytes);
 #pragma unroll
           for (int ch = 0; ch < CH; ++ch)
@@ -555,7 +601,7 @@ spmm_merge_kernel(const FwdParams p) {
             for (int ch = 0; ch < CH; ++ch)
               if (chmask & (1u << ch))
                 row_epilogue<DT, VEC>(acc[ch], dst + ch * LPR * VEC, p.bias, col0 + ch * LPR * VEC, fl,
-                                      (p.flags & kFwdAccumulate) != 0);
+                                      (p.flags & kFwdAccumulate) != 0, static_cast<float>(e1 - e0));
           }
 #pragma unroll
           for (int ch = 0; ch < CH; ++ch)
@@ -647,8 +693,12 @@ __global__ void __launch_bounds__(WARPS * 32) spmm_fixup_kernel(const FwdParams 
           }
         }
       }
-      if (p.flags != 0)
-        row_epilogue<DT, VEC>(sum, crow_out + c0, p.bias, c0, p.flags, !kF32Out && (p.flags & kFwdAccumulate) != 0);
+      if (p.flags != 0) {
+        const IdxT* crow_in = static_cast<const IdxT*>(p.crow);
+        const float len = (p.flags & kFwdMean) ? static_cast<float>(static_cast<long long>(crow_in[row + 1]) -
+                                                                    static_cast<long long>(crow_in[row])) : 0.f;
+        row_epilogue<DT, VEC>(sum, crow_out + c0, p.bias, c0, p.flags, !kF32Out && (p.flags & kFwdAccumulate) != 0, len);
+      }
       RowVec<DT, VEC>::store_stream(crow_out + c0, sum);
     }
   }

@@ -61,7 +61,7 @@ spmm_rows_kernel(const FwdParams p) {
       const int cc = __ldg(col + beg + e);
       if (static_cast<unsigned long long>(static_cast<long long>(cc)) < cols) {
         c = cc;
-        v = to_float(val[beg + e]);
+        v = val_at(val, beg + e);
       }
     }
     const int steps = min(LPR, maxlen - base);
@@ -73,7 +73,8 @@ spmm_rows_kernel(const FwdParams p) {
       for (int u = 0; u < 4; ++u) {
         // j + u < LPR always (LPR is a multiple of 4); entries past `steps` carry c = -1 anyway
         cj[u] = __shfl_sync(0xffffffffu, c, grp * LPR + j + u);
-        vj[u] = __shfl_sync(0xffffffffu, v, grp * LPR + j + u);
+        // a pattern matrix's value is 1 wherever something is gathered (cj >= 0): nothing to send
+        vj[u] = kIsUnit<ValT> ? 1.f : __shfl_sync(0xffffffffu, v, grp * LPR + j + u);
       }
 #pragma unroll
       for (int u = 0; u < 4; ++u) {
@@ -103,7 +104,7 @@ spmm_rows_kernel(const FwdParams p) {
       }
     }
   }
-  if (p.flags != 0) row_epilogue<DT, VEC>(acc, dst, p.bias, c0, p.flags, (p.flags & kFwdAccumulate) != 0);
+  if (p.flags != 0) row_epilogue<DT, VEC>(acc, dst, p.bias, c0, p.flags, (p.flags & kFwdAccumulate) != 0, static_cast<float>(len));
   RV::store_stream(dst, acc);
 }
 

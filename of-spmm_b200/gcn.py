@@ -80,6 +80,57 @@ class GCNConv:
         return torch.relu(out) if relu else out
 
 
+class SAGEConv:
+    """GraphSAGE layer with the mean aggregator
+
+        out = act(mean_{j∈N(i)} x_j · W_neigh + x_i · W_root + bias)
+
+    on the PATTERN matrix of the graph (``A.crow``, ``A.col``; ``A.val`` is never read): the
+    aggregation is ``spmm_csr(a_val=None, reduce="mean")``, so no values tensor exists anywhere.
+    Rows of A are the destination nodes; their root features are the first ``A.rows`` rows of X.
+
+    * **Ordering by width**, as in ``GCNConv``: the aggregation runs at the narrower width.
+      ``multiply first`` (out_dim ≤ in_dim): mean(X·W_neigh); ``aggregate first``: mean(X)·W_neigh.
+    * The root term is added with ``torch.addmm``.  The mean cannot accumulate into an existing
+      output (the division would apply to it too), so the SpMM epilogue fuses only the bias, and
+      only when there is no activation and the aggregation comes last (multiply first).
+    * An isolated node (empty row) aggregates to 0 and keeps its root term.
+
+    ``kernels``: None = the C ABI (``functional.OpsKernels``); the CPU tests inject a stand-in."""
+
+    def __init__(self, in_dim: int, out_dim: int, bias: bool = True, activation: Optional[str] = "relu",
+                 order: str = "auto", seed: int = 0, device="cuda", dtype=torch.float32, kernels=None):
+        assert activation in (None, "relu") and order in ("auto", "multiply_first", "aggregate_first")
+        self.in_dim, self.out_dim, self.activation = in_dim, out_dim, activation
+        self.multiply_first = order == "multiply_first" or (order == "auto" and out_dim <= in_dim)
+        self.weight_neigh = glorot(in_dim, out_dim, seed, device, dtype).requires_grad_(True)
+        self.weight_root = glorot(in_dim, out_dim, seed + 1, device, dtype).requires_grad_(True)
+        self.bias = torch.zeros(out_dim, device=device, dtype=dtype).requires_grad_(True) if bias else None
+        self.kernels = kernels
+
+    def parameters(self):
+        return [p for p in (self.weight_neigh, self.weight_root, self.bias) if p is not None]
+
+    def aggregation_width(self) -> int:
+        return self.out_dim if self.multiply_first else self.in_dim
+
+    def __call__(self, A: CsrMatrix, X: torch.Tensor, state: Optional[SpmmOpKernelState] = None) -> torch.Tensor:
+        from .functional import spmm_csr_bias_act
+        fuse_bias = self.bias if (self.multiply_first and self.activation is None) else None
+        if self.multiply_first:
+            z = (X @ self.weight_neigh).contiguous()
+            h = spmm_csr_bias_act(A.crow, A.col, None, z, A.rows, A.cols, fuse_bias, False, state, self.kernels,
+                                  reduce="mean")
+        else:
+            g = spmm_csr_bias_act(A.crow, A.col, None, X.contiguous(), A.rows, A.cols, None, False, state,
+                                  self.kernels, reduce="mean")
+            h = g @ self.weight_neigh
+        out = torch.addmm(h, X[:A.rows], self.weight_root)
+        if self.bias is not None and fuse_bias is None:
+            out = out + self.bias
+        return torch.relu(out) if self.activation == "relu" else out
+
+
 class GCN2:
     """Two GCNConv layers sharing one normalised adjacency Â = (crow, col, val)."""
 

@@ -100,7 +100,11 @@ def _check_packed(*tensors) -> None:
 
 
 def _csr_struct(a_crow, a_col, a_val, rows: int, cols: int, val_dtype=None) -> CsrStruct:
-    vd = _DENSE[a_val.dtype] if a_val is not None else _DENSE[val_dtype or torch.float32]
+    """``a_val`` None without a ``val_dtype`` is a pattern matrix (every stored entry 1.0)."""
+    if a_val is not None:
+        vd = _DENSE[a_val.dtype]
+    else:
+        vd = _DENSE[val_dtype] if val_dtype is not None else _lib.VAL_UNIT
     return CsrStruct(rows, cols, int(a_col.numel()), _ptr(a_crow), _ptr(a_col), _ptr(a_val),
                      _INDEX[a_crow.dtype], vd)
 
@@ -135,6 +139,7 @@ class SpmmPlan:
         self.t_crow = self.t_col = self.t_perm = self.t_part = None
         self.t_variant = _lib.VARIANT_AUTO
         self._t_val, self._t_val_key = None, None
+        self._inv_len = None
         if transpose:
             self.t_crow, self.t_col, _, self.t_perm = csr_transpose(a_crow, a_col, None, a_rows, a_cols, want_perm=True)
             self.t_variant, self.t_part = self._build(self.t_crow, a_cols, self.nnz, None)
@@ -172,6 +177,13 @@ class SpmmPlan:
                                                        _stream_ptr(a_val)), "permute_values")
             self._t_val, self._t_val_key = out, key
         return self._t_val
+
+    def inv_row_lengths(self) -> torch.Tensor:
+        """(rows, 1) float32: 1 / (stored entries of each row), 0 for an empty row — the row scale of
+        the mean aggregation's backward, computed once per structure."""
+        if self._inv_len is None:
+            self._inv_len = inv_row_lengths(self.a_crow)
+        return self._inv_len
 
     def prepared(self, transposed: bool = False) -> "_Prepared":
         """Low-host-overhead launcher of A·B (or, ``transposed``, of A^T·dY on the cached structure)."""
@@ -233,6 +245,18 @@ def _opts(flags: int = 0, tasks_per_warp: int = 0, variant: int = 0, part: Optio
                       acc32.data_ptr() if acc32 is not None else None)
 
 
+def inv_row_lengths(a_crow: torch.Tensor) -> torch.Tensor:
+    """(rows, 1) float32: 1 / (crow[i+1] - crow[i]), 0 for an empty row."""
+    lens = (a_crow[1:] - a_crow[:-1]).to(torch.float32)
+    return torch.where(lens > 0, 1.0 / lens.clamp(min=1), torch.zeros_like(lens)).unsqueeze(1)
+
+
+def reduce_flag(reduce: str) -> int:
+    """`reduce` argument -> OFSPMM_FWD_* bit ("sum": 0, "mean": OFSPMM_FWD_MEAN)."""
+    _chk(reduce in ("sum", "mean"), f"reduce must be 'sum' or 'mean', got {reduce!r}")
+    return _lib.FWD_MEAN if reduce == "mean" else 0
+
+
 def _acc32_flags(acc32, acc32_in: bool, acc32_out: bool, rows: int, n: int, dt) -> int:
     if not (acc32_in or acc32_out):
         return 0
@@ -248,14 +272,22 @@ def spmm_csr_compute(a_crow, a_col, a_val, b, a_rows: int, a_cols: int,
                      accumulate: bool = False, bias: Optional[torch.Tensor] = None, relu: bool = False,
                      tasks_per_warp: int = 0, variant: Optional[int] = None, order: Optional[str] = None,
                      acc32: Optional[torch.Tensor] = None, acc32_in: bool = False, acc32_out: bool = False,
-                     reserve_ctas: int = 0) -> torch.Tensor:
+                     reserve_ctas: int = 0, reduce: str = "sum") -> torch.Tensor:
     """SpmmCsrKernel::Compute — out[a_rows, n] = A · b  (``accumulate``: out += A · b; ``bias`` /
     ``relu``: epilogue fused into the store, applied to the complete row sum).
+
+    ``a_val`` None: pattern matrix, every stored entry is 1 and no values array is read.
+    ``reduce="mean"``: each row sum is divided by the row's stored-entry count before bias / ReLU
+    (an empty row gives 0; torch.sparse.mm(reduce="mean") semantics); not with ``accumulate`` or
+    the ``acc32`` passes.
 
     ``plan`` supplies the histogram-chosen variant and the cached task partition; ``tasks_per_warp``
     > 0 launches short-lived CTAs (multi-GPU overlap); ``order`` in {None, "dynamic", "static"}.
     ``acc32`` (+ ``acc32_in`` / ``acc32_out``): fp32 running sums of a bf16 product that is computed
     in several passes — rounded to bf16 once, by the pass without ``acc32_out``."""
+    mean = reduce_flag(reduce)
+    _chk(not (mean and (accumulate or acc32_in or acc32_out)),
+         "reduce='mean' divides the complete row sum: it cannot be combined with accumulate / acc32 passes")
     _check_device(a_crow, a_col, a_val, b, bias)
     (m, n), dt = infer_spmm_csr(a_crow, a_col, a_val, b, a_rows, a_cols)
     if out is None:
@@ -271,7 +303,7 @@ def spmm_csr_compute(a_crow, a_col, a_val, b, a_rows: int, a_cols: int,
     if plan is not None:
         _chk(plan.matches(a_crow, a_col, a_rows, a_cols, n, dt), "plan was built for another CSR structure / n / dtype")
     L = _lib.lib()
-    flags = (_lib.FWD_ACCUMULATE if accumulate else 0) | (_lib.FWD_BIAS if bias is not None else 0) | \
+    flags = mean | (_lib.FWD_ACCUMULATE if accumulate else 0) | (_lib.FWD_BIAS if bias is not None else 0) | \
             (_lib.FWD_RELU if relu else 0) | {None: 0, "dynamic": _lib.ORDER_DYNAMIC, "static": _lib.ORDER_STATIC}[order] | \
             _acc32_flags(acc32, acc32_in, acc32_out, m, n, dt)
     v = variant if variant is not None else (plan.variant if plan is not None else _lib.VARIANT_AUTO)
@@ -302,7 +334,9 @@ def spmm_csr_grad_b_compute(a_crow, a_col, a_val, dy, a_rows: int, a_cols: int,
       * ``transposed`` = (t_crow, t_col, t_val) from csr_transpose → forward kernel on that CSR;
       * default → ``ofspmm_bwd_b_transient`` (A^T built inside the workspace; deterministic and
         2-9x faster than the scatter on the BASELINE graphs);
-      * ``atomic=True`` → the reference-style vector-atomic scatter (order-nondeterministic)."""
+      * ``atomic=True`` → the reference-style vector-atomic scatter (order-nondeterministic).
+
+    ``a_val`` None: pattern matrix on every route; the plan route then caches no values of A^T."""
     _check_device(a_crow, a_col, a_val, dy)
     _chk(dy.dim() == 2 and dy.shape[0] == a_rows, f"dy must be (a_rows={a_rows}) x n")
     _check_packed(dy, out)
@@ -320,7 +354,7 @@ def spmm_csr_grad_b_compute(a_crow, a_col, a_val, dy, a_rows: int, a_cols: int,
         with torch.cuda.device(dy.device):
             if regather:   # the C ABI route the OneFlow glue uses: values gathered inside the call
                 A = _csr_struct(a_crow, a_col, a_val, a_rows, a_cols)
-                vs = 4 if A.val_dtype == _lib.DTYPE_FLOAT else 2
+                vs = {_lib.DTYPE_FLOAT: 4, _lib.DTYPE_BFLOAT16: 2, _lib.VAL_UNIT: 0}[A.val_dtype]
                 nbytes = ((max(A.nnz, 1) * vs + 255) // 256) * 256 + \
                     L.ofspmm_fwd_ex_workspace_bytes(a_cols, a_rows, A.nnz, n, _DENSE[dt], plan.t_variant)
                 nbytes = max(nbytes, L.ofspmm_bwd_b_cached_workspace_bytes(a_rows, a_cols, A.nnz, n, _DENSE[dt], A.val_dtype))
@@ -330,7 +364,8 @@ def spmm_csr_grad_b_compute(a_crow, a_col, a_val, dy, a_rows: int, a_cols: int,
                                             _ptr(dy), _ptr(out), n, _DENSE[dt], ctypes.byref(o), wsp, nbytes,
                                             _stream_ptr(dy)), "spmm_csr_grad_b(cached structure)")
             else:          # values of A^T kept while a_val's (pointer, version) is unchanged
-                At = _csr_struct(plan.t_crow, plan.t_col, plan.transposed_values(a_val), a_cols, a_rows)
+                t_val = plan.transposed_values(a_val) if a_val is not None else None
+                At = _csr_struct(plan.t_crow, plan.t_col, t_val, a_cols, a_rows)
                 nbytes = L.ofspmm_fwd_ex_workspace_bytes(a_cols, a_rows, At.nnz, n, _DENSE[dt], plan.t_variant)
                 ws, wsp = _workspace(nbytes, dy.device)
                 # acc32_out: the fp32 sums go to that buffer instead of `out` (16-bit products whose
@@ -348,6 +383,7 @@ def spmm_csr_grad_b_compute(a_crow, a_col, a_val, dy, a_rows: int, a_cols: int,
         if transposed is not None:
             t_crow, t_col, t_val = transposed
             _check_device(t_crow, t_col, t_val)
+            _chk((t_val is None) == (a_val is None), "transposed values must be given exactly when a_val is")
             At = _csr_struct(t_crow, t_col, t_val, a_cols, a_rows)
             At_ref = ctypes.byref(At)
         nbytes = L.ofspmm_bwd_b_workspace_bytes(a_rows, a_cols, A.nnz, n, _DENSE[dt], 1 if transposed is not None else 0)
