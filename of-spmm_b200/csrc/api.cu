@@ -217,12 +217,11 @@ int ofspmm_choose_variant(const int64_t* hist32_host, int64_t rows, int64_t nnz,
     // latencies dominate.  If no row reaches 512 non-zeros (histogram buckets >= 10 empty) and one
     // lane group per row yields at least 8 warps per SM, the whole-row kernel does the product in
     // ONE launch (cfg1: 34.6 -> see profiles/r2_cfg1_latency.md); otherwise 64-item tasks.
-    const int64_t vecw = dense_dtype == OFSPMM_DTYPE_BFLOAT16 ? 8 : 4;
     int64_t long_rows = 0;
     for (int b = 10; b < 32; ++b) long_rows += hist32_host[b];
-    if (n > 0 && n % vecw == 0 && n / vecw <= 32 && long_rows == 0) {
-      const int64_t lpr = n / vecw <= 8 ? 8 : (n / vecw <= 16 ? 16 : 32);
-      const int64_t warps = (rows * lpr + 31) / 32;
+    const LaneLayout rl = lane_layout(LaneOp::kFwdRows, dense_dtype, n, true);
+    if (rl.ok() && long_rows == 0) {
+      const int64_t warps = (rows * rl.lpr + 31) / 32;
       if (warps >= 148 * 8) return encode_variant(resolve_variant(OFSPMM_VARIANT_EXPLICIT | OFSPMM_VARIANT_ROWS, rows, nnz, n, dense_dtype));
     }
     return encode_variant(v);
@@ -234,8 +233,7 @@ int ofspmm_choose_variant(const int64_t* hist32_host, int64_t rows, int64_t nnz,
   // rows (median 256-511), where one long row piece leaves three of four groups idle
   // (profiles/r2_variant_sweeps.md).  Criterion: the MEDIAN row, empty rows included, has fewer
   // than 16 non-zeros, i.e. the per-row work dominates the per-non-zero work.
-  const int64_t vecw = dense_dtype == OFSPMM_DTYPE_BFLOAT16 ? 8 : 4;
-  const bool sub_warp_rows = n % vecw == 0 && n / vecw <= 16;
+  const bool sub_warp_rows = lane_layout(LaneOp::kFwdRowPar, dense_dtype, n, true).ok();
   int64_t below16 = 0;
   for (int b = 0; b <= 4; ++b) below16 += hist32_host[b];  // buckets 0..4 = lengths 0..15
   v.row_parallel = sub_warp_rows && 2 * below16 > rows;
@@ -661,8 +659,8 @@ const char* ofspmm_variant_name(int variant, int64_t rows, int64_t nnz, int64_t 
                     : v.row_parallel           ? "merge_path(256-item tasks, row-parallel groups)"
                                                : "merge_path(256-item tasks)";
   if (v.whole_rows) {
-    const int64_t nvec = n / (dense_dtype == OFSPMM_DTYPE_BFLOAT16 ? 8 : 4);
-    snprintf(buf, sizeof(buf), "%s/group-per-row(%d lanes x 16B, 4 gathers in flight)", fam, nvec <= 8 ? 8 : (nvec <= 16 ? 16 : 32));
+    snprintf(buf, sizeof(buf), "%s/group-per-row(%d lanes x 16B, 4 gathers in flight)", fam,
+             lane_layout(LaneOp::kFwdRows, dense_dtype, n, true).lpr);
     return buf;
   }
   snprintf(buf, sizeof(buf), "%s/%s", fam, fwd_variant_name(n, dense_dtype, true));

@@ -5,26 +5,19 @@
 
 namespace ofspmm {
 
-int launch_family_base(const FwdParams&, int, int, int, bool, const FwdLaunch&, cudaStream_t);
-int launch_family_small(const FwdParams&, int, int, int, bool, const FwdLaunch&, cudaStream_t);
-int launch_family_rowpar(const FwdParams&, int, int, int, bool, const FwdLaunch&, cudaStream_t);
-int launch_family_rows(const FwdParams&, int, int, cudaStream_t);
+int launch_family_base(const FwdParams&, const LaneLayout&, int, int, int, const FwdLaunch&, cudaStream_t);
+int launch_family_small(const FwdParams&, const LaneLayout&, int, int, int, const FwdLaunch&, cudaStream_t);
+int launch_family_rowpar(const FwdParams&, const LaneLayout&, int, int, int, const FwdLaunch&, cudaStream_t);
+int launch_family_rows(const FwdParams&, const LaneLayout&, int, int, cudaStream_t);
 
 namespace {
 
-int64_t vec_width(int dense_dtype) { return dense_dtype == OFSPMM_DTYPE_BFLOAT16 ? 8 : 4; }
-
-// Which dense widths the row-parallel family has kernels for (16-byte aligned rows assumed; fwd
-// falls back to the base family otherwise): the sub-warp layouts, 8 or 16 lanes per dense row.
-bool rowpar_supported(int64_t n, int dense_dtype) {
-  const int64_t v = vec_width(dense_dtype);
-  return n % v == 0 && n / v <= 16;
-}
-
-// Dense widths the whole-row family has kernels for: 16-byte vectors, at most 32 of them.
-bool rows_supported(int64_t n, int dense_dtype) {
-  const int64_t v = vec_width(dense_dtype);
-  return n > 0 && n % v == 0 && n / v <= 32;
+// B, C and the bias allow 16-byte vector rows: aligned addresses, strides a whole number of vectors.
+bool vec_rows_ok(const void* B, int64_t ldb, const void* C, int64_t ldc, int dense_dtype, const FwdLaunch& L) {
+  const int64_t v = dense_vec_width(dense_dtype);
+  const uintptr_t bits = reinterpret_cast<uintptr_t>(B) | reinterpret_cast<uintptr_t>(C) |
+                         ((L.flags & kFwdBias) ? reinterpret_cast<uintptr_t>(L.bias) : 0);
+  return (bits & 15) == 0 && ldb % v == 0 && ldc % v == 0;
 }
 
 }  // namespace
@@ -34,11 +27,14 @@ bool rows_supported(int64_t n, int dense_dtype) {
 // ofspmm_choose_variant() may also pick the row-parallel layout (api.cu).
 // Wide matrices (wide_nnz) have 256-item merge-path kernels only: an explicit whole-row or
 // 64-item code falls back to them (AUTO never picks 64-item tasks at that size anyway).
+// The row-parallel and whole-row layouts are looked up for 16-byte aligned rows; a launch whose
+// rows are not falls back to another family.
 FwdVariant resolve_variant(int variant, int64_t rows, int64_t nnz, int64_t n, int dense_dtype) {
+  const bool rowpar_supported = lane_layout(LaneOp::kFwdRowPar, dense_dtype, n, true).ok();
   FwdVariant v{kTaskItems, false, false};
   if (wide_nnz(nnz)) {
     v.row_parallel = (variant & OFSPMM_VARIANT_EXPLICIT) && (variant & OFSPMM_VARIANT_ROWPAR) &&
-                     !(variant & (OFSPMM_VARIANT_ROWS | OFSPMM_VARIANT_ITEMS64)) && rowpar_supported(n, dense_dtype);
+                     !(variant & (OFSPMM_VARIANT_ROWS | OFSPMM_VARIANT_ITEMS64)) && rowpar_supported;
     return v;
   }
   if (variant & OFSPMM_VARIANT_EXPLICIT) {
@@ -46,9 +42,9 @@ FwdVariant resolve_variant(int variant, int64_t rows, int64_t nnz, int64_t n, in
       // sized like the 64-item family, which is also what runs when a launch cannot use the
       // whole-row kernel (int64 indices, unaligned or strided-odd rows)
       v.items = kSmallTaskItems;
-      v.whole_rows = rows_supported(n, dense_dtype);
+      v.whole_rows = lane_layout(LaneOp::kFwdRows, dense_dtype, n, true).ok();
     } else if (variant & OFSPMM_VARIANT_ITEMS64) v.items = kSmallTaskItems;
-    else if ((variant & OFSPMM_VARIANT_ROWPAR) && rowpar_supported(n, dense_dtype)) v.row_parallel = true;
+    else if ((variant & OFSPMM_VARIANT_ROWPAR) && rowpar_supported) v.row_parallel = true;
     return v;
   }
   if (num_tasks(rows, nnz, kTaskItems) < kSmallProblemTasks) v.items = kSmallTaskItems;
@@ -90,11 +86,8 @@ int launch_task_partition(const void* crow, int idx_dtype, int64_t rows, int64_t
 // clears whole_rows for those; they have int64 indices besides).
 bool rows_kernel_applies(const ofspmm_csr* A, const void* B, int64_t ldb, const void* C, int64_t ldc, int64_t n,
                          int dense_dtype, const FwdLaunch& L) {
-  if (!L.variant.whole_rows || A->idx_dtype != OFSPMM_DTYPE_INT32 || !rows_supported(n, dense_dtype)) return false;
-  const int64_t v = vec_width(dense_dtype);
-  const uintptr_t bits = reinterpret_cast<uintptr_t>(B) | reinterpret_cast<uintptr_t>(C) |
-                         ((L.flags & kFwdBias) ? reinterpret_cast<uintptr_t>(L.bias) : 0);
-  return (bits & 15) == 0 && ldb % v == 0 && ldc % v == 0;
+  return L.variant.whole_rows && A->idx_dtype == OFSPMM_DTYPE_INT32 &&
+         lane_layout(LaneOp::kFwdRows, dense_dtype, n, vec_rows_ok(B, ldb, C, ldc, dense_dtype, L)).ok();
 }
 
 int launch_fwd(const ofspmm_csr* A, const void* B, int64_t ldb, void* C, int64_t ldc, int64_t n,
@@ -120,32 +113,28 @@ int launch_fwd(const ofspmm_csr* A, const void* B, int64_t ldb, void* C, int64_t
   p.flags = L.flags;
   p.acc32 = L.acc32;
   p.counter = L.dynamic ? static_cast<unsigned int*>(counter) : nullptr;
-  const int64_t v = vec_width(dense_dtype);
-  const bool aligned = ((reinterpret_cast<uintptr_t>(B) | reinterpret_cast<uintptr_t>(C) |
-                         ((L.flags & kFwdBias) ? reinterpret_cast<uintptr_t>(L.bias) : 0)) & 15) == 0;
-  const bool vec_rows = aligned && n % v == 0 && ldb % v == 0 && ldc % v == 0;
   if (rows_kernel_applies(A, B, ldb, C, ldc, n, dense_dtype, L)) {
     p.counter = nullptr;
-    return launch_family_rows(p, dense_dtype, A->val_dtype, stream);
+    return launch_family_rows(p, lane_layout(LaneOp::kFwdRows, dense_dtype, n, true), dense_dtype, A->val_dtype, stream);
   }
-  if (L.variant.items == kSmallTaskItems)
-    return launch_family_small(p, A->idx_dtype, dense_dtype, A->val_dtype, aligned, L, stream);
-  if (L.variant.row_parallel && vec_rows && rowpar_supported(n, dense_dtype))
-    return launch_family_rowpar(p, A->idx_dtype, dense_dtype, A->val_dtype, aligned, L, stream);
-  return launch_family_base(p, A->idx_dtype, dense_dtype, A->val_dtype, aligned, L, stream);
+  const bool vec_rows = vec_rows_ok(B, ldb, C, ldc, dense_dtype, L);
+  if (L.variant.row_parallel) {  // 256-item tasks only (resolve_variant)
+    const LaneLayout rowpar = lane_layout(LaneOp::kFwdRowPar, dense_dtype, n, vec_rows);
+    if (rowpar.ok()) return launch_family_rowpar(p, rowpar, A->idx_dtype, dense_dtype, A->val_dtype, L, stream);
+  }
+  const LaneLayout l = lane_layout(LaneOp::kFwd, dense_dtype, n, vec_rows);
+  if (L.variant.items == kSmallTaskItems) return launch_family_small(p, l, A->idx_dtype, dense_dtype, A->val_dtype, L, stream);
+  return launch_family_base(p, l, A->idx_dtype, dense_dtype, A->val_dtype, L, stream);
 }
 
 const char* fwd_variant_name(int64_t n, int dense_dtype, bool aligned) {
-  const int vecw = dense_dtype == OFSPMM_DTYPE_BFLOAT16 ? 8 : 4;
-  if (aligned && n % vecw == 0) {
-    const int64_t nvec = n / vecw;
-    if (nvec <= 8) return "vector-per-row(8 lanes x 16B, 4 nnz per step)";
-    if (nvec <= 16) return "vector-per-row(16 lanes x 16B, 2 nnz per step)";
-    if (nvec <= 32) return "warp-per-row(32 lanes x 16B)";
-    if (nvec <= 64) return "warp-per-row(32 lanes x 2 x 16B)";
-    return "warp-per-row(32 lanes x 4 x 16B, column panels)";
-  }
-  return "warp-per-row(scalar lanes, unaligned n)";
+  const LaneLayout l = lane_layout(LaneOp::kFwd, dense_dtype, n, aligned);
+  if (l.vec == 1) return "warp-per-row(scalar lanes, unaligned n)";
+  if (l.lpr == 8) return "vector-per-row(8 lanes x 16B, 4 nnz per step)";
+  if (l.lpr == 16) return "vector-per-row(16 lanes x 16B, 2 nnz per step)";
+  if (l.ch == 1) return "warp-per-row(32 lanes x 16B)";
+  if (l.ch == 2) return "warp-per-row(32 lanes x 2 x 16B)";
+  return "warp-per-row(32 lanes x 4 x 16B, column panels)";
 }
 
 }  // namespace ofspmm

@@ -4,8 +4,8 @@
 #include "fwd_launch.cuh"
 
 namespace ofspmm {
-int launch_family_rowpar(const FwdParams& p, int idx_dtype, int dense_dtype, int val_dtype, bool aligned,
+int launch_family_rowpar(const FwdParams& p, const LaneLayout& l, int idx_dtype, int dense_dtype, int val_dtype,
                          const FwdLaunch& L, cudaStream_t stream) {
-  return launch_family<true, kTaskItems>(p, idx_dtype, dense_dtype, val_dtype, aligned, L, stream);
+  return launch_family<true, kTaskItems>(p, l, idx_dtype, dense_dtype, val_dtype, L, stream);
 }
 }  // namespace ofspmm

@@ -1,6 +1,6 @@
 // fwd_rows.cu — the whole-row family (spmm_rows_kernel.cuh): one launch, no workspace; picked by
 // ofspmm_choose_variant for small problems whose longest row is short.
-#include "internal.h"
+#include "launch.cuh"
 #include "spmm_rows_kernel.cuh"
 
 namespace ofspmm {
@@ -17,27 +17,18 @@ int launch_rows_one(const FwdParams& p, cudaStream_t stream) {
   return OFSPMM_OK;
 }
 
-template <typename DT, typename ValT>
-int launch_rows_typed(const FwdParams& p, cudaStream_t stream) {
-  constexpr int VECW = 16 / sizeof(DT);
-  const int nvec = p.n / VECW;
-  if (nvec <= 8) return launch_rows_one<DT, ValT, VECW, 8>(p, stream);
-  if (nvec <= 16) return launch_rows_one<DT, ValT, VECW, 16>(p, stream);
-  return launch_rows_one<DT, ValT, VECW, 32>(p, stream);
-}
-
 }  // namespace
 
-// Preconditions (checked by the caller, fwd.cu:rows_kernel_applies): int32 indices, 16-byte
-// aligned rows, n a multiple of the 16-byte vector and at most 32 vectors wide.
-int launch_family_rows(const FwdParams& p, int dense_dtype, int val_dtype, cudaStream_t stream) {
-  if (dense_dtype == OFSPMM_DTYPE_FLOAT && val_dtype == OFSPMM_DTYPE_FLOAT) return launch_rows_typed<float, float>(p, stream);
-  if (dense_dtype == OFSPMM_DTYPE_BFLOAT16 && val_dtype == OFSPMM_DTYPE_FLOAT) return launch_rows_typed<__nv_bfloat16, float>(p, stream);
-  if (dense_dtype == OFSPMM_DTYPE_BFLOAT16 && val_dtype == OFSPMM_DTYPE_BFLOAT16)
-    return launch_rows_typed<__nv_bfloat16, __nv_bfloat16>(p, stream);
-  if (dense_dtype == OFSPMM_DTYPE_FLOAT && val_dtype == OFSPMM_VAL_UNIT) return launch_rows_typed<float, UnitVal>(p, stream);
-  if (dense_dtype == OFSPMM_DTYPE_BFLOAT16 && val_dtype == OFSPMM_VAL_UNIT) return launch_rows_typed<__nv_bfloat16, UnitVal>(p, stream);
-  return OFSPMM_ERR_UNSUPPORTED_DTYPE;
+// Preconditions (checked by the caller, fwd.cu:rows_layout): int32 indices, 16-byte aligned rows
+// and a layout of the whole-row ladder.
+int launch_family_rows(const FwdParams& p, const LaneLayout& l, int dense_dtype, int val_dtype, cudaStream_t stream) {
+  return dispatch_dtypes<true>(dense_dtype, val_dtype, [&](auto dense, auto val) {
+    using DT = typename decltype(dense)::type;
+    constexpr int V = vec_width(sizeof(DT));
+    return dispatch_lanes<Lanes<V, 8, 1>, Lanes<V, 16, 1>, Lanes<V, 32, 1>>(l, [&](auto lanes) {
+      return launch_rows_one<DT, typename decltype(val)::type, decltype(lanes)::VEC, decltype(lanes)::LPR>(p, stream);
+    });
+  });
 }
 
 }  // namespace ofspmm

@@ -5,6 +5,7 @@
 #include <stdint.h>
 
 #include <atomic>
+#include <initializer_list>
 
 #include "../../include/ofspmm.h"
 
@@ -48,6 +49,62 @@ struct FwdVariant {
   bool row_parallel;  // sub-warp per row (short rows, narrow dense operand) instead of nnz-parallel
   bool whole_rows;    // spmm_rows_kernel: one launch, no merge path (items = kSmallTaskItems for sizing)
 };
+
+// Elements in one 16-byte vector of a dense row (fp32: 4, bf16: 8).
+constexpr int vec_width(size_t elem_bytes) { return static_cast<int>(16 / elem_bytes); }
+inline int dense_vec_width(int dense_dtype) { return vec_width(dense_dtype == OFSPMM_DTYPE_BFLOAT16 ? 2 : 4); }
+
+// The kernels whose lane layout follows the dense width n: the merge-path forward (256- and 64-item
+// families; row-parallel family), the whole-row forward, the SDDMM (no layout: sddmm_wide_kernel)
+// and the atomic A^T.dY scatter.
+enum class LaneOp { kFwd, kFwdRowPar, kFwdRows, kSddmm, kAtomic };
+
+// Template parameters of a kernel's lanes: LPR lanes span a dense row, each holding CH chunks of VEC
+// elements; rows wider than one register tile (LPR * CH * VEC) run in `panels` column panels.
+// lpr 0: the kernel has no layout for this width.  full: n is a whole number of register tiles.
+struct LaneLayout {
+  int vec = 1, lpr = 0, ch = 0, panels = 1;
+  bool full = false;
+  bool ok() const { return lpr != 0; }
+};
+
+// Lane layout of `op` for n dense columns.  `vec_ok`: the operands' addresses and strides allow
+// 16-byte vector rows (n must also be a whole number of vectors).  Each op has its own ladders, one
+// for vector and one for scalar lanes; a rung serves rows of up to `top` vectors (scalar lanes:
+// elements), top 0 any wider row in column panels.
+inline LaneLayout lane_layout(LaneOp op, int dense_dtype, int64_t n, bool vec_ok) {
+  struct Rung { int64_t top; int lpr, ch; };
+  const int w = dense_vec_width(dense_dtype);
+  const bool vec = vec_ok && n % w == 0;
+  const int64_t units = vec ? n / w : n;
+  const int lane_vec = vec ? w : 1;
+  auto pick = [&](std::initializer_list<Rung> ladder) {
+    for (const Rung& r : ladder) {
+      if (r.top != 0 && units > r.top) continue;
+      const int64_t tile = int64_t{r.lpr} * r.ch;
+      const int panels = r.top == 0 ? static_cast<int>((units + tile - 1) / tile) : 1;
+      return LaneLayout{lane_vec, r.lpr, r.ch, panels, n % (tile * lane_vec) == 0};
+    }
+    return LaneLayout{lane_vec};
+  };
+  switch (op) {
+    case LaneOp::kFwd:
+      return vec ? pick({{8, 8, 1}, {16, 16, 1}, {32, 32, 1}, {64, 32, 2}, {0, 32, 4}})
+                 : pick({{32, 32, 1}, {64, 32, 2}, {128, 32, 4}, {0, 32, 8}});
+    case LaneOp::kFwdRowPar:  // sub-warp groups only
+      return vec ? pick({{8, 8, 1}, {16, 16, 1}}) : pick({});
+    case LaneOp::kFwdRows:
+      return vec && n > 0 ? pick({{8, 8, 1}, {16, 16, 1}, {32, 32, 1}}) : pick({});
+    case LaneOp::kSddmm:
+      return vec ? pick({{8, 8, 1}, {16, 16, 1}, {32, 32, 1}, {64, 32, 2}, {128, 32, 4}})
+                 : pick({{32, 32, 1}, {128, 32, 4}});
+    case LaneOp::kAtomic:
+      return vec ? pick({{8, 8, 1}, {16, 16, 1}, {32, 32, 1}, {64, 32, 2}, {0, 32, 4}})
+                 : pick({{32, 32, 1}, {128, 32, 4}, {0, 32, 8}});
+  }
+  return pick({});
+}
+
 FwdVariant resolve_variant(int variant, int64_t rows, int64_t nnz, int64_t n, int dense_dtype);
 struct FwdLaunch;
 bool rows_kernel_applies(const ofspmm_csr* A, const void* B, int64_t ldb, const void* C, int64_t ldc, int64_t n,

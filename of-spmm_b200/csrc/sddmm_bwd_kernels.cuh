@@ -27,6 +27,18 @@ __device__ __forceinline__ unsigned group_mask(int grp) {
   return ((1u << LPR) - 1u) << (grp * LPR);
 }
 
+// Coalesced write-back of the SDDMM results of non-zeros ns .. ns+cnt_nz-1, staged in sout;
+// out-of-range columns (badmask, one bit per staged non-zero and lane) give 0.
+template <typename ValT, typename NzT>
+__device__ __forceinline__ void store_dval(ValT* dval, NzT ns, const float* sout, int cnt_nz, unsigned badmask, int lane) {
+  __syncwarp();
+  for (int q0 = 0; q0 < cnt_nz; q0 += 32) {
+    const unsigned bad = __shfl_sync(0xffffffffu, badmask, q0 >> 5);
+    const int q = q0 + lane;
+    if (q < cnt_nz) dval[ns + q] = from_float<ValT>(((bad >> lane) & 1u) ? 0.f : sout[q]);
+  }
+}
+
 // dval[p] = <dY[i,:], B[col[p],:]>.
 // LPR lanes span one dense row (CH chunks of VEC each); the dY row chunk stays in registers while
 // the task walks the row's non-zeros.  Hot loop per 4 non-zeros and lane group: one LDS.128 of 4
@@ -46,21 +58,14 @@ sddmm_merge_kernel(const SddmmParams p) {
   using RV = RowVec<DT, VEC>;
   static_assert(LPR >= 4, "transpose-reduce needs at least 4 lanes per row");
 
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  Stage* stages = reinterpret_cast<Stage*>(smem_raw);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + sizeof(Stage) * WARPS);
-
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const int grp = lane / LPR;
   const int lig = lane % LPR;
   const unsigned gmask = group_mask<LPR>(grp);
-  Stage& st = stages[warp];
-  uint64_t* bar = &bars[warp];
+  uint64_t* bar;
+  Stage& st = warp_stage<Stage, WARPS>(warp, lane, bar);
   const uint32_t col_sa = smem_u32(st.col);
-  if (lane == 0) mbar_init(bar, 1);
-  fence_mbar_init();
-  __syncwarp();
 
   const uint64_t pol_stream = l2_policy_evict_first();
   const IdxT* __restrict__ crow = static_cast<const IdxT*>(p.crow);
@@ -220,13 +225,7 @@ sddmm_merge_kernel(const SddmmParams p) {
       }
       e = e_end;
     }
-    __syncwarp();
-    // coalesced write-back; out-of-range columns give 0
-    for (int q0 = 0; q0 < cnt_nz; q0 += 32) {
-      const unsigned bad = __shfl_sync(0xffffffffu, tk.badmask, q0 >> 5);
-      const int q = q0 + lane;
-      if (q < cnt_nz) dval[ns + q] = from_float<ValT>(((bad >> lane) & 1u) ? 0.f : sout[q]);
-    }
+    store_dval(dval, ns, sout, cnt_nz, tk.badmask, lane);
   }
 }
 
@@ -238,16 +237,10 @@ __global__ void __launch_bounds__(WARPS * 32) sddmm_wide_kernel(const SddmmParam
   const PartT* part = static_cast<const PartT*>(p.part);
   using Stage = TaskStage<IdxT, float, ITEMS>;
   using RV = RowVec<DT, VEC>;
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  Stage* stages = reinterpret_cast<Stage*>(smem_raw);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + sizeof(Stage) * WARPS);
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
-  Stage& st = stages[warp];
-  uint64_t* bar = &bars[warp];
-  if (lane == 0) mbar_init(bar, 1);
-  fence_mbar_init();
-  __syncwarp();
+  uint64_t* bar;
+  Stage& st = warp_stage<Stage, WARPS>(warp, lane, bar);
   const uint64_t pol_stream = l2_policy_evict_first();
   const IdxT* __restrict__ crow = static_cast<const IdxT*>(p.crow);
   const IdxT* __restrict__ col = static_cast<const IdxT*>(p.col);
@@ -287,12 +280,7 @@ __global__ void __launch_bounds__(WARPS * 32) sddmm_wide_kernel(const SddmmParam
       }
       if (e_end > e) e = e_end;
     }
-    __syncwarp();
-    for (int q0 = 0; q0 < cnt_nz; q0 += 32) {
-      const unsigned bad = __shfl_sync(0xffffffffu, tk.badmask, q0 >> 5);
-      const int q = q0 + lane;
-      if (q < cnt_nz) dval[ns + q] = from_float<ValT>(((bad >> lane) & 1u) ? 0.f : sout[q]);
-    }
+    store_dval(dval, ns, sout, cnt_nz, tk.badmask, lane);
   }
 }
 
@@ -332,18 +320,12 @@ __global__ void __launch_bounds__(WARPS * 32) bwd_atomic_kernel(const BwdAtomicP
   const PartT* part = static_cast<const PartT*>(p.part);
   constexpr int G = 32 / LPR;
   using Stage = TaskStage<IdxT, ValT, ITEMS>;
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  Stage* stages = reinterpret_cast<Stage*>(smem_raw);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + sizeof(Stage) * WARPS);
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const int grp = lane / LPR;
   const int lig = lane % LPR;
-  Stage& st = stages[warp];
-  uint64_t* bar = &bars[warp];
-  if (lane == 0) mbar_init(bar, 1);
-  fence_mbar_init();
-  __syncwarp();
+  uint64_t* bar;
+  Stage& st = warp_stage<Stage, WARPS>(warp, lane, bar);
 
   const uint64_t pol_stream = l2_policy_evict_first();
   const IdxT* __restrict__ crow = static_cast<const IdxT*>(p.crow);

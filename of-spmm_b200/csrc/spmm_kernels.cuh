@@ -317,6 +317,37 @@ __device__ __forceinline__ uint2 lds64(uint32_t addr) {
   return v;
 }
 
+// The 4 staged values at shared-memory byte address va as fp32 (a pattern matrix: four 1s).
+template <typename ValT>
+__device__ __forceinline__ void lds_vals4(uint32_t va, float (&v4)[4]) {
+  if constexpr (kIsUnit<ValT>) {
+    (void)va;
+    v4[0] = v4[1] = v4[2] = v4[3] = 1.f;
+  } else if constexpr (sizeof(ValT) == 4) {
+    const uint4 w = lds128(va);
+    v4[0] = __uint_as_float(w.x); v4[1] = __uint_as_float(w.y);
+    v4[2] = __uint_as_float(w.z); v4[3] = __uint_as_float(w.w);
+  } else {
+    const uint2 w = lds64(va);
+    v4[0] = __uint_as_float(w.x << 16); v4[1] = __uint_as_float(w.x & 0xffff0000u);
+    v4[2] = __uint_as_float(w.y << 16); v4[3] = __uint_as_float(w.y & 0xffff0000u);
+  }
+}
+
+// This warp's task stage, and its mbarrier initialised for one arrival, in the dynamic shared memory
+// of a merge-path kernel: WARPS stages, then WARPS mbarriers (kMergeSmem in launch.cuh).
+template <typename Stage, int WARPS>
+__device__ __forceinline__ Stage& warp_stage(int warp, int lane, uint64_t*& bar) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  Stage* stages = reinterpret_cast<Stage*>(smem_raw);
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + sizeof(Stage) * WARPS);
+  bar = &bars[warp];
+  if (lane == 0) mbar_init(bar, 1);
+  fence_mbar_init();
+  __syncwarp();
+  return stages[warp];
+}
+
 // kFull: n is a whole number of LPR*VEC*CH-column tiles, so no lane is ever masked and the chunk
 // offsets are immediates.  Otherwise masked chunks are pointed at column 0 (a valid address:
 // their loads are harmless duplicates) and only the stores are predicated.
@@ -333,22 +364,14 @@ spmm_merge_kernel(const FwdParams p) {
   using Stage = TaskStage<IdxT, ValT, ITEMS>;
   using RV = RowVec<DT, VEC>;
 
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  Stage* stages = reinterpret_cast<Stage*>(smem_raw);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + sizeof(Stage) * WARPS);
-
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const int grp = lane / LPR;  // which group of concurrent non-zeros
   const int lig = lane % LPR;  // lane in group -> column chunk
-  Stage& st = stages[warp];
-  uint64_t* bar = &bars[warp];
+  uint64_t* bar;
+  Stage& st = warp_stage<Stage, WARPS>(warp, lane, bar);
   const uint32_t col_sa = smem_u32(st.col);
   const uint32_t val_sa = staged_val_addr(st);
-
-  if (lane == 0) mbar_init(bar, 1);
-  fence_mbar_init();
-  __syncwarp();
 
   const uint64_t pol_stream = l2_policy_evict_first();
 #if OFSPMM_B_LOAD >= 2
@@ -453,21 +476,6 @@ spmm_merge_kernel(const FwdParams p) {
         const int s0 = tk.pre_c + e0, s1 = tk.pre_c + e1;
         const int cbase = s0 & ~3;
         const int nchunks = s1 > s0 ? ((s1 + 3) >> 2) - (s0 >> 2) : 0;
-        auto load_vals = [&](int sa, float (&v4)[4]) {
-          const uint32_t va = val_s0 + static_cast<uint32_t>(sa) * static_cast<uint32_t>(sizeof(ValT));
-          if constexpr (kUnit) {
-            (void)va;
-            v4[0] = v4[1] = v4[2] = v4[3] = 1.f;
-          } else if constexpr (sizeof(ValT) == 4) {
-            const uint4 w = lds128(va);
-            v4[0] = __uint_as_float(w.x); v4[1] = __uint_as_float(w.y);
-            v4[2] = __uint_as_float(w.z); v4[3] = __uint_as_float(w.w);
-          } else {
-            const uint2 w = lds64(va);
-            v4[0] = __uint_as_float(w.x << 16); v4[1] = __uint_as_float(w.x & 0xffff0000u);
-            v4[2] = __uint_as_float(w.y << 16); v4[3] = __uint_as_float(w.y & 0xffff0000u);
-          }
-        };
         // edge chunk (first / last of the row): per-slot predicated gathers, masked values
         auto edge_chunk = [&](int q) {
           const int sa = cbase + 4 * q;
@@ -486,7 +494,7 @@ spmm_merge_kernel(const FwdParams p) {
             }
           }
           float v4[4];
-          load_vals(sa, v4);
+          lds_vals4<ValT>(val_s0 + static_cast<uint32_t>(sa) * static_cast<uint32_t>(sizeof(ValT)), v4);
 #pragma unroll
           for (int u = 0; u < 4; ++u) {
             const float v = ok[u] ? v4[u] : 0.f;
@@ -519,18 +527,7 @@ spmm_merge_kernel(const FwdParams p) {
               ca += 16u * kChunkStride;
               if (ca < cend) cn = lds128(ca);  // next chunk's indices, while the gathers fly
               float v4[4];
-              if constexpr (kUnit) {
-                (void)va;
-                v4[0] = v4[1] = v4[2] = v4[3] = 1.f;
-              } else if constexpr (sizeof(ValT) == 4) {
-                const uint4 w = lds128(va);
-                v4[0] = __uint_as_float(w.x); v4[1] = __uint_as_float(w.y);
-                v4[2] = __uint_as_float(w.z); v4[3] = __uint_as_float(w.w);
-              } else {
-                const uint2 w = lds64(va);
-                v4[0] = __uint_as_float(w.x << 16); v4[1] = __uint_as_float(w.x & 0xffff0000u);
-                v4[2] = __uint_as_float(w.y << 16); v4[3] = __uint_as_float(w.y & 0xffff0000u);
-              }
+              lds_vals4<ValT>(va, v4);
 #pragma unroll
               for (int u = 0; u < 4; ++u)
 #pragma unroll

@@ -5,10 +5,14 @@ instantiations in the built library) and tests/test_gpu_kernel_matrix.py (every 
 fp64 oracle).
 
 Mirrored code:
-  * forward: fwd.cu (resolve_variant, rows_kernel_applies, launch_fwd), fwd_launch.cuh
-    (launch_family, launch_typed, launch_one, launch_full) and fwd_rows.cu;
+  * lane layouts: internal.h (lane_layout, one ladder per LaneOp) and the layouts each launcher
+    instantiates (dispatch_lanes in fwd_launch.cuh:launch_typed, fwd_rows.cu, sddmm.cu:launch_typed,
+    bwd.cu:launch_typed);
+  * type dispatch: launch.cuh (dispatch_dtypes, dispatch_index) as each launcher calls it;
+  * forward: fwd.cu (resolve_variant, vec_rows_ok, rows_layout, launch_fwd), fwd_launch.cuh
+    (launch_family, launch_typed, launch_full) and fwd_rows.cu (launch_family_rows);
   * SDDMM: sddmm.cu (launch_sddmm, launch_typed);
-  * atomic A^T.dY: bwd.cu (launch_bwd_atomic, launch_typed).
+  * atomic A^T.dY: bwd.cu (launch_bwd_atomic, launch_typed, launch_one).
 
 A kernel key is the demangled template argument list of the kernel the call launches, e.g.
 ("spmm_merge_kernel", "float", "float", "int", 4, 8, 1, True, False, 256, 4, "int2"): the same

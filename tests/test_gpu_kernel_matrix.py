@@ -2,7 +2,8 @@
 
 The cases come from tests/_kernel_matrix.py, which mirrors the dispatch code: each call asserts
 the kernel the mirror predicts through ofspmm_launch_count() (partition, merge kernel, fix-up when
-the matrix has more than one task; one launch for the whole-row kernel), and
+the matrix has more than one task; one launch for the whole-row kernel) and, once per case, by the
+kernel names torch.profiler records; and
 tests/test_kernel_matrix_host.py checks that the cases reach every instantiation in the library.
 
 The graphs are built to hit the places where such kernels go wrong: empty first and last rows and
@@ -18,6 +19,8 @@ Tolerances (oracle/oracle.py, SURVEY.md §8c):
     a second rounding (a bf16 partial row, a bf16 round trip between acc32 passes) fails it.
 """
 import os
+import re
+import subprocess
 import sys
 from functools import lru_cache
 
@@ -390,3 +393,52 @@ def test_sddmm(graphs, case):
     got = _launch(lambda: ops.sddmm_csr_compute(G.crow, G.col, dY, B, G.M, G.K, val_dtype=TORCH[case.val]), want, case.id)
     _check(got, ref, tol, case.val, case.id)
     assert torch.equal(got, ops.sddmm_csr_compute(G.crow, G.col, dY, B, G.M, G.K, val_dtype=TORCH[case.val]))
+
+
+# ------------------------------------------------------------------ kernel names
+
+def _profiled_key(name: str):
+    """KM.parse_demangled of a kernel name as torch.profiler reports it.  Demanglers differ in how
+    they spell template values (`(int)8`, `(bool)1` against c++filt's `8`, `true`), and a name that
+    arrives mangled is demangled with c++filt."""
+    if name.startswith("_Z"):
+        name = subprocess.run(["c++filt"], input=name, capture_output=True, text=True, check=True).stdout.strip()
+    name = re.sub(r"\(bool\)([01])", lambda m: "true" if m.group(1) == "1" else "false", name)
+    name = re.sub(r"\((?:int|unsigned int|long|unsigned long)\)(-?\d+)", r"\1", name)
+    return KM.parse_demangled(name)
+
+
+def _run_case(G, case):
+    """The calls case_kernels accounts for, on operands of the case's alignment: the forward plain,
+    with a bias and as a mean with a bias; the SDDMM; the atomic A^T.dY."""
+    n, dense, val = case.n, case.dense, case.val
+    dt = TORCH[dense]
+    if case.op == "fwd":
+        B = _carve(_host_dense(G.K, n, 1, dense, True), case.misaligned == "B")
+        bias = _carve(_host_dense(1, n, 3, dense)[0], case.misaligned == "bias")
+        v = KM.FAMILIES[case.family]
+        for kw in ({}, dict(bias=bias, relu=True), dict(bias=bias, relu=True, reduce="mean")):
+            C = _carve(torch.empty(G.M, n, dtype=dt), case.misaligned == "C")
+            ops.spmm_csr_compute(G.crow, G.col, G.val[val], B, G.M, G.K, out=C, variant=v, **kw)
+    elif case.op == "sddmm":
+        dY = _carve(_host_dense(G.M, n, 2, dense), case.misaligned == "dY")
+        B = _carve(_host_dense(G.K, n, 1, dense, True), case.misaligned == "B")
+        ops.sddmm_csr_compute(G.crow, G.col, dY, B, G.M, G.K, val_dtype=TORCH[val])
+    else:
+        dY = _carve(_host_dense(G.M, n, 2, dense), case.misaligned == "dY")
+        out = torch.empty(G.K, n, dtype=dt, device=DEV)
+        ops.spmm_csr_grad_b_compute(G.crow, G.col, G.val[val], dY, G.M, G.K, out=out, atomic=True)
+
+
+@pytest.mark.parametrize("case", list(KM.all_cases()), ids=lambda c: c.id)
+def test_launched_kernel_names(graphs, case):
+    """The kernels a case launches, by demangled name, are the ones the mirror predicts: a width
+    that moves to another lane layout keeps the launch count and the result, but not the name."""
+    G = graphs[case.idx]
+    with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
+        _run_case(G, case)
+        torch.cuda.synchronize()
+    names = {e.name for e in prof.events()} | {k.name for e in prof.events() for k in getattr(e, "kernels", ())}
+    got = {k for k in map(_profiled_key, names) if k is not None}
+    want = KM.case_kernels(case, G.M, G.nnz)
+    assert got == want, f"{case.id}: launched {sorted(map(KM.demangled, got))}, predicted {sorted(map(KM.demangled, want))}"
