@@ -374,6 +374,31 @@ OFSPMM_API int ofspmm_csr_normalize(const void* crow, const void* col, float* va
                                     int64_t rows, int64_t cols, int mode, float* dinv_rows,
                                     ofspmm_stream_t stream);
 
+/* ---- Neighbour sampling (mini-batch GraphSAGE): one fan-out-sampled bipartite block of a square A
+ * (rows == cols).  For destination v = dst[i] with deg = crow[v+1] - crow[v], k = deg if fanout == -1,
+ * else min(deg, fanout).  Entry j of row v (0-based) has the key
+ *     key(s, v, j) = mix(mix(s ^ v) + j)   (mod 2^64, compared unsigned; s = rng_seed)
+ * with mix = multiply by 0x9E3779B97F4A7C15, then the splitmix64 finaliser.  The k entries with the
+ * smallest (key, j) are selected: a uniform sample without replacement and a pure function of
+ * (rng_seed, v, j).  A selected entry whose column lies outside [0, cols) is dropped.
+ * Outputs (num_dst x num_src block, int32 blk_crow[num_dst+1] / blk_col):
+ *   - row i holds the kept entries of dst[i] in ascending j; blk_val (A's value dtype; non-NULL
+ *     exactly when A has values) holds val[crow[v] + j];
+ *   - blk_col are LOCAL ids into src_nodes (A's index dtype, room for num_dst + cap ids):
+ *     src_nodes = dst verbatim, then the distinct sampled ids that are not in dst, ascending;
+ *   - counts (device int64[3]): [0] = block nnz, [1] = num_src, [2] = invalid destinations (ids
+ *     outside [0, rows), and every occurrence of an id that occurs more than once; such a
+ *     destination reads nothing (degree 0) and the outputs are memory-safe but meaningless).
+ * `cap` is the capacity of blk_col / blk_val (cap >= 2^31-1: OFSPMM_ERR_TOO_LARGE).  If the sum of k
+ * exceeds it, counts[0] reports the size needed, nothing is written past any capacity and the outputs
+ * are invalid.  The workspace depends on (num_dst, cap) only, never on A's size.  num_dst == 0 writes
+ * blk_crow[0] = 0 and zero counts. */
+OFSPMM_API size_t ofspmm_sample_neighbors_workspace_bytes(int64_t num_dst, int64_t cap, int idx_dtype);
+OFSPMM_API int ofspmm_sample_neighbors(const ofspmm_csr* A, const void* dst, int64_t num_dst, int64_t fanout,
+                                       uint64_t rng_seed, int64_t cap, void* blk_crow, void* blk_col, void* blk_val,
+                                       void* src_nodes, int64_t* counts, void* workspace, size_t workspace_bytes,
+                                       ofspmm_stream_t stream);
+
 /* ---- Host-buffer convenience entry (what a CPU-tensor caller / the e2e benchmark uses): copies
  * the CSR arrays and B from HOST memory (pinned recommended) to device staging carved from
  * `workspace`, runs ofspmm_fwd, copies C back to `C_host`, all on `stream`; the caller

@@ -29,6 +29,7 @@ EXPORTS = (
     "ofspmm_gather_rows", "ofspmm_scatter_add_rows", "ofspmm_permute_values", "ofspmm_scatter_add_rows_f32",
     "ofspmm_cast_from_f32", "ofspmm_coo_to_csr_workspace_bytes", "ofspmm_coo_to_csr", "ofspmm_csr_expand_rows",
     "ofspmm_csr_normalize", "ofspmm_signal_peers", "ofspmm_pull_rows_multi", "ofspmm_combine_rows_multi",
+    "ofspmm_sample_neighbors_workspace_bytes", "ofspmm_sample_neighbors",
 )
 
 # ofspmm_opts.flags / variant codes (include/ofspmm.h)
@@ -171,6 +172,10 @@ def lib() -> ctypes.CDLL:
     L.ofspmm_gather_rows.restype = i32
     L.ofspmm_scatter_add_rows.argtypes = [vp, i64, vp, i64, vp, i32, i64, i64, i64, i32, i32, vp]
     L.ofspmm_scatter_add_rows.restype = i32
+    L.ofspmm_sample_neighbors_workspace_bytes.argtypes = [i64, i64, i32]
+    L.ofspmm_sample_neighbors_workspace_bytes.restype = sz
+    L.ofspmm_sample_neighbors.argtypes = [csr_p, vp, i64, i64, ctypes.c_uint64, i64, vp, vp, vp, vp, vp, vp, sz, vp]
+    L.ofspmm_sample_neighbors.restype = i32
     _LIB = L
     return L
 

@@ -405,6 +405,27 @@ int ofspmm_coo_to_csr(const int64_t* row, const int64_t* col, const float* val, 
                            workspace_bytes, reinterpret_cast<cudaStream_t>(stream));
 }
 
+size_t ofspmm_sample_neighbors_workspace_bytes(int64_t num_dst, int64_t cap, int idx_dtype) {
+  if (num_dst < 0 || cap < 0 || !idx_ok(idx_dtype)) return 0;
+  return sample_neighbors_workspace_bytes(num_dst, cap);
+}
+
+int ofspmm_sample_neighbors(const ofspmm_csr* A, const void* dst, int64_t num_dst, int64_t fanout, uint64_t rng_seed,
+                            int64_t cap, void* blk_crow, void* blk_col, void* blk_val, void* src_nodes, int64_t* counts,
+                            void* workspace, size_t workspace_bytes, ofspmm_stream_t stream) {
+  if (int rc = check_csr(A, true)) return rc;
+  if (A->rows != A->cols || fanout < -1 || num_dst < 0 || cap < 0) return OFSPMM_ERR_INVALID_ARG;
+  if (cap >= kWideNnz || num_dst >= kWideNnz) return OFSPMM_ERR_TOO_LARGE;   // int32 block offsets and local ids
+  if (blk_crow == nullptr || counts == nullptr) return OFSPMM_ERR_INVALID_ARG;
+  if (num_dst > 0 && (dst == nullptr || src_nodes == nullptr)) return OFSPMM_ERR_INVALID_ARG;
+  if (cap > 0 && (blk_col == nullptr || src_nodes == nullptr)) return OFSPMM_ERR_INVALID_ARG;
+  // a values array exactly when A has values (a forgotten value dtype is caught, not ignored)
+  if (unit(A) ? blk_val != nullptr : (cap > 0 && blk_val == nullptr)) return OFSPMM_ERR_INVALID_ARG;
+  if (int rc = check_ws(workspace, workspace_bytes, sample_neighbors_workspace_bytes(num_dst, cap))) return rc;
+  return launch_sample_neighbors(A, dst, num_dst, fanout, rng_seed, cap, blk_crow, blk_col, blk_val, src_nodes, counts,
+                                 workspace, reinterpret_cast<cudaStream_t>(stream));
+}
+
 int ofspmm_csr_expand_rows(const void* crow, int idx_dtype, int64_t rows, int64_t* row_of_nnz, ofspmm_stream_t stream) {
   if (rows < 0 || crow == nullptr || (rows > 0 && row_of_nnz == nullptr)) return OFSPMM_ERR_INVALID_ARG;
   if (!idx_ok(idx_dtype)) return OFSPMM_ERR_UNSUPPORTED_DTYPE;

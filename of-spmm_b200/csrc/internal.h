@@ -169,6 +169,10 @@ size_t coo_to_csr_workspace_bytes(int64_t n, int64_t rows, int64_t cols);
 int launch_coo_to_csr(const int64_t* row, const int64_t* col, const float* val, int64_t n, int64_t rows, int64_t cols,
                       int mode, int idx_dtype, void* crow, void* col_out, float* val_out, int64_t* counts, void* ws,
                       size_t ws_bytes, cudaStream_t stream);
+size_t sample_neighbors_workspace_bytes(int64_t num_dst, int64_t cap);
+int launch_sample_neighbors(const ofspmm_csr* A, const void* dst, int64_t num_dst, int64_t fanout, uint64_t seed,
+                            int64_t cap, void* blk_crow, void* blk_col, void* blk_val, void* src_nodes, int64_t* counts,
+                            void* ws, cudaStream_t stream);
 int launch_expand_rows(const void* crow, int idx_dtype, int64_t rows, int64_t* out, cudaStream_t stream);
 int launch_csr_normalize(const void* crow, const void* col, float* val, int idx_dtype, int64_t rows, int64_t cols, int mode,
                          float* dinv, cudaStream_t stream);

@@ -484,6 +484,54 @@ def csr_transpose(a_crow, a_col, a_val, a_rows: int, a_cols: int, want_perm: boo
     return (t_crow, t_col, t_val, t_perm) if want_perm else (t_crow, t_col, t_val)
 
 
+def sample_neighbors(a_crow, a_col, a_val, a_rows: int, a_cols: int, dst: torch.Tensor, fanout: int,
+                     rng_seed: int) -> Tuple[torch.Tensor, torch.Tensor, Optional[torch.Tensor], torch.Tensor]:
+    """One fan-out-sampled bipartite block of the square CSR A (``ofspmm_sample_neighbors``): for
+    each destination ``dst[i]``, at most ``fanout`` of its entries (all of them for -1), chosen by
+    the keys of include/ofspmm.h — uniform without replacement, a pure function of
+    (rng_seed, node, position).  Returns ``(blk_crow, blk_col, blk_val, src_nodes)``: an int32 CSR
+    of len(dst) x len(src_nodes) whose columns index ``src_nodes`` (dst first, then the other
+    sampled ids ascending); ``blk_val`` is None for a pattern matrix.  One device-to-host read (two
+    with fanout -1); invalid destinations (out of range, repeated) raise."""
+    _check_device(a_crow, a_col, a_val, dst)
+    _chk(a_crow.dim() == 1 and a_col.dim() == 1 and dst.dim() == 1, "a_crow, a_col and dst must be 1-D")
+    _chk(a_crow.dtype in _INDEX and a_col.dtype == a_crow.dtype, "a_crow / a_col must share an index dtype (int32/int64)")
+    _chk(a_rows == a_cols, f"neighbour sampling needs a square matrix, got {a_rows} x {a_cols}")
+    _chk(a_rows >= 0 and a_crow.numel() == a_rows + 1, f"a_crow must have a_rows+1 = {a_rows + 1} entries")
+    _chk(fanout >= -1, f"fanout must be >= 0, or -1 for all neighbours, got {fanout}")
+    if a_val is not None:
+        _chk(a_val.dim() == 1 and a_val.numel() == a_col.numel() and a_val.dtype in _DENSE,
+             "a_val must hold nnz float32 / bfloat16 values")
+    _chk(not dst.is_floating_point() and not dst.is_complex(), f"dst must hold node ids, got {dst.dtype}")
+    dev, idt = a_crow.device, a_crow.dtype
+    dst = dst.to(idt).contiguous()
+    num_dst, nnz = int(dst.numel()), int(a_col.numel())
+    if fanout == -1:
+        # the exact size: sum of the destinations' degrees (invalid ids count 0, read nothing)
+        ok = (dst >= 0) & (dst < a_rows)
+        d = torch.where(ok, dst, torch.zeros_like(dst)).long()
+        deg = (a_crow[1:][d] - a_crow[:-1][d]) * ok if a_rows > 0 else torch.zeros_like(d)
+        cap = int(deg.sum())
+    else:
+        cap = min(num_dst * fanout, nnz)   # at most one kept entry per non-zero of A
+    blk_crow = torch.empty(num_dst + 1, dtype=torch.int32, device=dev)
+    blk_col = torch.empty(cap, dtype=torch.int32, device=dev)
+    blk_val = torch.empty(cap, dtype=a_val.dtype, device=dev) if a_val is not None else None
+    src_nodes = torch.empty(num_dst + cap, dtype=idt, device=dev)
+    counts = torch.empty(3, dtype=torch.int64, device=dev)
+    L = _lib.lib()
+    with torch.cuda.device(dev):
+        A = _csr_struct(a_crow, a_col, a_val, a_rows, a_cols)
+        nbytes = L.ofspmm_sample_neighbors_workspace_bytes(num_dst, cap, _INDEX[idt])
+        ws, wsp = _workspace(nbytes, dev)
+        check(L.ofspmm_sample_neighbors(ctypes.byref(A), _ptr(dst), num_dst, fanout, rng_seed & (2 ** 64 - 1), cap,
+                                        _ptr(blk_crow), _ptr(blk_col), _ptr(blk_val), _ptr(src_nodes),
+                                        counts.data_ptr(), wsp, nbytes, _stream_ptr(dst)), "sample_neighbors")
+    nnz_blk, num_src, bad = counts.tolist()
+    _chk(bad == 0, f"sample_neighbors: {bad} destination ids are out of range [0, {a_rows}) or repeated")
+    return (blk_crow, blk_col[:nnz_blk], blk_val[:nnz_blk] if blk_val is not None else None, src_nodes[:num_src])
+
+
 def spmm_csr_grad_b_transient_compute(a_crow, a_col, a_val, dy, a_rows: int, a_cols: int,
                                       out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """db = A^T · dy through route (3) of the C ABI (``ofspmm_bwd_b_transient``): A^T is built
