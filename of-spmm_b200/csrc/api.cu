@@ -34,13 +34,13 @@ int get_dev_info(DevInfo* out) {
 FwdWorkspace fwd_workspace_layout(int64_t rows, int64_t nnz, int64_t n, int dense_dtype, int items) {
   FwdWorkspace L;
   const size_t P = static_cast<size_t>(num_tasks(rows, nnz, items));
-  L.counter_off = 0;  // task counter of the dynamic order (zeroed by a memset node before the launch)
-  L.part_off = 256;
-  L.carry_off = L.part_off + align_up((P + 1) * part_entry_bytes(nnz), 256);
-  const size_t rowbuf = align_up(P * static_cast<size_t>(n) * sizeof(float), 256);
-  L.head_off = L.carry_off + rowbuf;
-  L.total = L.head_off + (dense_dtype == OFSPMM_DTYPE_FLOAT ? 0 : rowbuf);
-  if (L.total == 0) L.total = 256;
+  const size_t rowbuf = P * static_cast<size_t>(n) * sizeof(float);
+  Carve c;
+  L.counter_off = c.take(256);  // task counter of the dynamic order (zeroed by a memset node before the launch)
+  L.part_off = c.take((P + 1) * part_entry_bytes(nnz));
+  L.carry_off = c.take(rowbuf);
+  L.head_off = c.take(dense_dtype == OFSPMM_DTYPE_FLOAT ? 0 : rowbuf);
+  L.total = c.total;
   return L;
 }
 
@@ -81,6 +81,37 @@ int check_dtypes(const ofspmm_csr* A, int dense_dtype) {
   return OFSPMM_OK;
 }
 
+// Checks of a product's A, dense dtype and width n.
+int check_product(const ofspmm_csr* A, bool need_val, int dense_dtype, int64_t n) {
+  if (int rc = check_csr(A, need_val)) return rc;
+  if (int rc = check_dtypes(A, dense_dtype)) return rc;
+  if (n < 0 || n >= (int64_t{1} << 31)) return OFSPMM_ERR_INVALID_ARG;
+  return OFSPMM_OK;
+}
+
+// Checks of the forward entry points: B may be NULL when no non-zero reads it.
+int check_fwd(const ofspmm_csr* A, const void* B, const void* C, int64_t n, int dense_dtype) {
+  if (int rc = check_product(A, true, dense_dtype, n)) return rc;
+  if (A->rows > 0 && n > 0 && (C == nullptr || (A->nnz > 0 && A->cols > 0 && B == nullptr))) return OFSPMM_ERR_INVALID_ARG;
+  return OFSPMM_OK;
+}
+
+// Checks of the A^T·dY entry points and the calls that need no product; *done: dB is complete,
+// because it has no elements or because A is empty and `zero_empty` zeroed it.
+int begin_bwd(const ofspmm_csr* A, const void* dY, void* dB, int64_t n, int dense_dtype, bool zero_empty,
+              cudaStream_t stream, bool* done) {
+  *done = true;
+  if (int rc = check_product(A, true, dense_dtype, n)) return rc;
+  if (A->cols == 0 || n == 0) return OFSPMM_OK;
+  if (dB == nullptr || (A->nnz > 0 && dY == nullptr)) return OFSPMM_ERR_INVALID_ARG;
+  if (zero_empty && (A->nnz == 0 || A->rows == 0)) {
+    OFSPMM_CUDA_OK(cudaMemsetAsync(dB, 0, static_cast<size_t>(A->cols) * n * dense_size(dense_dtype), stream));
+    return OFSPMM_OK;
+  }
+  *done = false;
+  return OFSPMM_OK;
+}
+
 int check_ws(const void* ws, size_t have, size_t need) {
   if (need == 0) return OFSPMM_OK;
   if (ws == nullptr || have < need) return OFSPMM_ERR_WORKSPACE;
@@ -96,6 +127,83 @@ size_t fwd_ws_auto(int64_t rows, int64_t nnz, int64_t n, int dense_dtype) {
 
 size_t plan_bytes_for(int64_t rows, int64_t nnz, int items) {
   return align_up((static_cast<size_t>(num_tasks(rows, nnz, items)) + 1) * part_entry_bytes(nnz), 256);
+}
+
+// Layout of the atomic route of ofspmm_bwd_b: [task partition | fp32 accumulator of a 16-bit dB]
+struct AtomicLayout {
+  size_t part, acc, total;
+};
+AtomicLayout atomic_layout(int64_t rows, int64_t cols, int64_t nnz, int64_t n, int dense_dtype) {
+  AtomicLayout L;
+  Carve c;
+  L.part = c.take(plan_bytes_for(rows, nnz, kTaskItems));
+  L.acc = c.take(dense_dtype == OFSPMM_DTYPE_FLOAT ? 0 : static_cast<size_t>(cols) * n * sizeof(float));
+  L.total = c.total;
+  return L;
+}
+
+// Layout of the transient-transpose route: [t_crow | t_col | t_val | transpose scratch | fwd scratch]
+struct TransientLayout {
+  size_t t_crow, t_col, t_val, tws, tws_bytes, fws, total;
+};
+TransientLayout transient_layout(int64_t rows, int64_t cols, int64_t nnz, int64_t n, int dense_dtype,
+                                 int idx_dtype, int val_dtype) {
+  TransientLayout L;
+  const size_t is = idx_size(idx_dtype), entries = static_cast<size_t>(nnz > 0 ? nnz : 1);
+  Carve c;
+  L.t_crow = c.take(static_cast<size_t>(cols + 1) * is);
+  L.t_col = c.take(entries * is);
+  L.t_val = c.take(entries * val_size(val_dtype));  // 0 for a pattern matrix
+  L.tws_bytes = transpose_workspace_bytes(rows, cols, nnz, idx_dtype);
+  L.tws = c.take(L.tws_bytes);
+  L.fws = c.take(fwd_ws_auto(cols, nnz, n, dense_dtype));
+  L.total = c.total;
+  return L;
+}
+
+// Layout of the cached-transpose route: [values of A^T | fwd scratch]
+struct CachedLayout {
+  size_t t_val, fws, total;
+};
+CachedLayout cached_layout(int64_t cols, int64_t nnz, int64_t n, int dense_dtype, int val_dtype) {
+  CachedLayout L;
+  Carve c;
+  L.t_val = c.take(static_cast<size_t>(nnz > 0 ? nnz : 1) * val_size(val_dtype));
+  L.fws = c.take(fwd_ws_auto(cols, nnz, n, dense_dtype));
+  L.total = c.total;
+  return L;
+}
+
+// Layout of the SDDMM: [task counter | task partition]
+struct SddmmLayout {
+  size_t counter, part, total;
+};
+SddmmLayout sddmm_layout(int64_t rows, int64_t nnz) {
+  SddmmLayout L;
+  Carve c;
+  L.counter = c.take(256);
+  L.part = c.take(plan_bytes_for(rows, nnz, kTaskItems));
+  L.total = c.total;
+  return L;
+}
+
+// Layout of ofspmm_fwd_host: [crow | col | val | B | C | fwd scratch], the operands staged on the device
+struct HostFwdLayout {
+  size_t crow, col, val, B, C, fws, total;
+};
+HostFwdLayout host_fwd_layout(int64_t rows, int64_t cols, int64_t nnz, int64_t n, int dense_dtype, int idx_dtype,
+                              int val_dtype) {
+  HostFwdLayout L;
+  const size_t is = idx_size(idx_dtype), ds = dense_size(dense_dtype);
+  Carve c;
+  L.crow = c.take(static_cast<size_t>(rows + 1) * is);
+  L.col = c.take(static_cast<size_t>(nnz) * is);
+  L.val = c.take(static_cast<size_t>(nnz) * val_size(val_dtype));
+  L.B = c.take(static_cast<size_t>(cols) * n * ds);
+  L.C = c.take(static_cast<size_t>(rows) * n * ds);
+  L.fws = c.take(fwd_ws_auto(rows, nnz, n, dense_dtype));
+  L.total = c.total;
+  return L;
 }
 
 // Options of one call -> launch description.  `opts` may be NULL (all defaults).
@@ -186,10 +294,7 @@ size_t ofspmm_fwd_ex_workspace_bytes(int64_t rows, int64_t cols, int64_t nnz, in
 int ofspmm_fwd_ex(const ofspmm_csr* A, const void* B, int64_t ldb, void* C, int64_t ldc, int64_t n,
                   int dense_dtype, const ofspmm_opts* opts, void* workspace, size_t workspace_bytes,
                   ofspmm_stream_t stream) {
-  if (int rc = check_csr(A, true)) return rc;
-  if (int rc = check_dtypes(A, dense_dtype)) return rc;
-  if (n < 0 || n >= (int64_t{1} << 31)) return OFSPMM_ERR_INVALID_ARG;
-  if (A->rows > 0 && n > 0 && (C == nullptr || (A->nnz > 0 && A->cols > 0 && B == nullptr))) return OFSPMM_ERR_INVALID_ARG;
+  if (int rc = check_fwd(A, B, C, n, dense_dtype)) return rc;
   return run_fwd(A, B, ldb, C, ldc, n, dense_dtype, opts, workspace, workspace_bytes, reinterpret_cast<cudaStream_t>(stream));
 }
 
@@ -243,39 +348,27 @@ int ofspmm_choose_variant(const int64_t* hist32_host, int64_t rows, int64_t nnz,
 
 int ofspmm_fwd(const ofspmm_csr* A, const void* B, void* C, int64_t n, int dense_dtype, void* workspace,
                size_t workspace_bytes, ofspmm_stream_t stream) {
-  if (int rc = check_csr(A, true)) return rc;
-  if (int rc = check_dtypes(A, dense_dtype)) return rc;
-  if (n < 0 || n >= (int64_t{1} << 31)) return OFSPMM_ERR_INVALID_ARG;
-  if (A->rows > 0 && n > 0 && (C == nullptr || (A->nnz > 0 && A->cols > 0 && B == nullptr))) return OFSPMM_ERR_INVALID_ARG;
-  return run_fwd(A, B, n, C, n, n, dense_dtype, nullptr, workspace, workspace_bytes, reinterpret_cast<cudaStream_t>(stream));
+  return ofspmm_fwd_ex(A, B, n, C, n, n, dense_dtype, nullptr, workspace, workspace_bytes, stream);
 }
 
 int ofspmm_fwd_strided(const ofspmm_csr* A, const void* B, int64_t ldb, void* C, int64_t ldc, int64_t n,
                        int dense_dtype, void* workspace, size_t workspace_bytes, ofspmm_stream_t stream) {
-  if (int rc = check_csr(A, true)) return rc;
-  if (int rc = check_dtypes(A, dense_dtype)) return rc;
-  if (n < 0 || n >= (int64_t{1} << 31)) return OFSPMM_ERR_INVALID_ARG;
-  if (A->rows > 0 && n > 0 && (C == nullptr || (A->nnz > 0 && A->cols > 0 && B == nullptr))) return OFSPMM_ERR_INVALID_ARG;
-  return run_fwd(A, B, ldb, C, ldc, n, dense_dtype, nullptr, workspace, workspace_bytes, reinterpret_cast<cudaStream_t>(stream));
+  return ofspmm_fwd_ex(A, B, ldb, C, ldc, n, dense_dtype, nullptr, workspace, workspace_bytes, stream);
 }
 
 size_t ofspmm_bwd_b_workspace_bytes(int64_t rows, int64_t cols, int64_t nnz, int64_t n, int dense_dtype,
                                     int have_transpose) {
   if (rows < 0 || cols < 0 || nnz < 0 || n < 0) return 0;
   if (have_transpose) return fwd_ws_auto(cols, nnz, n, dense_dtype);
-  size_t total = plan_bytes_for(rows, nnz, kTaskItems);
-  if (dense_dtype != OFSPMM_DTYPE_FLOAT) total += align_up(static_cast<size_t>(cols) * n * sizeof(float), 256);
-  return total;
+  return atomic_layout(rows, cols, nnz, n, dense_dtype).total;
 }
 
 int ofspmm_bwd_b(const ofspmm_csr* A, const ofspmm_csr* At, const void* dY, void* dB, int64_t n,
                  int dense_dtype, void* workspace, size_t workspace_bytes, ofspmm_stream_t stream_) {
   cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
-  if (int rc = check_csr(A, true)) return rc;
-  if (int rc = check_dtypes(A, dense_dtype)) return rc;
-  if (n < 0 || n >= (int64_t{1} << 31)) return OFSPMM_ERR_INVALID_ARG;
-  if (A->cols == 0 || n == 0) return OFSPMM_OK;
-  if (dB == nullptr || (A->nnz > 0 && dY == nullptr)) return OFSPMM_ERR_INVALID_ARG;
+  bool done;
+  // route (1) runs the forward kernel on A^T even when A is empty
+  if (int rc = begin_bwd(A, dY, dB, n, dense_dtype, At == nullptr, stream, &done); rc != OFSPMM_OK || done) return rc;
   if (At != nullptr) {  // route (1): forward kernel on the cached transpose
     if (int rc = check_csr(At, true)) return rc;
     if (At->rows != A->cols || At->cols != A->rows || At->nnz != A->nnz) return OFSPMM_ERR_INVALID_ARG;
@@ -283,42 +376,15 @@ int ofspmm_bwd_b(const ofspmm_csr* A, const ofspmm_csr* At, const void* dY, void
     return run_fwd(At, dY, n, dB, n, n, dense_dtype, nullptr, workspace, workspace_bytes, stream);
   }
   // route (2): vector-atomic scatter into an fp32 accumulator
-  const size_t out_elems = static_cast<size_t>(A->cols) * static_cast<size_t>(n);
-  if (A->nnz == 0 || A->rows == 0) {
-    OFSPMM_CUDA_OK(cudaMemsetAsync(dB, 0, out_elems * dense_size(dense_dtype), stream));
-    return OFSPMM_OK;
-  }
-  const size_t need = ofspmm_bwd_b_workspace_bytes(A->rows, A->cols, A->nnz, n, dense_dtype, 0);
-  if (int rc = check_ws(workspace, workspace_bytes, need)) return rc;
+  const AtomicLayout L = atomic_layout(A->rows, A->cols, A->nnz, n, dense_dtype);
+  if (int rc = check_ws(workspace, workspace_bytes, L.total)) return rc;
   unsigned char* w = static_cast<unsigned char*>(workspace);
   const int64_t P = num_tasks(A->rows, A->nnz);
-  const size_t part_bytes = plan_bytes_for(A->rows, A->nnz, kTaskItems);
-  if (int rc = launch_task_partition(A->crow, A->idx_dtype, A->rows, A->nnz, P, kTaskItems, w, stream)) return rc;
+  if (int rc = launch_task_partition(A->crow, A->idx_dtype, A->rows, A->nnz, P, kTaskItems, w + L.part, stream)) return rc;
   if (dense_dtype == OFSPMM_DTYPE_FLOAT)
-    return launch_bwd_atomic(A, dY, static_cast<float*>(dB), nullptr, n, dense_dtype, w, P, stream);
-  return launch_bwd_atomic(A, dY, reinterpret_cast<float*>(w + part_bytes), dB, n, dense_dtype, w, P, stream);
+    return launch_bwd_atomic(A, dY, static_cast<float*>(dB), nullptr, n, dense_dtype, w + L.part, P, stream);
+  return launch_bwd_atomic(A, dY, reinterpret_cast<float*>(w + L.acc), dB, n, dense_dtype, w + L.part, P, stream);
 }
-
-// Layout of the transient-transpose route: [t_crow | t_col | t_val | transpose scratch | fwd scratch]
-namespace {
-struct TransientLayout {
-  size_t t_crow, t_col, t_val, tws, tws_bytes, fws, total;
-};
-TransientLayout transient_layout(int64_t rows, int64_t cols, int64_t nnz, int64_t n, int dense_dtype,
-                                 int idx_dtype, int val_dtype) {
-  TransientLayout L;
-  const size_t is = idx_size(idx_dtype), vs = val_size(val_dtype);
-  size_t off = 0;
-  L.t_crow = off; off += align_up(static_cast<size_t>(cols + 1) * is, 256);
-  L.t_col = off;  off += align_up(static_cast<size_t>(nnz > 0 ? nnz : 1) * is, 256);
-  L.t_val = off;  off += align_up(static_cast<size_t>(nnz > 0 ? nnz : 1) * vs, 256);  // 0 for a pattern matrix
-  L.tws = off;    L.tws_bytes = transpose_workspace_bytes(rows, cols, nnz, idx_dtype);
-  off += align_up(L.tws_bytes, 256);
-  L.fws = off;    off += fwd_ws_auto(cols, nnz, n, dense_dtype);
-  L.total = off;
-  return L;
-}
-}  // namespace
 
 size_t ofspmm_bwd_b_transient_workspace_bytes(int64_t rows, int64_t cols, int64_t nnz, int64_t n,
                                               int dense_dtype, int idx_dtype, int val_dtype) {
@@ -329,15 +395,8 @@ size_t ofspmm_bwd_b_transient_workspace_bytes(int64_t rows, int64_t cols, int64_
 int ofspmm_bwd_b_transient(const ofspmm_csr* A, const void* dY, void* dB, int64_t n, int dense_dtype,
                            void* workspace, size_t workspace_bytes, ofspmm_stream_t stream_) {
   cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
-  if (int rc = check_csr(A, true)) return rc;
-  if (int rc = check_dtypes(A, dense_dtype)) return rc;
-  if (n < 0 || n >= (int64_t{1} << 31)) return OFSPMM_ERR_INVALID_ARG;
-  if (A->cols == 0 || n == 0) return OFSPMM_OK;
-  if (dB == nullptr || (A->nnz > 0 && dY == nullptr)) return OFSPMM_ERR_INVALID_ARG;
-  if (A->nnz == 0 || A->rows == 0) {
-    OFSPMM_CUDA_OK(cudaMemsetAsync(dB, 0, static_cast<size_t>(A->cols) * n * dense_size(dense_dtype), stream));
-    return OFSPMM_OK;
-  }
+  bool done;
+  if (int rc = begin_bwd(A, dY, dB, n, dense_dtype, true, stream, &done); rc != OFSPMM_OK || done) return rc;
   const TransientLayout L = transient_layout(A->rows, A->cols, A->nnz, n, dense_dtype, A->idx_dtype, A->val_dtype);
   if (int rc = check_ws(workspace, workspace_bytes, L.total)) return rc;
   unsigned char* w = static_cast<unsigned char*>(workspace);
@@ -355,36 +414,32 @@ int ofspmm_bwd_b_transient(const ofspmm_csr* A, const void* dY, void* dB, int64_
 size_t ofspmm_bwd_b_cached_workspace_bytes(int64_t rows, int64_t cols, int64_t nnz, int64_t n, int dense_dtype,
                                           int val_dtype) {
   if (rows < 0 || cols < 0 || nnz < 0 || n < 0) return 0;
-  const size_t vs = val_size(val_dtype);
-  return align_up(static_cast<size_t>(nnz > 0 ? nnz : 1) * vs, 256) + fwd_ws_auto(cols, nnz, n, dense_dtype);
+  return cached_layout(cols, nnz, n, dense_dtype, val_dtype).total;
 }
 
 int ofspmm_bwd_b_cached(const ofspmm_csr* A, const void* t_crow, const void* t_col, const void* t_perm,
                         const void* dY, void* dB, int64_t n, int dense_dtype, const ofspmm_opts* opts,
                         void* workspace, size_t workspace_bytes, ofspmm_stream_t stream_) {
   cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
-  if (int rc = check_csr(A, true)) return rc;
-  if (int rc = check_dtypes(A, dense_dtype)) return rc;
-  if (n < 0 || n >= (int64_t{1} << 31)) return OFSPMM_ERR_INVALID_ARG;
-  if (A->cols == 0 || n == 0) return OFSPMM_OK;
-  if (dB == nullptr || t_crow == nullptr || (A->nnz > 0 && (dY == nullptr || t_col == nullptr || t_perm == nullptr)))
-    return OFSPMM_ERR_INVALID_ARG;
-  const size_t tv_bytes = align_up(static_cast<size_t>(A->nnz > 0 ? A->nnz : 1) * val_size(A->val_dtype), 256);
-  const size_t need = ofspmm_bwd_b_cached_workspace_bytes(A->rows, A->cols, A->nnz, n, dense_dtype, A->val_dtype);
-  if (int rc = check_ws(workspace, workspace_bytes, need)) return rc;
+  bool done;
+  // an empty A runs the forward kernel, which writes the zeros of dB
+  if (int rc = begin_bwd(A, dY, dB, n, dense_dtype, false, stream, &done); rc != OFSPMM_OK || done) return rc;
+  if (t_crow == nullptr || (A->nnz > 0 && (t_col == nullptr || t_perm == nullptr))) return OFSPMM_ERR_INVALID_ARG;
+  const CachedLayout L = cached_layout(A->cols, A->nnz, n, dense_dtype, A->val_dtype);
+  if (int rc = check_ws(workspace, workspace_bytes, L.total)) return rc;
   unsigned char* w = static_cast<unsigned char*>(workspace);
   // the STRUCTURE of A^T is cached by the caller; the values are re-gathered from A on every call,
   // so in-place updates of a_val (learnable edge weights) are always seen.  A pattern matrix has
   // nothing to gather.
   if (!unit(A))
-    if (int rc = launch_gather_vals(A->val, A->val_dtype, t_perm, A->idx_dtype, A->nnz, w, stream)) return rc;
+    if (int rc = launch_gather_vals(A->val, A->val_dtype, t_perm, A->idx_dtype, A->nnz, w + L.t_val, stream)) return rc;
   ofspmm_csr At = *A;
   At.rows = A->cols;
   At.cols = A->rows;
   At.crow = t_crow;
   At.col = t_col;
-  At.val = unit(A) ? nullptr : w;
-  return run_fwd(&At, dY, n, dB, n, n, dense_dtype, opts, w + tv_bytes, workspace_bytes - tv_bytes, stream);
+  At.val = unit(A) ? nullptr : w + L.t_val;
+  return run_fwd(&At, dY, n, dB, n, n, dense_dtype, opts, w + L.fws, workspace_bytes - L.fws, stream);
 }
 
 size_t ofspmm_coo_to_csr_workspace_bytes(int64_t nnz_in, int64_t rows, int64_t cols) {
@@ -512,7 +567,7 @@ int ofspmm_scatter_add_rows(void* dst, int64_t ld_dst, const void* src, int64_t 
 size_t ofspmm_sddmm_workspace_bytes(int64_t rows, int64_t cols, int64_t nnz, int64_t n, int dense_dtype) {
   (void)cols; (void)n; (void)dense_dtype;
   if (rows < 0 || nnz < 0) return 0;
-  return 256 + plan_bytes_for(rows, nnz, kTaskItems);  // [task counter | task partition]
+  return sddmm_layout(rows, nnz).total;
 }
 
 int ofspmm_sddmm(const ofspmm_csr* A, const void* dY, const void* B, void* dval, int64_t n, int dense_dtype,
@@ -525,9 +580,7 @@ int ofspmm_sddmm_ex(const ofspmm_csr* A, const void* dY, const void* B, void* dv
   cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
   // val_dtype is the dtype of the output dval here: a pattern matrix has no values to differentiate
   if (A != nullptr && unit(A)) return OFSPMM_ERR_UNSUPPORTED_DTYPE;
-  if (int rc = check_csr(A, false)) return rc;
-  if (int rc = check_dtypes(A, dense_dtype)) return rc;
-  if (n < 0 || n >= (int64_t{1} << 31)) return OFSPMM_ERR_INVALID_ARG;
+  if (int rc = check_product(A, false, dense_dtype, n)) return rc;
   if (A->nnz == 0) return OFSPMM_OK;
   if (dval == nullptr) return OFSPMM_ERR_INVALID_ARG;
   const size_t val_size = A->val_dtype == OFSPMM_DTYPE_FLOAT ? 4 : 2;
@@ -537,17 +590,17 @@ int ofspmm_sddmm_ex(const ofspmm_csr* A, const void* dY, const void* B, void* dv
   }
   if (dY == nullptr || B == nullptr) return OFSPMM_ERR_INVALID_ARG;
   const int64_t P = num_tasks(A->rows, A->nnz);
-  const size_t need = ofspmm_sddmm_workspace_bytes(A->rows, A->cols, A->nnz, n, dense_dtype);
-  if (int rc = check_ws(workspace, workspace_bytes, need)) return rc;
+  const SddmmLayout L = sddmm_layout(A->rows, A->nnz);
+  if (int rc = check_ws(workspace, workspace_bytes, L.total)) return rc;
   unsigned char* w = static_cast<unsigned char*>(workspace);
   const uint32_t fl = opts ? opts->flags : 0u;
   const bool dynamic = OFSPMM_DEFAULT_DYNAMIC_ORDER ? (fl & OFSPMM_ORDER_STATIC) == 0 : (fl & OFSPMM_ORDER_DYNAMIC) != 0;
-  void* counter = dynamic ? w : nullptr;
+  void* counter = dynamic ? w + L.counter : nullptr;
   // the SDDMM kernels use 256-item tasks: a plan of that task size is taken as is
   if (opts != nullptr && opts->plan != nullptr && opts->plan_bytes == plan_bytes_for(A->rows, A->nnz, kTaskItems))
     return launch_sddmm(A, dY, B, dval, n, dense_dtype, opts->plan, counter, P, stream);
-  if (int rc = launch_task_partition(A->crow, A->idx_dtype, A->rows, A->nnz, P, kTaskItems, w + 256, stream)) return rc;
-  return launch_sddmm(A, dY, B, dval, n, dense_dtype, w + 256, counter, P, stream);
+  if (int rc = launch_task_partition(A->crow, A->idx_dtype, A->rows, A->nnz, P, kTaskItems, w + L.part, stream)) return rc;
+  return launch_sddmm(A, dY, B, dval, n, dense_dtype, w + L.part, counter, P, stream);
 }
 
 int ofspmm_partition(const void* crow, int idx_dtype, int64_t rows, int64_t nnz, int64_t parts,
@@ -601,52 +654,33 @@ int ofspmm_csr_transpose(const ofspmm_csr* A, void* t_crow, void* t_col, void* t
 size_t ofspmm_fwd_host_workspace_bytes(int64_t rows, int64_t cols, int64_t nnz, int64_t n, int dense_dtype,
                                        int idx_dtype, int val_dtype) {
   if (rows < 0 || cols < 0 || nnz < 0 || n < 0) return 0;
-  const size_t vs = val_size(val_dtype);
-  size_t total = 0;
-  total += align_up(static_cast<size_t>(rows + 1) * idx_size(idx_dtype), 256);
-  total += align_up(static_cast<size_t>(nnz) * idx_size(idx_dtype), 256);
-  total += align_up(static_cast<size_t>(nnz) * vs, 256);
-  total += align_up(static_cast<size_t>(cols) * n * dense_size(dense_dtype), 256);
-  total += align_up(static_cast<size_t>(rows) * n * dense_size(dense_dtype), 256);
-  total += fwd_ws_auto(rows, nnz, n, dense_dtype);
-  return total;
+  return host_fwd_layout(rows, cols, nnz, n, dense_dtype, idx_dtype, val_dtype).total;
 }
 
 int ofspmm_fwd_host(const ofspmm_csr* Ah, const void* B_host, void* C_host, int64_t n, int dense_dtype,
                     void* workspace, size_t workspace_bytes, ofspmm_stream_t stream_) {
   cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
-  if (int rc = check_csr(Ah, true)) return rc;
-  if (int rc = check_dtypes(Ah, dense_dtype)) return rc;
-  if (n < 0 || n >= (int64_t{1} << 31)) return OFSPMM_ERR_INVALID_ARG;
+  if (int rc = check_fwd(Ah, B_host, C_host, n, dense_dtype)) return rc;
   if (Ah->rows == 0 || n == 0) return OFSPMM_OK;
-  if (C_host == nullptr || (Ah->nnz > 0 && Ah->cols > 0 && B_host == nullptr)) return OFSPMM_ERR_INVALID_ARG;
-  const size_t need = ofspmm_fwd_host_workspace_bytes(Ah->rows, Ah->cols, Ah->nnz, n, dense_dtype,
-                                                      Ah->idx_dtype, Ah->val_dtype);
-  if (int rc = check_ws(workspace, workspace_bytes, need)) return rc;
+  const HostFwdLayout L = host_fwd_layout(Ah->rows, Ah->cols, Ah->nnz, n, dense_dtype, Ah->idx_dtype, Ah->val_dtype);
+  if (int rc = check_ws(workspace, workspace_bytes, L.total)) return rc;
   const size_t is = idx_size(Ah->idx_dtype), vs = val_size(Ah->val_dtype);
   const size_t ds = dense_size(dense_dtype);
   unsigned char* w = static_cast<unsigned char*>(workspace);
-  size_t off = 0;
-  auto carve = [&](size_t bytes) { void* p = w + off; off += align_up(bytes, 256); return p; };
-  void* d_crow = carve(static_cast<size_t>(Ah->rows + 1) * is);
-  void* d_col = carve(static_cast<size_t>(Ah->nnz) * is);
-  void* d_val = carve(static_cast<size_t>(Ah->nnz) * vs);
-  void* d_B = carve(static_cast<size_t>(Ah->cols) * n * ds);
-  void* d_C = carve(static_cast<size_t>(Ah->rows) * n * ds);
-  OFSPMM_CUDA_OK(cudaMemcpyAsync(d_crow, Ah->crow, static_cast<size_t>(Ah->rows + 1) * is, cudaMemcpyHostToDevice, stream));
+  OFSPMM_CUDA_OK(cudaMemcpyAsync(w + L.crow, Ah->crow, static_cast<size_t>(Ah->rows + 1) * is, cudaMemcpyHostToDevice, stream));
   if (Ah->nnz > 0) {
-    OFSPMM_CUDA_OK(cudaMemcpyAsync(d_col, Ah->col, static_cast<size_t>(Ah->nnz) * is, cudaMemcpyHostToDevice, stream));
+    OFSPMM_CUDA_OK(cudaMemcpyAsync(w + L.col, Ah->col, static_cast<size_t>(Ah->nnz) * is, cudaMemcpyHostToDevice, stream));
     if (!unit(Ah))
-      OFSPMM_CUDA_OK(cudaMemcpyAsync(d_val, Ah->val, static_cast<size_t>(Ah->nnz) * vs, cudaMemcpyHostToDevice, stream));
+      OFSPMM_CUDA_OK(cudaMemcpyAsync(w + L.val, Ah->val, static_cast<size_t>(Ah->nnz) * vs, cudaMemcpyHostToDevice, stream));
   }
   if (Ah->cols > 0 && B_host != nullptr)
-    OFSPMM_CUDA_OK(cudaMemcpyAsync(d_B, B_host, static_cast<size_t>(Ah->cols) * n * ds, cudaMemcpyHostToDevice, stream));
+    OFSPMM_CUDA_OK(cudaMemcpyAsync(w + L.B, B_host, static_cast<size_t>(Ah->cols) * n * ds, cudaMemcpyHostToDevice, stream));
   ofspmm_csr Ad = *Ah;
-  Ad.crow = d_crow;
-  Ad.col = d_col;
-  Ad.val = unit(Ah) ? nullptr : d_val;
-  if (int rc = run_fwd(&Ad, d_B, n, d_C, n, n, dense_dtype, nullptr, w + off, workspace_bytes - off, stream)) return rc;
-  OFSPMM_CUDA_OK(cudaMemcpyAsync(C_host, d_C, static_cast<size_t>(Ah->rows) * n * ds, cudaMemcpyDeviceToHost, stream));
+  Ad.crow = w + L.crow;
+  Ad.col = w + L.col;
+  Ad.val = unit(Ah) ? nullptr : w + L.val;
+  if (int rc = run_fwd(&Ad, w + L.B, n, w + L.C, n, n, dense_dtype, nullptr, w + L.fws, workspace_bytes - L.fws, stream)) return rc;
+  OFSPMM_CUDA_OK(cudaMemcpyAsync(C_host, w + L.C, static_cast<size_t>(Ah->rows) * n * ds, cudaMemcpyDeviceToHost, stream));
   return OFSPMM_OK;
 }
 

@@ -11,8 +11,7 @@
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 
-#include "common.cuh"
-#include "internal.h"
+#include "launch.cuh"
 
 namespace ofspmm {
 
@@ -150,16 +149,16 @@ struct CooLayout {
 
 CooLayout coo_layout(int64_t n, int64_t rows, int64_t cols) {
   CooLayout L;
-  const size_t a64 = align_up(static_cast<size_t>(n > 0 ? n : 1) * sizeof(long long), 256);
-  const size_t a32 = align_up(static_cast<size_t>(n > 0 ? n : 1) * sizeof(int), 256);
-  size_t off = 0;
-  L.keys_in = off; off += a64;
-  L.keys_out = off; off += a64;
-  L.idx_in = off; off += a64;
-  L.perm = off; off += a64;
-  L.ukeys = off; off += a64;
-  L.flag = off; off += a32;
-  L.pos = off; off += a32;
+  const size_t a64 = static_cast<size_t>(n > 0 ? n : 1) * sizeof(long long);
+  const size_t a32 = static_cast<size_t>(n > 0 ? n : 1) * sizeof(int);
+  Carve c;
+  L.keys_in = c.take(a64);
+  L.keys_out = c.take(a64);
+  L.idx_in = c.take(a64);
+  L.perm = c.take(a64);
+  L.ukeys = c.take(a64);
+  L.flag = c.take(a32);
+  L.pos = c.take(a32);
   size_t sort_bytes = 0, scan_bytes = 0;
   cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, static_cast<const long long*>(nullptr), static_cast<long long*>(nullptr),
                                   static_cast<const long long*>(nullptr), static_cast<long long*>(nullptr),
@@ -167,8 +166,8 @@ CooLayout coo_layout(int64_t n, int64_t rows, int64_t cols) {
   cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, static_cast<const int*>(nullptr), static_cast<int*>(nullptr),
                                 static_cast<long long>(n));
   L.cub_bytes = sort_bytes > scan_bytes ? sort_bytes : scan_bytes;
-  L.cub_tmp = off; off += align_up(L.cub_bytes, 256);
-  L.total = off;
+  L.cub_tmp = c.take(L.cub_bytes);
+  L.total = c.total;
   return L;
 }
 
@@ -207,9 +206,7 @@ int coo_impl(const int64_t* row, const int64_t* col, const float* val, int64_t n
   }
   coo_offsets_kernel<IdxT><<<static_cast<unsigned>((rows + 1 + 255) / 256), 256, 0, stream>>>(
       ukeys, keys_out, flag, pos, n, rows, cols, static_cast<IdxT*>(crow), reinterpret_cast<long long*>(counts));
-  count_launch();
-  OFSPMM_CUDA_OK(cudaGetLastError());
-  return OFSPMM_OK;
+  return launched();
 }
 
 }  // namespace
@@ -220,9 +217,10 @@ int launch_coo_to_csr(const int64_t* row, const int64_t* col, const float* val, 
                       int mode, int idx_dtype, void* crow, void* col_out, float* val_out, int64_t* counts, void* ws,
                       size_t ws_bytes, cudaStream_t stream) {
   if (ws == nullptr || ws_bytes < coo_layout(n, rows, cols).total) return OFSPMM_ERR_WORKSPACE;
-  if (idx_dtype == OFSPMM_DTYPE_INT32) return coo_impl<int32_t>(row, col, val, n, rows, cols, mode, crow, col_out, val_out, counts, ws, stream);
-  if (idx_dtype == OFSPMM_DTYPE_INT64) return coo_impl<int64_t>(row, col, val, n, rows, cols, mode, crow, col_out, val_out, counts, ws, stream);
-  return OFSPMM_ERR_UNSUPPORTED_DTYPE;
+  return dispatch_idx(idx_dtype, [&](auto idx) {
+    return coo_impl<typename decltype(idx)::type>(row, col, val, n, rows, cols, mode, crow, col_out, val_out, counts, ws,
+                                                  stream);
+  });
 }
 
 int launch_expand_rows(const void* crow, int idx_dtype, int64_t rows, int64_t* out, cudaStream_t stream) {
@@ -230,12 +228,11 @@ int launch_expand_rows(const void* crow, int idx_dtype, int64_t rows, int64_t* o
   DevInfo dev;
   if (int rc = get_dev_info(&dev)) return rc;
   const int grid = dev.sms * 8;
-  if (idx_dtype == OFSPMM_DTYPE_INT32) expand_rows_kernel<int32_t><<<grid, 256, 0, stream>>>(static_cast<const int32_t*>(crow), rows, reinterpret_cast<long long*>(out));
-  else if (idx_dtype == OFSPMM_DTYPE_INT64) expand_rows_kernel<int64_t><<<grid, 256, 0, stream>>>(static_cast<const int64_t*>(crow), rows, reinterpret_cast<long long*>(out));
-  else return OFSPMM_ERR_UNSUPPORTED_DTYPE;
-  count_launch();
-  OFSPMM_CUDA_OK(cudaGetLastError());
-  return OFSPMM_OK;
+  return dispatch_idx(idx_dtype, [&](auto idx) {
+    using IdxT = typename decltype(idx)::type;
+    expand_rows_kernel<IdxT><<<grid, 256, 0, stream>>>(static_cast<const IdxT*>(crow), rows, reinterpret_cast<long long*>(out));
+    return launched();
+  });
 }
 
 int launch_csr_normalize(const void* crow, const void* col, float* val, int idx_dtype, int64_t rows, int64_t cols, int mode,
@@ -244,18 +241,13 @@ int launch_csr_normalize(const void* crow, const void* col, float* val, int idx_
   DevInfo dev;
   if (int rc = get_dev_info(&dev)) return rc;
   const int grid = dev.sms * 8;
-  if (idx_dtype == OFSPMM_DTYPE_INT32) {
-    row_dinv_kernel<int32_t><<<grid, 256, 0, stream>>>(static_cast<const int32_t*>(crow), val, rows, mode, dinv);
-    scale_kernel<int32_t><<<grid, 256, 0, stream>>>(static_cast<const int32_t*>(crow), static_cast<const int32_t*>(col), rows, cols, mode, dinv, val);
-  } else if (idx_dtype == OFSPMM_DTYPE_INT64) {
-    row_dinv_kernel<int64_t><<<grid, 256, 0, stream>>>(static_cast<const int64_t*>(crow), val, rows, mode, dinv);
-    scale_kernel<int64_t><<<grid, 256, 0, stream>>>(static_cast<const int64_t*>(crow), static_cast<const int64_t*>(col), rows, cols, mode, dinv, val);
-  } else {
-    return OFSPMM_ERR_UNSUPPORTED_DTYPE;
-  }
-  count_launch(2);
-  OFSPMM_CUDA_OK(cudaGetLastError());
-  return OFSPMM_OK;
+  return dispatch_idx(idx_dtype, [&](auto idx) {
+    using IdxT = typename decltype(idx)::type;
+    row_dinv_kernel<IdxT><<<grid, 256, 0, stream>>>(static_cast<const IdxT*>(crow), val, rows, mode, dinv);
+    scale_kernel<IdxT><<<grid, 256, 0, stream>>>(static_cast<const IdxT*>(crow), static_cast<const IdxT*>(col), rows, cols,
+                                                 mode, dinv, val);
+    return launched(2);
+  });
 }
 
 }  // namespace ofspmm

@@ -62,16 +62,13 @@ int launch_bwd_atomic(const ofspmm_csr* A, const void* dY, float* acc, void* dB_
                           typename decltype(part)::type>(p, l, stream);
     });
   });
-  if (rc != OFSPMM_OK) return rc;
-  if (dB_cast_out != nullptr) {  // bf16 output: cast the fp32 accumulator once
-    DevInfo dev;
-    if (int rc2 = get_dev_info(&dev)) return rc2;
-    cast_from_f32_kernel<__nv_bfloat16><<<dev.sms * 8, 256, 0, stream>>>(
-        acc, static_cast<__nv_bfloat16*>(dB_cast_out), static_cast<long long>(out_elems));
-    count_launch();
-    OFSPMM_CUDA_OK(cudaGetLastError());
-  }
-  return OFSPMM_OK;
+  if (rc != OFSPMM_OK || dB_cast_out == nullptr) return rc;
+  // bf16 output: cast the fp32 accumulator once
+  DevInfo dev;
+  if (int rc2 = get_dev_info(&dev)) return rc2;
+  cast_from_f32_kernel<__nv_bfloat16><<<dev.sms * 8, 256, 0, stream>>>(
+      acc, static_cast<__nv_bfloat16*>(dB_cast_out), static_cast<long long>(out_elems));
+  return launched();
 }
 
 }  // namespace ofspmm

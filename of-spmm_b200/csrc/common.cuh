@@ -91,6 +91,15 @@ template <> __device__ __forceinline__ __nv_bfloat16 from_float<__nv_bfloat16>(f
   return __float2bfloat16_rn(v);
 }
 
+// out[i] = DT(in[i]) — the cast that follows an fp32 accumulation for bf16 outputs
+// (reference idiom: oneflow/user/kernels/unsorted_segment_sum_kernel.cpp:162-186).
+template <typename DT>
+__global__ void cast_from_f32_kernel(const float* __restrict__ in, DT* __restrict__ out, long long count) {
+  const long long stride = static_cast<long long>(gridDim.x) * blockDim.x;
+  for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < count; i += stride)
+    out[i] = from_float<DT>(in[i]);
+}
+
 // ---------------------------------------------------------------- VEC-wide dense row access
 // VEC elements of DT per lane: 16 bytes when vectorised (4 x fp32 / 8 x bf16) or 1 element.
 

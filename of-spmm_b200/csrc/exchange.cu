@@ -25,8 +25,7 @@
 // Peer loads see ~2 us of latency: the register kernels keep UNROLL independent 16-byte units in
 // flight per thread, and every grid is capped (`max_ctas`) so the copy shares the GPU with the
 // SpMM kernel it overlaps.
-#include "common.cuh"
-#include "internal.h"
+#include "launch.cuh"
 
 namespace ofspmm {
 
@@ -195,13 +194,6 @@ __global__ void scatter_add_rows_bf16_to_f32_scalar_kernel(float* __restrict__ d
     const int c = static_cast<int>(u - r * n);
     dst[list_at(list, r, off) * ld_dst + c] += to_float(*static_cast<const volatile __nv_bfloat16*>(src + r * ld_src + c));
   }
-}
-
-template <typename DT>
-__global__ void cast_rows_from_f32_kernel(const float* __restrict__ in, DT* __restrict__ out, long long count) {
-  const long long stride = static_cast<long long>(gridDim.x) * blockDim.x;
-  for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < count; i += stride)
-    out[i] = from_float<DT>(in[i]);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -455,13 +447,6 @@ __global__ void gather_vals_kernel(const ValT* __restrict__ val, const IdxT* __r
     out[q] = val[perm[q]];
 }
 
-int grid_for(long long work_items, int threads, int max_ctas, int sms) {
-  long long g = (work_items + threads - 1) / threads;
-  const long long cap = max_ctas > 0 ? max_ctas : static_cast<long long>(sms) * 4;
-  if (g > cap) g = cap;
-  return g < 1 ? 1 : static_cast<int>(g);
-}
-
 template <typename IdxT, typename DT>
 int rows_impl(bool add, void* dst, int64_t ld_dst, const void* src, int64_t ld_src, const void* list,
               int64_t off, int64_t count, int64_t n, int max_ctas, cudaStream_t stream) {
@@ -488,24 +473,19 @@ int rows_impl(bool add, void* dst, int64_t ld_dst, const void* src, int64_t ld_s
       gather_rows_scalar_kernel<IdxT, DT><<<grid, 256, 0, stream>>>(
           static_cast<DT*>(dst), ld_dst, static_cast<const DT*>(src), ld_src, l, off, count, static_cast<int>(n));
   }
-  count_launch();
-  OFSPMM_CUDA_OK(cudaGetLastError());
-  return OFSPMM_OK;
+  return launched();
 }
 
 int rows_dispatch(bool add, void* dst, int64_t ld_dst, const void* src, int64_t ld_src, const void* list,
                   int idx_dtype, int64_t off, int64_t count, int64_t n, int dense_dtype, int max_ctas,
                   cudaStream_t stream) {
   if (count == 0 || n == 0) return OFSPMM_OK;
-  const bool f32 = dense_dtype == OFSPMM_DTYPE_FLOAT;
-  if (!f32 && dense_dtype != OFSPMM_DTYPE_BFLOAT16) return OFSPMM_ERR_UNSUPPORTED_DTYPE;
-  if (idx_dtype == OFSPMM_DTYPE_INT32)
-    return f32 ? rows_impl<int32_t, float>(add, dst, ld_dst, src, ld_src, list, off, count, n, max_ctas, stream)
-               : rows_impl<int32_t, __nv_bfloat16>(add, dst, ld_dst, src, ld_src, list, off, count, n, max_ctas, stream);
-  if (idx_dtype == OFSPMM_DTYPE_INT64)
-    return f32 ? rows_impl<int64_t, float>(add, dst, ld_dst, src, ld_src, list, off, count, n, max_ctas, stream)
-               : rows_impl<int64_t, __nv_bfloat16>(add, dst, ld_dst, src, ld_src, list, off, count, n, max_ctas, stream);
-  return OFSPMM_ERR_UNSUPPORTED_DTYPE;
+  return dispatch_dense(dense_dtype, [&](auto dense) {
+    return dispatch_idx(idx_dtype, [&](auto idx) {
+      return rows_impl<typename decltype(idx)::type, typename decltype(dense)::type>(add, dst, ld_dst, src, ld_src, list,
+                                                                                    off, count, n, max_ctas, stream);
+    });
+  });
 }
 
 }  // namespace
@@ -533,20 +513,21 @@ int launch_scatter_add_rows_f32(float* dst, int64_t ld_dst, const void* src, int
   if (int rc = get_dev_info(&dev)) return rc;
   const bool vec = n % 8 == 0 && ld_dst % 8 == 0 && ld_src % 8 == 0 &&
                    ((reinterpret_cast<uintptr_t>(dst) & 31) == 0) && ((reinterpret_cast<uintptr_t>(src) & 15) == 0);
-  const bool i32 = idx_dtype == OFSPMM_DTYPE_INT32;
-  if (vec) {
-    const int units = static_cast<int>(n / 8);
-    const int grid = grid_for(count * units, kThreads, max_ctas, dev.sms);
-    if (i32) scatter_add_rows_bf16_to_f32_kernel<int32_t><<<grid, kThreads, 0, stream>>>(dst, ld_dst, static_cast<const char*>(src), ld_src * 2, static_cast<const int32_t*>(list), idx_offset, count, units);
-    else scatter_add_rows_bf16_to_f32_kernel<int64_t><<<grid, kThreads, 0, stream>>>(dst, ld_dst, static_cast<const char*>(src), ld_src * 2, static_cast<const int64_t*>(list), idx_offset, count, units);
-  } else {
-    const int grid = grid_for(count * n, 256, max_ctas, dev.sms);
-    if (i32) scatter_add_rows_bf16_to_f32_scalar_kernel<int32_t><<<grid, 256, 0, stream>>>(dst, ld_dst, static_cast<const __nv_bfloat16*>(src), ld_src, static_cast<const int32_t*>(list), idx_offset, count, static_cast<int>(n));
-    else scatter_add_rows_bf16_to_f32_scalar_kernel<int64_t><<<grid, 256, 0, stream>>>(dst, ld_dst, static_cast<const __nv_bfloat16*>(src), ld_src, static_cast<const int64_t*>(list), idx_offset, count, static_cast<int>(n));
-  }
-  count_launch();
-  OFSPMM_CUDA_OK(cudaGetLastError());
-  return OFSPMM_OK;
+  return dispatch_idx(idx_dtype, [&](auto idx) {
+    using IdxT = typename decltype(idx)::type;
+    const IdxT* l = static_cast<const IdxT*>(list);
+    if (vec) {
+      const int units = static_cast<int>(n / 8);
+      const int grid = grid_for(count * units, kThreads, max_ctas, dev.sms);
+      scatter_add_rows_bf16_to_f32_kernel<IdxT><<<grid, kThreads, 0, stream>>>(
+          dst, ld_dst, static_cast<const char*>(src), ld_src * 2, l, idx_offset, count, units);
+    } else {
+      const int grid = grid_for(count * n, 256, max_ctas, dev.sms);
+      scatter_add_rows_bf16_to_f32_scalar_kernel<IdxT><<<grid, 256, 0, stream>>>(
+          dst, ld_dst, static_cast<const __nv_bfloat16*>(src), ld_src, l, idx_offset, count, static_cast<int>(n));
+    }
+    return launched();
+  });
 }
 
 int launch_cast_from_f32(const float* src, void* dst, int64_t count, int dst_dtype, cudaStream_t stream) {
@@ -554,16 +535,11 @@ int launch_cast_from_f32(const float* src, void* dst, int64_t count, int dst_dty
   DevInfo dev;
   if (int rc = get_dev_info(&dev)) return rc;
   const int grid = grid_for(count, 256, dev.sms * 8, dev.sms);
-  if (dst_dtype == OFSPMM_DTYPE_BFLOAT16) {
-    cast_rows_from_f32_kernel<__nv_bfloat16><<<grid, 256, 0, stream>>>(src, static_cast<__nv_bfloat16*>(dst), count);
-  } else if (dst_dtype == OFSPMM_DTYPE_FLOAT) {
-    cast_rows_from_f32_kernel<float><<<grid, 256, 0, stream>>>(src, static_cast<float*>(dst), count);
-  } else {
-    return OFSPMM_ERR_UNSUPPORTED_DTYPE;
-  }
-  count_launch();
-  OFSPMM_CUDA_OK(cudaGetLastError());
-  return OFSPMM_OK;
+  return dispatch_dense(dst_dtype, [&](auto dt) {
+    using DT = typename decltype(dt)::type;
+    cast_from_f32_kernel<DT><<<grid, 256, 0, stream>>>(src, static_cast<DT*>(dst), count);
+    return launched();
+  });
 }
 
 int launch_signal_peers(void* const* slots, int n, unsigned long long epoch, cudaStream_t stream) {
@@ -573,9 +549,7 @@ int launch_signal_peers(void* const* slots, int n, unsigned long long epoch, cud
   a.n = n;
   for (int i = 0; i < n; ++i) a.slot[i] = static_cast<unsigned long long*>(slots[i]);
   signal_peers_kernel<<<1, 32, 0, stream>>>(a, epoch);
-  count_launch();
-  OFSPMM_CUDA_OK(cudaGetLastError());
-  return OFSPMM_OK;
+  return launched();
 }
 
 int launch_pull_rows_multi(void* dst, int64_t ld_dst, int64_t ld_src, const ofspmm_pull_seg* segs, int nseg,
@@ -605,78 +579,64 @@ int launch_pull_rows_multi(void* dst, int64_t ld_dst, int64_t ld_src, const ofsp
   if (int rc = get_dev_info(&dev)) return rc;
   const int units = static_cast<int>(n * es / 16);
   const size_t row_bytes = static_cast<size_t>(n) * es;
-  if (idx_dtype != OFSPMM_DTYPE_INT32 && idx_dtype != OFSPMM_DTYPE_INT64) return OFSPMM_ERR_UNSUPPORTED_DTYPE;
-  if (ld_dst == n && row_bytes <= static_cast<size_t>(kStageBytes)) {
-    // TMA path: destination rows packed (one bulk store per stage), a row fits a stage
-    const int rows_per_stage = static_cast<int>(kStageBytes / row_bytes);
-    const size_t smem = static_cast<size_t>(kStages) * kStageBytes + kStages * sizeof(uint64_t);
-    int grid = max_ctas > 0 ? max_ctas : dev.sms * 2;
-    const long long need = (rows + rows_per_stage - 1) / rows_per_stage;
-    if (grid > need) grid = static_cast<int>(need < 1 ? 1 : need);
-    if (idx_dtype == OFSPMM_DTYPE_INT32) {
-      static KernelLaunchCache cache;
+  return dispatch_idx(idx_dtype, [&](auto idx) -> int {
+    using IdxT = typename decltype(idx)::type;
+    if (ld_dst == n && row_bytes <= static_cast<size_t>(kStageBytes)) {
+      // TMA path: destination rows packed (one bulk store per stage), a row fits a stage
+      const int rows_per_stage = static_cast<int>(kStageBytes / row_bytes);
+      const size_t smem = static_cast<size_t>(kStages) * kStageBytes + kStages * sizeof(uint64_t);
+      int grid = max_ctas > 0 ? max_ctas : dev.sms * 2;
+      const long long need = (rows + rows_per_stage - 1) / rows_per_stage;
+      if (grid > need) grid = static_cast<int>(need < 1 ? 1 : need);
+      static KernelLaunchCache cache;  // one per index type
       if (cache.get(dev.ordinal) == 0) {
-        OFSPMM_CUDA_OK(cudaFuncSetAttribute(pull_rows_tma_kernel<int32_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+        OFSPMM_CUDA_OK(cudaFuncSetAttribute(pull_rows_tma_kernel<IdxT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                            static_cast<int>(smem)));
         cache.set(dev.ordinal, 1);
       }
-      pull_rows_tma_kernel<int32_t><<<grid, 32, smem, stream>>>(static_cast<char*>(dst), ld_dst * es, ld_src * es, a, epoch,
-                                                               static_cast<uint32_t>(row_bytes));
+      pull_rows_tma_kernel<IdxT><<<grid, 32, smem, stream>>>(static_cast<char*>(dst), ld_dst * es, ld_src * es, a, epoch,
+                                                            static_cast<uint32_t>(row_bytes));
     } else {
-      static KernelLaunchCache cache;
-      if (cache.get(dev.ordinal) == 0) {
-        OFSPMM_CUDA_OK(cudaFuncSetAttribute(pull_rows_tma_kernel<int64_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-        cache.set(dev.ordinal, 1);
-      }
-      pull_rows_tma_kernel<int64_t><<<grid, 32, smem, stream>>>(static_cast<char*>(dst), ld_dst * es, ld_src * es, a, epoch,
-                                                               static_cast<uint32_t>(row_bytes));
+      int grid = max_ctas > 0 ? max_ctas : dev.sms * 2;
+      const long long need = (rows * units + kPullThreads * kUnroll - 1) / (kPullThreads * kUnroll);
+      if (grid > need) grid = static_cast<int>(need < 1 ? 1 : need);
+      pull_rows_multi_kernel<IdxT><<<grid, kPullThreads, 0, stream>>>(static_cast<char*>(dst), ld_dst * es, ld_src * es, a,
+                                                                     epoch, units);
     }
-  } else {
-    int grid = max_ctas > 0 ? max_ctas : dev.sms * 2;
-    const long long need = (rows * units + kPullThreads * kUnroll - 1) / (kPullThreads * kUnroll);
-    if (grid > need) grid = static_cast<int>(need < 1 ? 1 : need);
-    if (idx_dtype == OFSPMM_DTYPE_INT32)
-      pull_rows_multi_kernel<int32_t><<<grid, kPullThreads, 0, stream>>>(static_cast<char*>(dst), ld_dst * es, ld_src * es, a, epoch, units);
-    else
-      pull_rows_multi_kernel<int64_t><<<grid, kPullThreads, 0, stream>>>(static_cast<char*>(dst), ld_dst * es, ld_src * es, a, epoch, units);
-  }
-  count_launch();
-  OFSPMM_CUDA_OK(cudaGetLastError());
-  return OFSPMM_OK;
+    return launched();
+  });
 }
 
 int launch_combine_rows_multi(float* acc, int64_t ld_acc, int64_t ld_src, const ofspmm_combine_seg* segs, int nseg,
                               unsigned long long epoch, int64_t rows, int64_t n, int src_dtype, int max_ctas,
                               cudaStream_t stream) {
   if (nseg < 0 || nseg > kMaxSegs) return OFSPMM_ERR_INVALID_ARG;
-  if (src_dtype != OFSPMM_DTYPE_FLOAT && src_dtype != OFSPMM_DTYPE_BFLOAT16) return OFSPMM_ERR_UNSUPPORTED_DTYPE;
-  const size_t es = src_dtype == OFSPMM_DTYPE_FLOAT ? 4 : 2;
-  // one 16-byte source unit = 4 fp32 (16 B of fp32 accumulator) or 8 bf16 (32 B of accumulator)
-  const size_t acc_unit = src_dtype == OFSPMM_DTYPE_FLOAT ? 16 : 32;
-  if ((n * es) % 16 != 0 || (ld_src * es) % 16 != 0 || (ld_acc * 4) % acc_unit != 0 ||
-      (reinterpret_cast<uintptr_t>(acc) & (acc_unit - 1)))
-    return OFSPMM_ERR_INVALID_ARG;
-  if (nseg == 0 || rows == 0 || n == 0) return OFSPMM_OK;
-  CombineArgs a;
-  a.nseg = nseg;
-  for (int i = 0; i < nseg; ++i) {
-    if (segs[i].src == nullptr || segs[i].inv == nullptr || segs[i].flag == nullptr) return OFSPMM_ERR_INVALID_ARG;
-    a.seg[i].src = static_cast<const char*>(segs[i].src);
-    a.seg[i].inv = static_cast<const int*>(segs[i].inv);
-    a.seg[i].flag = static_cast<const unsigned long long*>(segs[i].flag);
-  }
-  DevInfo dev;
-  if (int rc = get_dev_info(&dev)) return rc;
-  const int units = static_cast<int>(n * es / 16);
-  int grid = max_ctas > 0 ? max_ctas : dev.sms * 8;
-  const long long need = (rows * units + kPullThreads * kUnroll - 1) / (kPullThreads * kUnroll);
-  if (grid > need) grid = static_cast<int>(need < 1 ? 1 : need);
-  if (src_dtype == OFSPMM_DTYPE_FLOAT)
-    combine_rows_multi_kernel<float><<<grid, kPullThreads, 0, stream>>>(acc, ld_acc, ld_src * es, a, epoch, rows, units);
-  else
-    combine_rows_multi_kernel<__nv_bfloat16><<<grid, kPullThreads, 0, stream>>>(acc, ld_acc, ld_src * es, a, epoch, rows, units);
-  count_launch();
-  OFSPMM_CUDA_OK(cudaGetLastError());
-  return OFSPMM_OK;
+  return dispatch_dense(src_dtype, [&](auto st) -> int {
+    using SrcT = typename decltype(st)::type;
+    constexpr size_t es = sizeof(SrcT);
+    // one 16-byte source unit = 4 fp32 (16 B of fp32 accumulator) or 8 bf16 (32 B of accumulator)
+    constexpr size_t acc_unit = 16 / es * sizeof(float);
+    if ((n * es) % 16 != 0 || (ld_src * es) % 16 != 0 || (ld_acc * 4) % acc_unit != 0 ||
+        (reinterpret_cast<uintptr_t>(acc) & (acc_unit - 1)))
+      return OFSPMM_ERR_INVALID_ARG;
+    if (nseg == 0 || rows == 0 || n == 0) return OFSPMM_OK;
+    CombineArgs a;
+    a.nseg = nseg;
+    for (int i = 0; i < nseg; ++i) {
+      if (segs[i].src == nullptr || segs[i].inv == nullptr || segs[i].flag == nullptr) return OFSPMM_ERR_INVALID_ARG;
+      a.seg[i].src = static_cast<const char*>(segs[i].src);
+      a.seg[i].inv = static_cast<const int*>(segs[i].inv);
+      a.seg[i].flag = static_cast<const unsigned long long*>(segs[i].flag);
+    }
+    DevInfo dev;
+    if (int rc = get_dev_info(&dev)) return rc;
+    const int units = static_cast<int>(n * es / 16);
+    int grid = max_ctas > 0 ? max_ctas : dev.sms * 8;
+    const long long need = (rows * units + kPullThreads * kUnroll - 1) / (kPullThreads * kUnroll);
+    if (grid > need) grid = static_cast<int>(need < 1 ? 1 : need);
+    combine_rows_multi_kernel<SrcT><<<grid, kPullThreads, 0, stream>>>(acc, ld_acc, ld_src * es, a, epoch, rows, units);
+    return launched();
+  });
 }
 
 int launch_gather_vals(const void* val, int val_dtype, const void* perm, int idx_dtype, int64_t nnz,
@@ -685,19 +645,15 @@ int launch_gather_vals(const void* val, int val_dtype, const void* perm, int idx
   DevInfo dev;
   if (int rc = get_dev_info(&dev)) return rc;
   const int grid = grid_for(nnz, 256, dev.sms * 8, dev.sms);
-  const bool i32 = idx_dtype == OFSPMM_DTYPE_INT32;
-  if (val_dtype == OFSPMM_DTYPE_FLOAT) {
-    if (i32) gather_vals_kernel<int32_t, float><<<grid, 256, 0, stream>>>(static_cast<const float*>(val), static_cast<const int32_t*>(perm), nnz, static_cast<float*>(out));
-    else gather_vals_kernel<int64_t, float><<<grid, 256, 0, stream>>>(static_cast<const float*>(val), static_cast<const int64_t*>(perm), nnz, static_cast<float*>(out));
-  } else if (val_dtype == OFSPMM_DTYPE_BFLOAT16) {
-    if (i32) gather_vals_kernel<int32_t, __nv_bfloat16><<<grid, 256, 0, stream>>>(static_cast<const __nv_bfloat16*>(val), static_cast<const int32_t*>(perm), nnz, static_cast<__nv_bfloat16*>(out));
-    else gather_vals_kernel<int64_t, __nv_bfloat16><<<grid, 256, 0, stream>>>(static_cast<const __nv_bfloat16*>(val), static_cast<const int64_t*>(perm), nnz, static_cast<__nv_bfloat16*>(out));
-  } else {
-    return OFSPMM_ERR_UNSUPPORTED_DTYPE;
-  }
-  count_launch();
-  OFSPMM_CUDA_OK(cudaGetLastError());
-  return OFSPMM_OK;
+  return dispatch_dense(val_dtype, [&](auto vt) {
+    return dispatch_idx(idx_dtype, [&](auto idx) {
+      using ValT = typename decltype(vt)::type;
+      using IdxT = typename decltype(idx)::type;
+      gather_vals_kernel<IdxT, ValT><<<grid, 256, 0, stream>>>(static_cast<const ValT*>(val), static_cast<const IdxT*>(perm),
+                                                              nnz, static_cast<ValT*>(out));
+      return launched();
+    });
+  });
 }
 
 }  // namespace ofspmm

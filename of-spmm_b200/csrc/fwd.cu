@@ -1,6 +1,6 @@
 // fwd.cu — variant resolution and dispatch of the merge-path SpMM forward to its kernel family
 // (fwd_launch.cuh), plus the task partitioner launch.
-#include "internal.h"
+#include "launch.cuh"
 #include "spmm_kernels.cuh"
 
 namespace ofspmm {
@@ -63,22 +63,14 @@ int launch_task_partition(const void* crow, int idx_dtype, int64_t rows, int64_t
                           int items, void* part, cudaStream_t stream) {
   const int threads = 256;
   const unsigned blocks = static_cast<unsigned>((P + 1 + threads - 1) / threads);
-  if (idx_dtype == OFSPMM_DTYPE_INT32) {
-    task_partition_kernel<int32_t, int2><<<blocks, threads, 0, stream>>>(
-        static_cast<const int32_t*>(crow), static_cast<int>(rows), static_cast<int>(nnz), items,
-        static_cast<int>(P), static_cast<int2*>(part));
-  } else if (!wide_nnz(nnz)) {
-    task_partition_kernel<int64_t, int2><<<blocks, threads, 0, stream>>>(
-        static_cast<const int64_t*>(crow), static_cast<int>(rows), static_cast<int>(nnz), items,
-        static_cast<int>(P), static_cast<int2*>(part));
-  } else {
-    task_partition_kernel<int64_t, longlong2><<<blocks, threads, 0, stream>>>(
-        static_cast<const int64_t*>(crow), static_cast<int>(rows), static_cast<long long>(nnz), items,
-        static_cast<int>(P), static_cast<longlong2*>(part));
-  }
-  count_launch();
-  OFSPMM_CUDA_OK(cudaGetLastError());
-  return OFSPMM_OK;
+  return dispatch_index<true>(idx_dtype, wide_nnz(nnz), [&](auto idx, auto pt) {
+    using IdxT = typename decltype(idx)::type;
+    using PartT = typename decltype(pt)::type;
+    task_partition_kernel<IdxT, PartT><<<blocks, threads, 0, stream>>>(
+        static_cast<const IdxT*>(crow), static_cast<int>(rows), static_cast<typename PartOf<PartT>::Nz>(nnz), items,
+        static_cast<int>(P), static_cast<PartT*>(part));
+    return launched();
+  });
 }
 
 // The whole-row kernel needs what resolve_variant cannot see: the pointers' alignment, the

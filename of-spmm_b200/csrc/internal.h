@@ -124,6 +124,17 @@ struct FwdLaunch {
 };
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
+// Lays out a workspace region after region, each starting 256-byte aligned: take() returns the
+// offset of the next region, `total` is the size so far.
+struct Carve {
+  size_t total = 0;
+  size_t take(size_t bytes) {
+    const size_t at = total;
+    total += align_up(bytes, 256);
+    return at;
+  }
+};
+
 struct DevInfo {
   int sms;
   int cc_major;

@@ -1,6 +1,6 @@
-// launch.cuh — host-side dispatch shared by the launchers of the merge-path kernels (fwd_launch.cuh,
-// fwd_rows.cu, sddmm.cu, bwd.cu): runtime dtype codes and lane layouts to template arguments, and
-// the launch constants of a kernel on the current device.
+// launch.cuh — host-side dispatch shared by every launcher: runtime dtype codes and lane layouts to
+// template arguments, and the launch constants of a kernel on the current device.  Each dispatch
+// returns OFSPMM_ERR_UNSUPPORTED_DTYPE for a code it has no type for.
 #pragma once
 #include "common.cuh"
 #include "internal.h"
@@ -9,6 +9,22 @@ namespace ofspmm {
 
 template <typename T>
 struct Tag { using type = T; };
+
+// f(Tag<IdxT>{}) for an index dtype.
+template <typename F>
+int dispatch_idx(int idx_dtype, F&& f) {
+  if (idx_dtype == OFSPMM_DTYPE_INT32) return f(Tag<int32_t>{});
+  if (idx_dtype == OFSPMM_DTYPE_INT64) return f(Tag<int64_t>{});
+  return OFSPMM_ERR_UNSUPPORTED_DTYPE;
+}
+
+// f(Tag<DT>{}) for a dense (or stored-value) dtype.
+template <typename F>
+int dispatch_dense(int dtype, F&& f) {
+  if (dtype == OFSPMM_DTYPE_FLOAT) return f(Tag<float>{});
+  if (dtype == OFSPMM_DTYPE_BFLOAT16) return f(Tag<__nv_bfloat16>{});
+  return OFSPMM_ERR_UNSUPPORTED_DTYPE;
+}
 
 // f(Tag<DT>{}, Tag<ValT>{}) for a (dense, value) dtype pair; kUnit: the caller has kernels for
 // pattern matrices (UnitVal) too.
@@ -48,6 +64,20 @@ int dispatch_lanes(const LaneLayout& l, F&& f) {
   int rc = OFSPMM_ERR_INVALID_ARG;
   (void)((l.vec == Ls::VEC && l.lpr == Ls::LPR && l.ch == Ls::CH && ((rc = f(Ls{})), true)) || ...);
   return rc;
+}
+
+// Status after `k` kernel launches: counts them and reports a launch error.
+inline int launched(uint64_t k = 1) {
+  count_launch(k);
+  return cudaGetLastError() == cudaSuccess ? OFSPMM_OK : OFSPMM_ERR_CUDA;
+}
+
+// CTAs for `work_items` at `threads` per CTA, at most `max_ctas` (0: 4 per SM), at least 1.
+inline int grid_for(long long work_items, int threads, int max_ctas, int sms) {
+  long long g = (work_items + threads - 1) / threads;
+  const long long cap = max_ctas > 0 ? max_ctas : static_cast<long long>(sms) * 4;
+  if (g > cap) g = cap;
+  return g < 1 ? 1 : static_cast<int>(g);
 }
 
 // Dynamic shared memory of a merge-path kernel: one task stage and one mbarrier per warp.

@@ -2,8 +2,7 @@
 // CSR -> CSR(A^T) transpose (plan / OpKernelState construction; not on the per-step path).
 #include <cub/device/device_radix_sort.cuh>
 
-#include "common.cuh"
-#include "internal.h"
+#include "launch.cuh"
 
 namespace ofspmm {
 
@@ -131,14 +130,23 @@ template <typename IdxT, typename KeyT>
 TransposeLayout transpose_layout(int64_t cols, int64_t nnz) {
   TransposeLayout L;
   const size_t n = static_cast<size_t>(nnz > 0 ? nnz : 1);
-  const size_t karr = align_up(n * sizeof(KeyT), 256);
-  L.keys_a = 0;
-  L.keys_b = karr;
-  L.pos = 2 * karr;
-  L.cub_tmp = L.pos + align_up(n * sizeof(IdxT), 256);
+  Carve c;
+  L.keys_a = c.take(n * sizeof(KeyT));
+  L.keys_b = c.take(n * sizeof(KeyT));
+  L.pos = c.take(n * sizeof(IdxT));
   L.cub_bytes = cub_sort_temp_bytes<KeyT, IdxT>(nnz, bits_for(cols + 1));
-  L.total = L.cub_tmp + align_up(L.cub_bytes, 256);
+  L.cub_tmp = c.take(L.cub_bytes);
+  L.total = c.total;
   return L;
+}
+
+// f(Tag<IdxT>{}, Tag<KeyT>{}) of A's transpose.
+template <typename F>
+int dispatch_transpose(int idx_dtype, int64_t cols, F&& f) {
+  return dispatch_idx(idx_dtype, [&](auto idx) {
+    if constexpr (std::is_same_v<typename decltype(idx)::type, int32_t>) return f(idx, Tag<int32_t>{});
+    else return narrow_keys(cols) ? f(idx, Tag<int32_t>{}) : f(idx, Tag<int64_t>{});
+  });
 }
 
 template <typename IdxT, typename KeyT>
@@ -176,26 +184,17 @@ int transpose_impl(const ofspmm_csr* A, void* t_crow, void* t_col, void* t_val, 
   IdxT* pos_out = perm;
   transpose_offsets_kernel<IdxT, KeyT><<<static_cast<unsigned>((cols + 1 + 255) / 256), 256, 0, stream>>>(
       keys_out, nnz, cols, static_cast<IdxT*>(t_crow));
+  if (nnz == 0) return launched();
   count_launch();
-  if (nnz > 0) {
-    if (A->val == nullptr || t_val == nullptr) {
-      transpose_fill_kernel<IdxT, KeyT, float><<<grid, 256, 0, stream>>>(
-          static_cast<const IdxT*>(A->crow), rows, nullptr, pos_out, keys_out, cols, nnz, static_cast<IdxT*>(t_col), nullptr);
-    } else if (A->val_dtype == OFSPMM_DTYPE_FLOAT) {
-      transpose_fill_kernel<IdxT, KeyT, float><<<grid, 256, 0, stream>>>(
-          static_cast<const IdxT*>(A->crow), rows, static_cast<const float*>(A->val), pos_out, keys_out, cols, nnz,
-          static_cast<IdxT*>(t_col), static_cast<float*>(t_val));
-    } else if (A->val_dtype == OFSPMM_DTYPE_BFLOAT16) {
-      transpose_fill_kernel<IdxT, KeyT, __nv_bfloat16><<<grid, 256, 0, stream>>>(
-          static_cast<const IdxT*>(A->crow), rows, static_cast<const __nv_bfloat16*>(A->val), pos_out, keys_out, cols, nnz,
-          static_cast<IdxT*>(t_col), static_cast<__nv_bfloat16*>(t_val));
-    } else {
-      return OFSPMM_ERR_UNSUPPORTED_DTYPE;
-    }
-    count_launch();
-  }
-  OFSPMM_CUDA_OK(cudaGetLastError());
-  return OFSPMM_OK;
+  auto fill = [&](auto v, const void* val, void* out) {
+    using ValT = typename decltype(v)::type;
+    transpose_fill_kernel<IdxT, KeyT, ValT><<<grid, 256, 0, stream>>>(
+        static_cast<const IdxT*>(A->crow), rows, static_cast<const ValT*>(val), pos_out, keys_out, cols, nnz,
+        static_cast<IdxT*>(t_col), static_cast<ValT*>(out));
+    return launched();
+  };
+  if (A->val == nullptr || t_val == nullptr) return fill(Tag<float>{}, nullptr, nullptr);
+  return dispatch_dense(A->val_dtype, [&](auto v) { return fill(v, A->val, t_val); });
 }
 
 }  // namespace
@@ -203,20 +202,13 @@ int transpose_impl(const ofspmm_csr* A, void* t_crow, void* t_col, void* t_val, 
 int launch_partition_public(const void* crow, int idx_dtype, int64_t rows, int64_t nnz, int64_t parts,
                             int64_t* out_row, int64_t* out_nz, cudaStream_t stream) {
   const unsigned blocks = static_cast<unsigned>((parts + 1 + 255) / 256);
-  if (idx_dtype == OFSPMM_DTYPE_INT32) {
-    partition_public_kernel<int32_t><<<blocks, 256, 0, stream>>>(
-        static_cast<const int32_t*>(crow), rows, nnz, parts, reinterpret_cast<long long*>(out_row),
-        reinterpret_cast<long long*>(out_nz));
-  } else if (idx_dtype == OFSPMM_DTYPE_INT64) {
-    partition_public_kernel<int64_t><<<blocks, 256, 0, stream>>>(
-        static_cast<const int64_t*>(crow), rows, nnz, parts, reinterpret_cast<long long*>(out_row),
-        reinterpret_cast<long long*>(out_nz));
-  } else {
-    return OFSPMM_ERR_UNSUPPORTED_DTYPE;
-  }
-  count_launch();
-  OFSPMM_CUDA_OK(cudaGetLastError());
-  return OFSPMM_OK;
+  return dispatch_idx(idx_dtype, [&](auto idx) {
+    using IdxT = typename decltype(idx)::type;
+    partition_public_kernel<IdxT><<<blocks, 256, 0, stream>>>(static_cast<const IdxT*>(crow), rows, nnz, parts,
+                                                             reinterpret_cast<long long*>(out_row),
+                                                             reinterpret_cast<long long*>(out_nz));
+    return launched();
+  });
 }
 
 int launch_row_hist(const void* crow, int idx_dtype, int64_t rows, int64_t* hist32, cudaStream_t stream) {
@@ -224,36 +216,31 @@ int launch_row_hist(const void* crow, int idx_dtype, int64_t rows, int64_t* hist
   if (rows == 0) return OFSPMM_OK;
   DevInfo dev;
   if (int rc = get_dev_info(&dev)) return rc;
-  int64_t blocks = (rows + 255) / 256;
-  if (blocks > dev.sms * 8) blocks = dev.sms * 8;
-  if (idx_dtype == OFSPMM_DTYPE_INT32) {
-    row_hist_kernel<int32_t><<<static_cast<unsigned>(blocks), 256, 0, stream>>>(
-        static_cast<const int32_t*>(crow), rows, reinterpret_cast<unsigned long long*>(hist32));
-  } else if (idx_dtype == OFSPMM_DTYPE_INT64) {
-    row_hist_kernel<int64_t><<<static_cast<unsigned>(blocks), 256, 0, stream>>>(
-        static_cast<const int64_t*>(crow), rows, reinterpret_cast<unsigned long long*>(hist32));
-  } else {
-    return OFSPMM_ERR_UNSUPPORTED_DTYPE;
-  }
-  count_launch();
-  OFSPMM_CUDA_OK(cudaGetLastError());
-  return OFSPMM_OK;
+  const int blocks = grid_for(rows, 256, dev.sms * 8, dev.sms);
+  return dispatch_idx(idx_dtype, [&](auto idx) {
+    using IdxT = typename decltype(idx)::type;
+    row_hist_kernel<IdxT><<<blocks, 256, 0, stream>>>(static_cast<const IdxT*>(crow), rows,
+                                                     reinterpret_cast<unsigned long long*>(hist32));
+    return launched();
+  });
 }
 
 size_t transpose_workspace_bytes(int64_t rows, int64_t cols, int64_t nnz, int idx_dtype) {
   (void)rows;
-  if (idx_dtype == OFSPMM_DTYPE_INT32) return transpose_layout<int32_t, int32_t>(cols, nnz).total;
-  if (narrow_keys(cols)) return transpose_layout<int64_t, int32_t>(cols, nnz).total;
-  return transpose_layout<int64_t, int64_t>(cols, nnz).total;
+  size_t bytes = 0;
+  dispatch_transpose(idx_dtype, cols, [&](auto idx, auto key) {
+    bytes = transpose_layout<typename decltype(idx)::type, typename decltype(key)::type>(cols, nnz).total;
+    return OFSPMM_OK;
+  });
+  return bytes;
 }
 
 int launch_transpose(const ofspmm_csr* A, void* t_crow, void* t_col, void* t_val, void* t_perm,
                      void* ws, size_t ws_bytes, cudaStream_t stream) {
-  if (A->idx_dtype == OFSPMM_DTYPE_INT32) return transpose_impl<int32_t, int32_t>(A, t_crow, t_col, t_val, t_perm, ws, ws_bytes, stream);
-  if (A->idx_dtype == OFSPMM_DTYPE_INT64 && narrow_keys(A->cols))
-    return transpose_impl<int64_t, int32_t>(A, t_crow, t_col, t_val, t_perm, ws, ws_bytes, stream);
-  if (A->idx_dtype == OFSPMM_DTYPE_INT64) return transpose_impl<int64_t, int64_t>(A, t_crow, t_col, t_val, t_perm, ws, ws_bytes, stream);
-  return OFSPMM_ERR_UNSUPPORTED_DTYPE;
+  return dispatch_transpose(A->idx_dtype, A->cols, [&](auto idx, auto key) {
+    return transpose_impl<typename decltype(idx)::type, typename decltype(key)::type>(A, t_crow, t_col, t_val, t_perm,
+                                                                                    ws, ws_bytes, stream);
+  });
 }
 
 }  // namespace ofspmm

@@ -15,8 +15,7 @@
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 
-#include "common.cuh"
-#include "internal.h"
+#include "launch.cuh"
 
 namespace ofspmm {
 
@@ -328,21 +327,20 @@ struct SampleLayout {
 SampleLayout sample_layout(int64_t num_dst, int64_t cap) {
   SampleLayout L;
   const size_t nd = static_cast<size_t>(num_dst > 0 ? num_dst : 1), nc = static_cast<size_t>(cap > 0 ? cap : 1);
-  size_t off = 0;
-  auto take = [&](size_t bytes) { const size_t at = off; off += align_up(bytes, 256); return at; };
-  L.hdr = take(256);
-  L.dkey_in = take(nd * 4);
-  L.dkey_out = take(nd * 4);
-  L.didx_in = take(nd * 4);
-  L.didx_out = take(nd * 4);
-  L.kcnt = take((nd + 1) * 8);
-  L.slot = take((nd + 1) * 8);
-  L.longs = take(nd * 4);
-  L.stage_col = take(nc * 4);
-  L.ids = take(nc * 4);
-  L.stage_val = take(nc * 4);
-  L.flag = take((nc + 1) * 8);
-  L.scan = take((nc + 1) * 8);
+  Carve c;
+  L.hdr = c.take(256);
+  L.dkey_in = c.take(nd * 4);
+  L.dkey_out = c.take(nd * 4);
+  L.didx_in = c.take(nd * 4);
+  L.didx_out = c.take(nd * 4);
+  L.kcnt = c.take((nd + 1) * 8);
+  L.slot = c.take((nd + 1) * 8);
+  L.longs = c.take(nd * 4);
+  L.stage_col = c.take(nc * 4);
+  L.ids = c.take(nc * 4);
+  L.stage_val = c.take(nc * 4);
+  L.flag = c.take((nc + 1) * 8);
+  L.scan = c.take((nc + 1) * 8);
   // temporary storage of the widest key range (32 bits) bounds that of every narrower one
   size_t b1 = 0, b2 = 0, b3 = 0, b4 = 0;
   cub::DeviceRadixSort::SortPairs(nullptr, b1, static_cast<const unsigned*>(nullptr), static_cast<unsigned*>(nullptr),
@@ -357,8 +355,8 @@ SampleLayout sample_layout(int64_t num_dst, int64_t cap) {
   if (b2 > L.cub_bytes) L.cub_bytes = b2;
   if (b3 > L.cub_bytes) L.cub_bytes = b3;
   if (b4 > L.cub_bytes) L.cub_bytes = b4;
-  L.cub_tmp = take(L.cub_bytes);
-  L.total = off;
+  L.cub_tmp = c.take(L.cub_bytes);
+  L.total = c.total;
   return L;
 }
 
@@ -391,17 +389,13 @@ int sample_impl(const ofspmm_csr* A, const void* dst_v, int64_t num_dst, int64_t
   const int bits = id_bits(rows);
   DevInfo dev;
   if (int rc = get_dev_info(&dev)) return rc;
-  const int grid = dev.sms * 8;
-  auto blocks = [&](long long n, int threads) {
-    const long long g = (n + threads - 1) / threads;
-    return static_cast<unsigned>(g < 1 ? 1 : (g > grid ? grid : g));
-  };
+  auto blocks = [&](long long n) { return grid_for(n, 256, dev.sms * 8, dev.sms); };
 
   OFSPMM_CUDA_OK(cudaMemsetAsync(counts, 0, 3 * sizeof(int64_t), stream));
   OFSPMM_CUDA_OK(cudaMemsetAsync(nlong, 0, sizeof(unsigned), stream));
   size_t cub_bytes = L.cub_bytes;
   if (num_dst > 0) {
-    sample_dst_keys_kernel<IdxT><<<blocks(num_dst, 256), 256, 0, stream>>>(dst, num_dst, rows, dkey_in, didx_in);
+    sample_dst_keys_kernel<IdxT><<<blocks(num_dst), 256, 0, stream>>>(dst, num_dst, rows, dkey_in, didx_in);
     count_launch();
     OFSPMM_CUDA_OK(cub::DeviceRadixSort::SortPairs(tmp, cub_bytes, static_cast<const unsigned*>(dkey_in), dkey,
                                                    static_cast<const int*>(didx_in), didx, static_cast<int>(num_dst), 0,
@@ -416,7 +410,7 @@ int sample_impl(const ofspmm_csr* A, const void* dst_v, int64_t num_dst, int64_t
                                                static_cast<int>(num_dst + 1), stream));
   count_launch(2);
   if (cap > 0) {
-    sample_fill_kernel<<<blocks(cap, 256), 256, 0, stream>>>(slot, num_dst, cap, sentinel, stage_col);
+    sample_fill_kernel<<<blocks(cap), 256, 0, stream>>>(slot, num_dst, cap, sentinel, stage_col);
     count_launch();
   }
   if (num_dst > 0) {
@@ -435,31 +429,17 @@ int sample_impl(const ofspmm_csr* A, const void* dst_v, int64_t num_dst, int64_t
                                                   static_cast<int>(cap), 0, bits, stream));
     count_launch(4);
   }
-  sample_flags_kernel<<<blocks(cap + 1, 256), 256, 0, stream>>>(stage_col, ids, cap, dkey, num_dst, sentinel, flag);
+  sample_flags_kernel<<<blocks(cap + 1), 256, 0, stream>>>(stage_col, ids, cap, dkey, num_dst, sentinel, flag);
   count_launch();
   cub_bytes = L.cub_bytes;
   OFSPMM_CUDA_OK(cub::DeviceScan::ExclusiveSum(tmp, cub_bytes, static_cast<const long long*>(flag), scan,
                                                static_cast<int>(cap + 1), stream));
   count_launch(2);
-  sample_emit_kernel<IdxT, VT><<<blocks(cap > num_dst + 1 ? cap : num_dst + 1, 256), 256, 0, stream>>>(
+  sample_emit_kernel<IdxT, VT><<<blocks(cap > num_dst + 1 ? cap : num_dst + 1), 256, 0, stream>>>(
       dst, num_dst, slot, cap, stage_col, stage_val, ids, dkey, didx, flag, scan, sentinel,
       static_cast<int*>(blk_crow), static_cast<int*>(blk_col), static_cast<VT*>(blk_val), static_cast<IdxT*>(src_nodes),
       reinterpret_cast<long long*>(counts));
-  count_launch();
-  OFSPMM_CUDA_OK(cudaGetLastError());
-  return OFSPMM_OK;
-}
-
-template <typename IdxT>
-int sample_by_val(const ofspmm_csr* A, const void* dst, int64_t num_dst, int64_t fanout, uint64_t seed, int64_t cap,
-                  void* blk_crow, void* blk_col, void* blk_val, void* src_nodes, int64_t* counts, void* ws,
-                  cudaStream_t stream) {
-  // values are copied bit for bit: fp32 as 32-bit, bf16 as 16-bit words
-  if (A->val_dtype == OFSPMM_DTYPE_FLOAT)
-    return sample_impl<IdxT, uint32_t>(A, dst, num_dst, fanout, seed, cap, blk_crow, blk_col, blk_val, src_nodes, counts, ws, stream);
-  if (A->val_dtype == OFSPMM_DTYPE_BFLOAT16)
-    return sample_impl<IdxT, uint16_t>(A, dst, num_dst, fanout, seed, cap, blk_crow, blk_col, blk_val, src_nodes, counts, ws, stream);
-  return sample_impl<IdxT, uint8_t>(A, dst, num_dst, fanout, seed, cap, blk_crow, blk_col, nullptr, src_nodes, counts, ws, stream);
+  return launched();
 }
 
 }  // namespace
@@ -469,9 +449,18 @@ size_t sample_neighbors_workspace_bytes(int64_t num_dst, int64_t cap) { return s
 int launch_sample_neighbors(const ofspmm_csr* A, const void* dst, int64_t num_dst, int64_t fanout, uint64_t seed,
                             int64_t cap, void* blk_crow, void* blk_col, void* blk_val, void* src_nodes, int64_t* counts,
                             void* ws, cudaStream_t stream) {
-  if (A->idx_dtype == OFSPMM_DTYPE_INT32)
-    return sample_by_val<int32_t>(A, dst, num_dst, fanout, seed, cap, blk_crow, blk_col, blk_val, src_nodes, counts, ws, stream);
-  return sample_by_val<int64_t>(A, dst, num_dst, fanout, seed, cap, blk_crow, blk_col, blk_val, src_nodes, counts, ws, stream);
+  return dispatch_idx(A->idx_dtype, [&](auto idx) {
+    using IdxT = typename decltype(idx)::type;
+    // values are copied bit for bit: fp32 as 32-bit, bf16 as 16-bit words; a pattern matrix has none
+    if (A->val_dtype == OFSPMM_VAL_UNIT)
+      return sample_impl<IdxT, uint8_t>(A, dst, num_dst, fanout, seed, cap, blk_crow, blk_col, nullptr, src_nodes, counts,
+                                        ws, stream);
+    return dispatch_dense(A->val_dtype, [&](auto vt) {
+      using VT = std::conditional_t<sizeof(typename decltype(vt)::type) == 4, uint32_t, uint16_t>;
+      return sample_impl<IdxT, VT>(A, dst, num_dst, fanout, seed, cap, blk_crow, blk_col, blk_val, src_nodes, counts, ws,
+                                   stream);
+    });
+  });
 }
 
 }  // namespace ofspmm

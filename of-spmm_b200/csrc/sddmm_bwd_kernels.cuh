@@ -378,13 +378,4 @@ __global__ void __launch_bounds__(WARPS * 32) bwd_atomic_kernel(const BwdAtomicP
   }
 }
 
-// out[i] = DT(acc[i]) — the cast that follows an fp32 accumulation for bf16 outputs
-// (reference idiom: oneflow/user/kernels/unsorted_segment_sum_kernel.cpp:162-186).
-template <typename DT>
-__global__ void cast_from_f32_kernel(const float* __restrict__ in, DT* __restrict__ out, long long count) {
-  const long long stride = static_cast<long long>(gridDim.x) * blockDim.x;
-  for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < count; i += stride)
-    out[i] = from_float<DT>(in[i]);
-}
-
 }  // namespace ofspmm
