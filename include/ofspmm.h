@@ -399,6 +399,58 @@ OFSPMM_API int ofspmm_sample_neighbors(const ofspmm_csr* A, const void* dst, int
                                        void* src_nodes, int64_t* counts, void* workspace, size_t workspace_bytes,
                                        ofspmm_stream_t stream);
 
+/* ---- Neighbour sampling with options: weighted (biased) sampling, sampling with replacement, and
+ * the edge ids of the sampled entries.  Notation as above: v = dst[i], deg = crow[v+1] - crow[v],
+ * x(s, v, j) = mix(mix(s ^ v) + j) is the key of the uniform mode, and position j of row v is entry
+ * crow[v] + j of A.  A NULL `opts` (or flags 0 and prob NULL) is ofspmm_sample_neighbors exactly.
+ *
+ * Weighted, without replacement (prob != NULL): `prob` holds nnz weights of dtype `prob_dtype`
+ * (FLOAT or BFLOAT16; it may be A->val itself).  Entry j is eligible iff its weight w_j, widened
+ * exactly to fp64, satisfies 0 < w_j < +inf: NaN, zero, negative and infinite weights are never
+ * selected.  npos = eligible entries of the row; k = min(fanout, npos), npos for fanout -1.  The key
+ * of an eligible entry is wkey_j = neglog(U_j) / w_j (fp64, correctly rounded division) with
+ *     U_j = ((x(s, v, j) >> 11) + 1) * 2^-53   in (0, 1],
+ * and the k eligible entries with the smallest (bits(wkey_j), j) are selected, bits = the
+ * non-negative double read as uint64 (order-preserving).  This is the exponential race
+ * (Efraimidis-Spirakis): with k = 1, entry j is picked with probability w_j / sum(w).  neglog is
+ * -ln computed only from correctly rounded fp64 add / mul / div / fma and exact bit manipulation, in
+ * one fixed order (csrc/sample_key.h, whose C restatement reproduces every key bit for bit); its
+ * error against -ln U is below 4 ulp over the whole domain and neglog(1) = 0.  Rows hold the
+ * selected entries in ascending j, out-of-range columns are dropped, src_nodes as above.
+ *
+ * Uniform, with replacement (OFSPMM_SAMPLE_REPLACE, prob NULL): for deg > 0, destination v gets
+ * k = fanout independent draws; draw t in [0, k) takes position j_t = mulhi64(x(s, v, t), deg) =
+ * floor(x * deg / 2^64).  deg == 0 or fanout == 0 gives none; fanout == -1 takes every entry once,
+ * bit-identical to the mode without replacement.  The row holds the draws in draw order t,
+ * duplicates kept: a repeated column is a multi-edge, which the SpMM sums and the mean counts.  The
+ * sum of k can exceed nnz, so `cap` is not bounded by nnz in this mode.
+ *
+ * Weighted with replacement is not offered: an inverse-CDF draw needs a per-row prefix sum of the
+ * floating-point weights, whose summation order would have to be fixed and restated by every
+ * reference; REPLACE together with prob returns OFSPMM_ERR_INVALID_ARG.
+ *
+ * Edge ids (OFSPMM_SAMPLE_EDGE_IDS), in every mode: blk_eid[q] (A's index dtype, capacity `cap`) is
+ * the position crow[v] + j in A of kept entry q, so that A.col[blk_eid] == src_nodes[blk_col] and
+ * A.val[blk_eid] equals blk_val bit for bit; a gradient wrt A's edge weights flows back through it.
+ * blk_eid must be non-NULL with the flag (when cap > 0) and NULL without it.
+ *
+ * OFSPMM_ERR_INVALID_ARG also for an unknown flag bit and a prob_dtype other than FLOAT / BFLOAT16.
+ * The workspace depends on (num_dst, cap, flags) only; the workspace query returns 0 for invalid
+ * arguments. */
+typedef struct ofspmm_sample_opts {
+  uint32_t flags;      /* OFSPMM_SAMPLE_* */
+  int32_t prob_dtype;  /* dtype of prob: OFSPMM_DTYPE_FLOAT or OFSPMM_DTYPE_BFLOAT16 */
+  const void* prob;    /* NULL: uniform; else nnz per-entry weights (device) */
+} ofspmm_sample_opts;
+enum { OFSPMM_SAMPLE_REPLACE = 1, OFSPMM_SAMPLE_EDGE_IDS = 2 };
+OFSPMM_API size_t ofspmm_sample_neighbors_ex_workspace_bytes(int64_t num_dst, int64_t cap, int idx_dtype,
+                                                             const ofspmm_sample_opts* opts);
+OFSPMM_API int ofspmm_sample_neighbors_ex(const ofspmm_csr* A, const ofspmm_sample_opts* opts, const void* dst,
+                                          int64_t num_dst, int64_t fanout, uint64_t rng_seed, int64_t cap,
+                                          void* blk_crow, void* blk_col, void* blk_val, void* blk_eid, void* src_nodes,
+                                          int64_t* counts, void* workspace, size_t workspace_bytes,
+                                          ofspmm_stream_t stream);
+
 /* ---- Host-buffer convenience entry (what a CPU-tensor caller / the e2e benchmark uses): copies
  * the CSR arrays and B from HOST memory (pinned recommended) to device staging carved from
  * `workspace`, runs ofspmm_fwd, copies C back to `C_host`, all on `stream`; the caller

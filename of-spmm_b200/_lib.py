@@ -30,12 +30,15 @@ EXPORTS = (
     "ofspmm_cast_from_f32", "ofspmm_coo_to_csr_workspace_bytes", "ofspmm_coo_to_csr", "ofspmm_csr_expand_rows",
     "ofspmm_csr_normalize", "ofspmm_signal_peers", "ofspmm_pull_rows_multi", "ofspmm_combine_rows_multi",
     "ofspmm_sample_neighbors_workspace_bytes", "ofspmm_sample_neighbors",
+    "ofspmm_sample_neighbors_ex_workspace_bytes", "ofspmm_sample_neighbors_ex",
 )
 
 # ofspmm_opts.flags / variant codes (include/ofspmm.h)
 FWD_ACCUMULATE, FWD_BIAS, FWD_RELU, ORDER_DYNAMIC, ORDER_STATIC, FWD_ACC32_IN, FWD_ACC32_OUT = 1, 2, 4, 8, 16, 32, 64
 FWD_MEAN = 128
 VARIANT_AUTO, VARIANT_ITEMS64, VARIANT_ROWPAR, VARIANT_ROWS, VARIANT_EXPLICIT = 0, 1, 2, 4, 0x100
+# ofspmm_sample_opts.flags
+SAMPLE_REPLACE, SAMPLE_EDGE_IDS = 1, 2
 
 
 class OfspmmLibraryError(ImportError):
@@ -72,6 +75,11 @@ class OptsStruct(ctypes.Structure):
     _fields_ = [("flags", ctypes.c_uint32), ("tasks_per_warp", ctypes.c_int32), ("variant", ctypes.c_int32),
                 ("reserve_ctas_per_sm", ctypes.c_int32), ("plan", ctypes.c_void_p), ("plan_bytes", ctypes.c_size_t),
                 ("bias", ctypes.c_void_p), ("acc32", ctypes.c_void_p)]
+
+
+class SampleOptsStruct(ctypes.Structure):
+    """struct ofspmm_sample_opts (include/ofspmm.h)."""
+    _fields_ = [("flags", ctypes.c_uint32), ("prob_dtype", ctypes.c_int32), ("prob", ctypes.c_void_p)]
 
 
 _LIB = None
@@ -176,6 +184,12 @@ def lib() -> ctypes.CDLL:
     L.ofspmm_sample_neighbors_workspace_bytes.restype = sz
     L.ofspmm_sample_neighbors.argtypes = [csr_p, vp, i64, i64, ctypes.c_uint64, i64, vp, vp, vp, vp, vp, vp, sz, vp]
     L.ofspmm_sample_neighbors.restype = i32
+    sopts_p = ctypes.POINTER(SampleOptsStruct)
+    L.ofspmm_sample_neighbors_ex_workspace_bytes.argtypes = [i64, i64, i32, sopts_p]
+    L.ofspmm_sample_neighbors_ex_workspace_bytes.restype = sz
+    L.ofspmm_sample_neighbors_ex.argtypes = [csr_p, sopts_p, vp, i64, i64, ctypes.c_uint64, i64, vp, vp, vp, vp, vp, vp,
+                                             vp, sz, vp]
+    L.ofspmm_sample_neighbors_ex.restype = i32
     _LIB = L
     return L
 

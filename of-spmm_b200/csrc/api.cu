@@ -112,6 +112,16 @@ int begin_bwd(const ofspmm_csr* A, const void* dY, void* dB, int64_t n, int dens
   return OFSPMM_OK;
 }
 
+// Checks of the sampling options (NULL: none): known flags only; weights of a dense dtype, and not
+// with replacement.
+int check_sample_opts(const ofspmm_sample_opts* o) {
+  if (o == nullptr) return OFSPMM_OK;
+  if (o->flags & ~static_cast<uint32_t>(OFSPMM_SAMPLE_REPLACE | OFSPMM_SAMPLE_EDGE_IDS)) return OFSPMM_ERR_INVALID_ARG;
+  if (o->prob != nullptr && ((o->flags & OFSPMM_SAMPLE_REPLACE) || !dense_ok(o->prob_dtype))) return OFSPMM_ERR_INVALID_ARG;
+  return OFSPMM_OK;
+}
+bool sample_edge_ids(const ofspmm_sample_opts* o) { return o != nullptr && (o->flags & OFSPMM_SAMPLE_EDGE_IDS); }
+
 int check_ws(const void* ws, size_t have, size_t need) {
   if (need == 0) return OFSPMM_OK;
   if (ws == nullptr || have < need) return OFSPMM_ERR_WORKSPACE;
@@ -461,13 +471,26 @@ int ofspmm_coo_to_csr(const int64_t* row, const int64_t* col, const float* val, 
 }
 
 size_t ofspmm_sample_neighbors_workspace_bytes(int64_t num_dst, int64_t cap, int idx_dtype) {
-  if (num_dst < 0 || cap < 0 || !idx_ok(idx_dtype)) return 0;
-  return sample_neighbors_workspace_bytes(num_dst, cap);
+  return ofspmm_sample_neighbors_ex_workspace_bytes(num_dst, cap, idx_dtype, nullptr);
+}
+
+size_t ofspmm_sample_neighbors_ex_workspace_bytes(int64_t num_dst, int64_t cap, int idx_dtype,
+                                                  const ofspmm_sample_opts* opts) {
+  if (num_dst < 0 || cap < 0 || !idx_ok(idx_dtype) || check_sample_opts(opts) != OFSPMM_OK) return 0;
+  return sample_neighbors_workspace_bytes(num_dst, cap, sample_edge_ids(opts));
 }
 
 int ofspmm_sample_neighbors(const ofspmm_csr* A, const void* dst, int64_t num_dst, int64_t fanout, uint64_t rng_seed,
                             int64_t cap, void* blk_crow, void* blk_col, void* blk_val, void* src_nodes, int64_t* counts,
                             void* workspace, size_t workspace_bytes, ofspmm_stream_t stream) {
+  return ofspmm_sample_neighbors_ex(A, nullptr, dst, num_dst, fanout, rng_seed, cap, blk_crow, blk_col, blk_val, nullptr,
+                                    src_nodes, counts, workspace, workspace_bytes, stream);
+}
+
+int ofspmm_sample_neighbors_ex(const ofspmm_csr* A, const ofspmm_sample_opts* opts, const void* dst, int64_t num_dst,
+                               int64_t fanout, uint64_t rng_seed, int64_t cap, void* blk_crow, void* blk_col,
+                               void* blk_val, void* blk_eid, void* src_nodes, int64_t* counts, void* workspace,
+                               size_t workspace_bytes, ofspmm_stream_t stream) {
   if (int rc = check_csr(A, true)) return rc;
   if (A->rows != A->cols || fanout < -1 || num_dst < 0 || cap < 0) return OFSPMM_ERR_INVALID_ARG;
   if (cap >= kWideNnz || num_dst >= kWideNnz) return OFSPMM_ERR_TOO_LARGE;   // int32 block offsets and local ids
@@ -476,9 +499,14 @@ int ofspmm_sample_neighbors(const ofspmm_csr* A, const void* dst, int64_t num_ds
   if (cap > 0 && (blk_col == nullptr || src_nodes == nullptr)) return OFSPMM_ERR_INVALID_ARG;
   // a values array exactly when A has values (a forgotten value dtype is caught, not ignored)
   if (unit(A) ? blk_val != nullptr : (cap > 0 && blk_val == nullptr)) return OFSPMM_ERR_INVALID_ARG;
-  if (int rc = check_ws(workspace, workspace_bytes, sample_neighbors_workspace_bytes(num_dst, cap))) return rc;
-  return launch_sample_neighbors(A, dst, num_dst, fanout, rng_seed, cap, blk_crow, blk_col, blk_val, src_nodes, counts,
-                                 workspace, reinterpret_cast<cudaStream_t>(stream));
+  if (int rc = check_sample_opts(opts)) return rc;
+  // an edge-id array exactly when asked for
+  const bool eid = sample_edge_ids(opts);
+  if (eid ? (cap > 0 && blk_eid == nullptr) : blk_eid != nullptr) return OFSPMM_ERR_INVALID_ARG;
+  if (int rc = check_ws(workspace, workspace_bytes, sample_neighbors_workspace_bytes(num_dst, cap, eid))) return rc;
+  return launch_sample_neighbors(A, opts, dst, num_dst, fanout, rng_seed, cap, blk_crow, blk_col, blk_val,
+                                 eid ? blk_eid : nullptr, src_nodes, counts, workspace,
+                                 reinterpret_cast<cudaStream_t>(stream));
 }
 
 int ofspmm_csr_expand_rows(const void* crow, int idx_dtype, int64_t rows, int64_t* row_of_nnz, ofspmm_stream_t stream) {

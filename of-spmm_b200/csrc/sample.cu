@@ -1,13 +1,19 @@
-// sample.cu — device neighbour sampling (DESIGN.md §3.8): for each destination v, the k = min(deg,
-// fanout) entries of row v with the smallest (key, j), key = mix(mix(seed ^ v) + j) (splitmix64), then
-// a relabel of the sampled columns into a bipartite block (DGL's block convention: the destinations
-// come first in src_nodes, then the other sampled ids in ascending order).
+// sample.cu — device neighbour sampling (DESIGN.md §3.8): for each destination v, the k entries of
+// row v with the smallest (key, j), then a relabel of the sampled columns into a bipartite block
+// (DGL's block convention: the destinations come first in src_nodes, then the other sampled ids in
+// ascending order).  Uniform: k = min(deg, fanout), key = x = mix(mix(seed ^ v) + j) (splitmix64);
+// weighted: k = min(npos, fanout), key = bits(neglog(U(x)) / w_j), all ones for an ineligible weight
+// (sample_key.h); with replacement: k = fanout independent draws j_t = mulhi(x(seed, v, t), deg).
 //   count   one thread per destination: validity (range, repeats found in the sorted ids), k, and a
 //           list of the rows long enough for a whole CTA;
+//   npos    weighted only: eligible entries per row, one warp per row (one CTA per long row);
+//           k = min(npos, fanout);
 //   select  one warp per destination (one CTA per long row): radix selection of the k-th smallest
-//           key over re-hashed keys, 8 bits per pass, stopping as soon as the bucket holding the
+//           key over re-computed keys, 8 bits per pass, stopping as soon as the bucket holding the
 //           k-th key is taken whole; then one pass that emits the selected entries in ascending j
 //           (ballot compaction), loading col / val for those only.  A row with deg <= k is copied.
+//   draw    with replacement: one warp per destination, the draws in order t, col / val loaded at
+//           the drawn positions only.
 //   relabel radix sort of the sampled ids (cub, as the transpose does), unique / not-a-destination
 //           flags, one scan that also compacts away the out-of-range columns, and a binary search
 //           per kept entry for its local id.
@@ -16,6 +22,7 @@
 #include <cub/device/device_scan.cuh>
 
 #include "launch.cuh"
+#include "sample_key.h"
 
 namespace ofspmm {
 
@@ -26,15 +33,33 @@ constexpr int kSampleWarps = 8;         // warps per CTA of the warp-per-row ker
 constexpr int kLongThreads = 512;       // threads per CTA of the long-row kernel
 constexpr long long kLongRow = 4096;    // rows longer than this are sampled by a whole CTA
 
-__device__ __forceinline__ unsigned long long mix64(unsigned long long x) {
-  x *= 0x9E3779B97F4A7C15ull;
-  x ^= x >> 30;
-  x *= 0xBF58476D1CE4E5B9ull;
-  x ^= x >> 27;
-  x *= 0x94D049BB133111EBull;
-  x ^= x >> 31;
-  return x;
-}
+enum SampleMode { kUniform, kWeighted, kReplace };
+
+// Keys of the selection: position j of the row that starts at entry b of A.
+struct UniformKey {
+  unsigned long long h0;
+  __device__ __forceinline__ UniformKey(unsigned long long seed, long long v, long long, const void*)
+      : h0(sk_mix64(seed ^ static_cast<unsigned long long>(v))) {}
+  __device__ __forceinline__ unsigned long long operator()(long long j) const {
+    return sk_mix64(h0 + static_cast<unsigned long long>(j));
+  }
+};
+
+// A weight widened exactly to fp64: fp32 bits, or bf16 bits (the high half of an fp32).
+__device__ __forceinline__ double widen(uint32_t b) { return static_cast<double>(__uint_as_float(b)); }
+__device__ __forceinline__ double widen(uint16_t b) { return static_cast<double>(__uint_as_float(static_cast<uint32_t>(b) << 16)); }
+
+// PT: uint32_t (fp32 weights) or uint16_t (bf16 weights).  The weight is re-read per evaluation.
+template <typename PT>
+struct WeightedKey {
+  unsigned long long h0;
+  const PT* p;
+  __device__ __forceinline__ WeightedKey(unsigned long long seed, long long v, long long b, const void* prob)
+      : h0(sk_mix64(seed ^ static_cast<unsigned long long>(v))), p(static_cast<const PT*>(prob) + b) {}
+  __device__ __forceinline__ unsigned long long operator()(long long j) const {
+    return sk_weighted_key(sk_mix64(h0 + static_cast<unsigned long long>(j)), widen(p[j]));
+  }
+};
 
 // Bits of a sort key that holds ids in [0, rows] (rows itself is the "no id" sentinel).
 int id_bits(long long rows) {
@@ -66,10 +91,11 @@ __global__ void sample_dst_keys_kernel(const IdxT* __restrict__ dst, long long n
 }
 
 // kcnt[i] = k of destination i (0 for an invalid one: out of range, or an id that occurs more than
-// once); kcnt[num_dst] = 0 so that the exclusive scan ends in the total.
+// once); kcnt[num_dst] = 0 so that the exclusive scan ends in the total.  Weighted: k from deg is
+// only an upper bound, which sample_npos / sample_npos_long turn into min(npos, fanout).
 template <typename IdxT>
 __global__ void sample_count_kernel(const IdxT* __restrict__ crow, const IdxT* __restrict__ dst, long long num_dst,
-                                    long long rows, long long fanout, const unsigned* __restrict__ dkey_sorted,
+                                    long long rows, long long fanout, int mode, const unsigned* __restrict__ dkey_sorted,
                                     long long* __restrict__ kcnt, int* __restrict__ longs, unsigned* __restrict__ nlong,
                                     long long* __restrict__ counts) {
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
@@ -85,12 +111,65 @@ __global__ void sample_count_kernel(const IdxT* __restrict__ crow, const IdxT* _
   long long k = 0;
   if (valid) {
     const long long deg = static_cast<long long>(crow[v + 1]) - static_cast<long long>(crow[v]);
-    k = fanout < 0 ? deg : (deg < fanout ? deg : fanout);
-    if (k > 0 && deg > kLongRow) longs[atomicAdd(nlong, 1u)] = static_cast<int>(i);
+    if (mode == kReplace) {
+      k = deg > 0 ? fanout : 0;   // fanout >= 0: draws need no selection, hence no long-row list
+    } else {
+      k = fanout < 0 ? deg : (deg < fanout ? deg : fanout);
+      if (k > 0 && deg > kLongRow) longs[atomicAdd(nlong, 1u)] = static_cast<int>(i);
+    }
   } else {
     atomicAdd(reinterpret_cast<unsigned long long*>(&counts[2]), 1ull);
   }
   kcnt[i] = k;
+}
+
+// Weighted: kcnt[i] = min(npos, fanout) (npos for fanout -1) of the listed long rows, one CTA per
+// row, as their selection runs.
+template <typename IdxT, typename PT>
+__global__ void __launch_bounds__(kLongThreads)
+sample_npos_long_kernel(const IdxT* __restrict__ crow, const IdxT* __restrict__ dst, long long fanout,
+                        const PT* __restrict__ prob, const int* __restrict__ longs, const unsigned* __restrict__ nlong,
+                        long long* __restrict__ kcnt) {
+  __shared__ unsigned warp_cnt[kLongThreads / 32];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const unsigned n = *nlong;
+  for (unsigned r = blockIdx.x; r < n; r += gridDim.x) {
+    const long long i = longs[r];
+    const long long v = static_cast<long long>(dst[i]);
+    const long long b = static_cast<long long>(crow[v]), deg = static_cast<long long>(crow[v + 1]) - b;
+    unsigned c = 0;
+    for (long long j = threadIdx.x; j < deg; j += kLongThreads) c += sk_eligible(widen(prob[b + j])) ? 1u : 0u;
+    c = __reduce_add_sync(kFull, c);
+    if (lane == 0) warp_cnt[warp] = c;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      long long npos = 0;
+#pragma unroll
+      for (int w = 0; w < kLongThreads / 32; ++w) npos += warp_cnt[w];
+      kcnt[i] = fanout >= 0 && npos > fanout ? fanout : npos;
+    }
+    __syncthreads();   // warp_cnt is rewritten for the next row
+  }
+}
+
+// Weighted: kcnt[i] = min(npos, fanout) (npos for fanout -1), one warp per destination of at most
+// kLongRow entries; the longer ones are sample_npos_long's.
+template <typename IdxT, typename PT>
+__global__ void __launch_bounds__(kSampleWarps * 32)
+sample_npos_kernel(const IdxT* __restrict__ crow, const IdxT* __restrict__ dst, long long num_dst, long long fanout,
+                   const PT* __restrict__ prob, long long* __restrict__ kcnt) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const long long step = static_cast<long long>(gridDim.x) * kSampleWarps;
+  for (long long i = static_cast<long long>(blockIdx.x) * kSampleWarps + warp; i < num_dst; i += step) {
+    if (kcnt[i] == 0) continue;   // invalid, empty row or fanout 0
+    const long long v = static_cast<long long>(dst[i]);
+    const long long b = static_cast<long long>(crow[v]), deg = static_cast<long long>(crow[v + 1]) - b;
+    if (deg > kLongRow) continue;
+    unsigned c = 0;
+    for (long long j = lane; j < deg; j += 32) c += sk_eligible(widen(prob[b + j])) ? 1u : 0u;
+    const long long npos = __reduce_add_sync(kFull, c);
+    if (lane == 0) kcnt[i] = fanout >= 0 && npos > fanout ? fanout : npos;
+  }
 }
 
 // Slots the selection does not fill (all of them when the capacity is exceeded) hold the sentinel,
@@ -134,12 +213,14 @@ __device__ __forceinline__ long long group_prefix(int* slots, int warp, int lane
   return before;
 }
 
-// Samples row v (entries [b, b + deg) of A) into stage slots [off, off + k), in ascending j.
-// Uniform over the group: every thread calls it with the same arguments except `tid`.
-template <int G, typename IdxT, typename VT>
+// Samples row v (entries [b, b + deg) of A) into stage slots [off, off + k), in ascending j, by the
+// keys key(j).  Uniform over the group: every thread calls it with the same arguments except `tid`.
+// stage_eid (may be null) receives the positions b + j in A.
+template <int G, typename IdxT, typename VT, typename Key>
 __device__ void sample_row(RowShared<G>& sh, int tid, const IdxT* __restrict__ col, const VT* __restrict__ val,
-                           long long b, long long deg, long long k, unsigned long long h0, long long cols,
-                           long long off, unsigned* __restrict__ stage_col, VT* __restrict__ stage_val) {
+                           long long b, long long deg, long long k, const Key& key_of, long long cols,
+                           long long off, unsigned* __restrict__ stage_col, VT* __restrict__ stage_val,
+                           long long* __restrict__ stage_eid) {
   const int lane = tid & 31, warp = tid >> 5;
   const unsigned lt_mask = (1u << lane) - 1u;
   const bool all = k >= deg;
@@ -153,7 +234,7 @@ __device__ void sample_row(RowShared<G>& sh, int tid, const IdxT* __restrict__ c
       for (int i = tid; i < 256; i += G) sh.hist[i] = 0;
       group_sync<G>();
       for (long long j = tid; j < deg; j += G) {
-        const unsigned long long key = mix64(h0 + static_cast<unsigned long long>(j));
+        const unsigned long long key = key_of(j);
         if ((key & mask) == prefix) atomicAdd(&sh.hist[(key >> shift) & 255], 1u);
       }
       group_sync<G>();
@@ -198,7 +279,7 @@ __device__ void sample_row(RowShared<G>& sh, int tid, const IdxT* __restrict__ c
     const bool in = j < deg;
     bool sel = in;
     if (!all) {
-      const unsigned long long key = in ? mix64(h0 + static_cast<unsigned long long>(j)) : 0ull;
+      const unsigned long long key = in ? key_of(j) : 0ull;
       const bool eq = in && key == thr;
       const unsigned eqm = __ballot_sync(kFull, eq);
       long long eq_rank = eq_before + __popc(eqm & lt_mask), eq_total = __popc(eqm);
@@ -213,18 +294,20 @@ __device__ void sample_row(RowShared<G>& sh, int tid, const IdxT* __restrict__ c
       const long long c = static_cast<long long>(col[b + j]);
       stage_col[off + pos] = static_cast<unsigned>(c >= 0 && c < cols ? c : cols);
       if (val != nullptr) stage_val[off + pos] = val[b + j];
+      if (stage_eid != nullptr) stage_eid[off + pos] = b + j;
     }
     sel_before += sel_total;
     group_sync<G>();   // warp_eq / warp_sel are rewritten by the next chunk
   }
 }
 
-template <typename IdxT, typename VT>
+template <typename IdxT, typename VT, typename Key>
 __global__ void __launch_bounds__(kSampleWarps * 32)
 sample_rows_warp_kernel(const IdxT* __restrict__ crow, const IdxT* __restrict__ col, const VT* __restrict__ val,
                         long long cols, const IdxT* __restrict__ dst, long long num_dst,
                         const long long* __restrict__ slot, long long cap, unsigned long long seed,
-                        unsigned* __restrict__ stage_col, VT* __restrict__ stage_val) {
+                        const void* __restrict__ prob, unsigned* __restrict__ stage_col, VT* __restrict__ stage_val,
+                        long long* __restrict__ stage_eid) {
   __shared__ RowShared<32> sh[kSampleWarps];
   if (slot[num_dst] > cap) return;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -235,28 +318,56 @@ sample_rows_warp_kernel(const IdxT* __restrict__ crow, const IdxT* __restrict__ 
     const long long v = static_cast<long long>(dst[i]);
     const long long b = static_cast<long long>(crow[v]), deg = static_cast<long long>(crow[v + 1]) - b;
     if (deg > kLongRow) continue;
-    sample_row<32>(sh[warp], lane, col, val, b, deg, k, mix64(seed ^ static_cast<unsigned long long>(v)), cols, off,
-                   stage_col, stage_val);
+    sample_row<32>(sh[warp], lane, col, val, b, deg, k, Key(seed, v, b, prob), cols, off, stage_col, stage_val,
+                   stage_eid);
   }
 }
 
-template <typename IdxT, typename VT>
+template <typename IdxT, typename VT, typename Key>
 __global__ void __launch_bounds__(kLongThreads)
 sample_long_rows_kernel(const IdxT* __restrict__ crow, const IdxT* __restrict__ col, const VT* __restrict__ val,
                         long long cols, const IdxT* __restrict__ dst, long long num_dst,
                         const long long* __restrict__ slot, long long cap, unsigned long long seed,
-                        const int* __restrict__ longs, const unsigned* __restrict__ nlong,
-                        unsigned* __restrict__ stage_col, VT* __restrict__ stage_val) {
+                        const void* __restrict__ prob, const int* __restrict__ longs, const unsigned* __restrict__ nlong,
+                        unsigned* __restrict__ stage_col, VT* __restrict__ stage_val, long long* __restrict__ stage_eid) {
   __shared__ RowShared<kLongThreads> sh;
   if (slot[num_dst] > cap) return;
   const unsigned n = *nlong;
   for (unsigned r = blockIdx.x; r < n; r += gridDim.x) {
     const long long i = longs[r];
     const long long off = slot[i], k = slot[i + 1] - off;
+    if (k == 0) continue;   // weighted: no eligible entry
     const long long v = static_cast<long long>(dst[i]);
     const long long b = static_cast<long long>(crow[v]), deg = static_cast<long long>(crow[v + 1]) - b;
-    sample_row<kLongThreads>(sh, threadIdx.x, col, val, b, deg, k, mix64(seed ^ static_cast<unsigned long long>(v)),
-                             cols, off, stage_col, stage_val);
+    sample_row<kLongThreads>(sh, threadIdx.x, col, val, b, deg, k, Key(seed, v, b, prob), cols, off, stage_col,
+                             stage_val, stage_eid);
+  }
+}
+
+// With replacement: draw t of destination v takes position j_t = mulhi(x(seed, v, t), deg) into
+// slot off + t; one warp per destination, col / val read at the drawn positions only.
+template <typename IdxT, typename VT>
+__global__ void __launch_bounds__(kSampleWarps * 32)
+sample_draw_kernel(const IdxT* __restrict__ crow, const IdxT* __restrict__ col, const VT* __restrict__ val,
+                   long long cols, const IdxT* __restrict__ dst, long long num_dst, const long long* __restrict__ slot,
+                   long long cap, unsigned long long seed, unsigned* __restrict__ stage_col,
+                   VT* __restrict__ stage_val, long long* __restrict__ stage_eid) {
+  if (slot[num_dst] > cap) return;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const long long step = static_cast<long long>(gridDim.x) * kSampleWarps;
+  for (long long i = static_cast<long long>(blockIdx.x) * kSampleWarps + warp; i < num_dst; i += step) {
+    const long long off = slot[i], k = slot[i + 1] - off;
+    if (k == 0) continue;
+    const long long v = static_cast<long long>(dst[i]);
+    const long long b = static_cast<long long>(crow[v]), deg = static_cast<long long>(crow[v + 1]) - b;
+    const UniformKey x(seed, v, b, nullptr);
+    for (long long t = lane; t < k; t += 32) {
+      const long long e = b + static_cast<long long>(__umul64hi(x(t), static_cast<unsigned long long>(deg)));
+      const long long c = static_cast<long long>(col[e]);
+      stage_col[off + t] = static_cast<unsigned>(c >= 0 && c < cols ? c : cols);
+      if (val != nullptr) stage_val[off + t] = val[e];
+      if (stage_eid != nullptr) stage_eid[off + t] = e;
+    }
   }
 }
 
@@ -282,11 +393,13 @@ __global__ void sample_flags_kernel(const unsigned* __restrict__ stage_col, cons
 template <typename IdxT, typename VT>
 __global__ void sample_emit_kernel(const IdxT* __restrict__ dst, long long num_dst, const long long* __restrict__ slot,
                                    long long cap, const unsigned* __restrict__ stage_col,
-                                   const VT* __restrict__ stage_val, const unsigned* __restrict__ ids,
+                                   const VT* __restrict__ stage_val, const long long* __restrict__ stage_eid,
+                                   const unsigned* __restrict__ ids,
                                    const unsigned* __restrict__ dkey_sorted, const int* __restrict__ didx_sorted,
                                    const long long* __restrict__ flag, const long long* __restrict__ scan,
                                    unsigned sentinel, int* __restrict__ blk_crow, int* __restrict__ blk_col,
-                                   VT* __restrict__ blk_val, IdxT* __restrict__ src_nodes, long long* __restrict__ counts) {
+                                   VT* __restrict__ blk_val, IdxT* __restrict__ blk_eid, IdxT* __restrict__ src_nodes,
+                                   long long* __restrict__ counts) {
   const long long total = slot[num_dst];
   const long long tid = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (total > cap) {   // outputs invalid: only the needed size is reported
@@ -307,6 +420,7 @@ __global__ void sample_emit_kernel(const IdxT* __restrict__ dst, long long num_d
         const long long q = scan[p] >> 32;
         blk_col[q] = static_cast<int>(local);
         if (blk_val != nullptr) blk_val[q] = stage_val[p];
+        if (blk_eid != nullptr) blk_eid[q] = static_cast<IdxT>(stage_eid[p]);
       }
       if (flag[p] & 1) src_nodes[num_dst + (scan[p] & kLow)] = static_cast<IdxT>(ids[p]);
     }
@@ -321,10 +435,10 @@ __global__ void sample_emit_kernel(const IdxT* __restrict__ dst, long long num_d
 
 struct SampleLayout {
   size_t hdr, dkey_in, dkey_out, didx_in, didx_out, kcnt, slot, longs, stage_col, ids, stage_val, flag, scan, cub_tmp,
-      cub_bytes, total;
+      cub_bytes, stage_eid, total;
 };
 
-SampleLayout sample_layout(int64_t num_dst, int64_t cap) {
+SampleLayout sample_layout(int64_t num_dst, int64_t cap, bool edge_ids) {
   SampleLayout L;
   const size_t nd = static_cast<size_t>(num_dst > 0 ? num_dst : 1), nc = static_cast<size_t>(cap > 0 ? cap : 1);
   Carve c;
@@ -356,15 +470,23 @@ SampleLayout sample_layout(int64_t num_dst, int64_t cap) {
   if (b3 > L.cub_bytes) L.cub_bytes = b3;
   if (b4 > L.cub_bytes) L.cub_bytes = b4;
   L.cub_tmp = c.take(L.cub_bytes);
+  L.stage_eid = edge_ids ? c.take(nc * 8) : 0;   // last, so that the layout without it is unchanged
   L.total = c.total;
   return L;
 }
 
+// The sampling mode of a call and its weights (validated options; NULL options: uniform).
+struct SampleCall {
+  int mode;
+  const void* prob;
+  int prob_dtype;
+};
+
 template <typename IdxT, typename VT>
-int sample_impl(const ofspmm_csr* A, const void* dst_v, int64_t num_dst, int64_t fanout, uint64_t seed, int64_t cap,
-                void* blk_crow, void* blk_col, void* blk_val, void* src_nodes, int64_t* counts, void* ws,
-                cudaStream_t stream) {
-  const SampleLayout L = sample_layout(num_dst, cap);
+int sample_impl(const ofspmm_csr* A, const SampleCall& m, const void* dst_v, int64_t num_dst, int64_t fanout,
+                uint64_t seed, int64_t cap, void* blk_crow, void* blk_col, void* blk_val, void* blk_eid,
+                void* src_nodes, int64_t* counts, void* ws, cudaStream_t stream) {
+  const SampleLayout L = sample_layout(num_dst, cap, blk_eid != nullptr);
   unsigned char* w = static_cast<unsigned char*>(ws);
   unsigned* nlong = reinterpret_cast<unsigned*>(w + L.hdr);
   unsigned* dkey_in = reinterpret_cast<unsigned*>(w + L.dkey_in);
@@ -377,6 +499,7 @@ int sample_impl(const ofspmm_csr* A, const void* dst_v, int64_t num_dst, int64_t
   unsigned* stage_col = reinterpret_cast<unsigned*>(w + L.stage_col);
   unsigned* ids = reinterpret_cast<unsigned*>(w + L.ids);
   VT* stage_val = reinterpret_cast<VT*>(w + L.stage_val);
+  long long* stage_eid = blk_eid != nullptr ? reinterpret_cast<long long*>(w + L.stage_eid) : nullptr;
   long long* flag = reinterpret_cast<long long*>(w + L.flag);
   long long* scan = reinterpret_cast<long long*>(w + L.scan);
   void* tmp = w + L.cub_tmp;
@@ -390,6 +513,8 @@ int sample_impl(const ofspmm_csr* A, const void* dst_v, int64_t num_dst, int64_t
   DevInfo dev;
   if (int rc = get_dev_info(&dev)) return rc;
   auto blocks = [&](long long n) { return grid_for(n, 256, dev.sms * 8, dev.sms); };
+  const long long wblocks = (num_dst + kSampleWarps - 1) / kSampleWarps;
+  const unsigned wgrid = static_cast<unsigned>(wblocks < dev.sms * 16 ? wblocks : dev.sms * 16);
 
   OFSPMM_CUDA_OK(cudaMemsetAsync(counts, 0, 3 * sizeof(int64_t), stream));
   OFSPMM_CUDA_OK(cudaMemsetAsync(nlong, 0, sizeof(unsigned), stream));
@@ -403,8 +528,30 @@ int sample_impl(const ofspmm_csr* A, const void* dst_v, int64_t num_dst, int64_t
     count_launch(4);
   }
   sample_count_kernel<IdxT><<<static_cast<unsigned>((num_dst + 1 + 255) / 256), 256, 0, stream>>>(
-      crow, dst, num_dst, rows, fanout, dkey, kcnt, longs, nlong, reinterpret_cast<long long*>(counts));
+      crow, dst, num_dst, rows, fanout, m.mode, dkey, kcnt, longs, nlong, reinterpret_cast<long long*>(counts));
   count_launch();
+  // f(Tag<PT>{}) for the weights' bit type: fp32 or bf16 words
+  auto by_prob = [&](auto&& f) { m.prob_dtype == OFSPMM_DTYPE_FLOAT ? f(Tag<uint32_t>{}) : f(Tag<uint16_t>{}); };
+  if (m.mode == kWeighted && num_dst > 0) {
+    by_prob([&](auto pt) {   // k = min(npos, fanout)
+      using PT = typename decltype(pt)::type;
+      const PT* prob = static_cast<const PT*>(m.prob);
+      const long long lgrid = num_dst < dev.sms * 2 ? num_dst : dev.sms * 2;
+      sample_npos_long_kernel<IdxT, PT><<<static_cast<unsigned>(lgrid), kLongThreads, 0, stream>>>(
+          crow, dst, fanout, prob, longs, nlong, kcnt);
+      sample_npos_kernel<IdxT, PT><<<wgrid, kSampleWarps * 32, 0, stream>>>(crow, dst, num_dst, fanout, prob, kcnt);
+      count_launch(2);
+    });
+  }
+  auto select = [&](auto key) {
+    using Key = typename decltype(key)::type;
+    sample_rows_warp_kernel<IdxT, VT, Key><<<wgrid, kSampleWarps * 32, 0, stream>>>(
+        crow, col, val, A->cols, dst, num_dst, slot, cap, seed, m.prob, stage_col, stage_val, stage_eid);
+    const long long lgrid = num_dst < dev.sms * 2 ? num_dst : dev.sms * 2;
+    sample_long_rows_kernel<IdxT, VT, Key><<<static_cast<unsigned>(lgrid), kLongThreads, 0, stream>>>(
+        crow, col, val, A->cols, dst, num_dst, slot, cap, seed, m.prob, longs, nlong, stage_col, stage_val, stage_eid);
+    count_launch(2);
+  };
   cub_bytes = L.cub_bytes;
   OFSPMM_CUDA_OK(cub::DeviceScan::ExclusiveSum(tmp, cub_bytes, static_cast<const long long*>(kcnt), slot,
                                                static_cast<int>(num_dst + 1), stream));
@@ -414,14 +561,15 @@ int sample_impl(const ofspmm_csr* A, const void* dst_v, int64_t num_dst, int64_t
     count_launch();
   }
   if (num_dst > 0) {
-    const long long wblocks = (num_dst + kSampleWarps - 1) / kSampleWarps;
-    const unsigned wgrid = static_cast<unsigned>(wblocks < dev.sms * 16 ? wblocks : dev.sms * 16);
-    sample_rows_warp_kernel<IdxT, VT><<<wgrid, kSampleWarps * 32, 0, stream>>>(
-        crow, col, val, A->cols, dst, num_dst, slot, cap, seed, stage_col, stage_val);
-    const long long lgrid = num_dst < dev.sms * 2 ? num_dst : dev.sms * 2;
-    sample_long_rows_kernel<IdxT, VT><<<static_cast<unsigned>(lgrid), kLongThreads, 0, stream>>>(
-        crow, col, val, A->cols, dst, num_dst, slot, cap, seed, longs, nlong, stage_col, stage_val);
-    count_launch(2);
+    if (m.mode == kReplace) {
+      sample_draw_kernel<IdxT, VT><<<wgrid, kSampleWarps * 32, 0, stream>>>(
+          crow, col, val, A->cols, dst, num_dst, slot, cap, seed, stage_col, stage_val, stage_eid);
+      count_launch();
+    } else if (m.mode == kWeighted) {
+      by_prob([&](auto pt) { select(Tag<WeightedKey<typename decltype(pt)::type>>{}); });
+    } else {
+      select(Tag<UniformKey>{});
+    }
   }
   if (cap > 0) {
     cub_bytes = L.cub_bytes;
@@ -436,29 +584,35 @@ int sample_impl(const ofspmm_csr* A, const void* dst_v, int64_t num_dst, int64_t
                                                static_cast<int>(cap + 1), stream));
   count_launch(2);
   sample_emit_kernel<IdxT, VT><<<blocks(cap > num_dst + 1 ? cap : num_dst + 1), 256, 0, stream>>>(
-      dst, num_dst, slot, cap, stage_col, stage_val, ids, dkey, didx, flag, scan, sentinel,
-      static_cast<int*>(blk_crow), static_cast<int*>(blk_col), static_cast<VT*>(blk_val), static_cast<IdxT*>(src_nodes),
-      reinterpret_cast<long long*>(counts));
+      dst, num_dst, slot, cap, stage_col, stage_val, stage_eid, ids, dkey, didx, flag, scan, sentinel,
+      static_cast<int*>(blk_crow), static_cast<int*>(blk_col), static_cast<VT*>(blk_val), static_cast<IdxT*>(blk_eid),
+      static_cast<IdxT*>(src_nodes), reinterpret_cast<long long*>(counts));
   return launched();
 }
 
 }  // namespace
 
-size_t sample_neighbors_workspace_bytes(int64_t num_dst, int64_t cap) { return sample_layout(num_dst, cap).total; }
+size_t sample_neighbors_workspace_bytes(int64_t num_dst, int64_t cap, bool edge_ids) {
+  return sample_layout(num_dst, cap, edge_ids).total;
+}
 
-int launch_sample_neighbors(const ofspmm_csr* A, const void* dst, int64_t num_dst, int64_t fanout, uint64_t seed,
-                            int64_t cap, void* blk_crow, void* blk_col, void* blk_val, void* src_nodes, int64_t* counts,
-                            void* ws, cudaStream_t stream) {
+int launch_sample_neighbors(const ofspmm_csr* A, const ofspmm_sample_opts* opts, const void* dst, int64_t num_dst,
+                            int64_t fanout, uint64_t seed, int64_t cap, void* blk_crow, void* blk_col, void* blk_val,
+                            void* blk_eid, void* src_nodes, int64_t* counts, void* ws, cudaStream_t stream) {
+  SampleCall m{kUniform, nullptr, 0};
+  if (opts != nullptr && opts->prob != nullptr) m = {kWeighted, opts->prob, opts->prob_dtype};
+  // fanout -1 with replacement is every entry once: the same block as without replacement
+  else if (opts != nullptr && (opts->flags & OFSPMM_SAMPLE_REPLACE) && fanout >= 0) m.mode = kReplace;
   return dispatch_idx(A->idx_dtype, [&](auto idx) {
     using IdxT = typename decltype(idx)::type;
     // values are copied bit for bit: fp32 as 32-bit, bf16 as 16-bit words; a pattern matrix has none
     if (A->val_dtype == OFSPMM_VAL_UNIT)
-      return sample_impl<IdxT, uint8_t>(A, dst, num_dst, fanout, seed, cap, blk_crow, blk_col, nullptr, src_nodes, counts,
-                                        ws, stream);
+      return sample_impl<IdxT, uint8_t>(A, m, dst, num_dst, fanout, seed, cap, blk_crow, blk_col, nullptr, blk_eid,
+                                        src_nodes, counts, ws, stream);
     return dispatch_dense(A->val_dtype, [&](auto vt) {
       using VT = std::conditional_t<sizeof(typename decltype(vt)::type) == 4, uint32_t, uint16_t>;
-      return sample_impl<IdxT, VT>(A, dst, num_dst, fanout, seed, cap, blk_crow, blk_col, blk_val, src_nodes, counts, ws,
-                                   stream);
+      return sample_impl<IdxT, VT>(A, m, dst, num_dst, fanout, seed, cap, blk_crow, blk_col, blk_val, blk_eid,
+                                   src_nodes, counts, ws, stream);
     });
   });
 }

@@ -485,15 +485,27 @@ def csr_transpose(a_crow, a_col, a_val, a_rows: int, a_cols: int, want_perm: boo
 
 
 def sample_neighbors(a_crow, a_col, a_val, a_rows: int, a_cols: int, dst: torch.Tensor, fanout: int,
-                     rng_seed: int) -> Tuple[torch.Tensor, torch.Tensor, Optional[torch.Tensor], torch.Tensor]:
-    """One fan-out-sampled bipartite block of the square CSR A (``ofspmm_sample_neighbors``): for
+                     rng_seed: int, *, prob: Optional[torch.Tensor] = None, replace: bool = False,
+                     return_eid: bool = False):
+    """One fan-out-sampled bipartite block of the square CSR A (``ofspmm_sample_neighbors_ex``): for
     each destination ``dst[i]``, at most ``fanout`` of its entries (all of them for -1), chosen by
     the keys of include/ofspmm.h — uniform without replacement, a pure function of
     (rng_seed, node, position).  Returns ``(blk_crow, blk_col, blk_val, src_nodes)``: an int32 CSR
     of len(dst) x len(src_nodes) whose columns index ``src_nodes`` (dst first, then the other
     sampled ids ascending); ``blk_val`` is None for a pattern matrix.  One device-to-host read (two
-    with fanout -1); invalid destinations (out of range, repeated) raise."""
-    _check_device(a_crow, a_col, a_val, dst)
+    with fanout -1); invalid destinations (out of range, repeated) raise.
+
+    ``prob`` (nnz float32 / bfloat16 weights, e.g. ``a_val``): weighted sampling without
+    replacement, entry j of a row picked with probability proportional to its weight (k = 1);
+    entries whose weight is not positive and finite are never picked.  ``replace=True``: exactly
+    ``fanout`` uniform draws per non-empty row, in draw order, repeats kept (multi-edges); not with
+    ``prob``.  ``return_eid=True`` appends ``eid``, the position in A (A's index dtype) of every
+    block entry: ``a_col[eid] == src_nodes[blk_col]`` and ``a_val[eid] == blk_val``."""
+    if prob is not None:
+        _chk(not replace, "weighted sampling with replacement is not supported (prob with replace=True)")
+        _chk(prob.dim() == 1 and prob.numel() == a_col.numel() and prob.dtype in _DENSE,
+             "prob must hold nnz float32 / bfloat16 weights")
+    _check_device(a_crow, a_col, a_val, dst, prob)
     _chk(a_crow.dim() == 1 and a_col.dim() == 1 and dst.dim() == 1, "a_crow, a_col and dst must be 1-D")
     _chk(a_crow.dtype in _INDEX and a_col.dtype == a_crow.dtype, "a_crow / a_col must share an index dtype (int32/int64)")
     _chk(a_rows == a_cols, f"neighbour sampling needs a square matrix, got {a_rows} x {a_cols}")
@@ -512,24 +524,32 @@ def sample_neighbors(a_crow, a_col, a_val, a_rows: int, a_cols: int, dst: torch.
         d = torch.where(ok, dst, torch.zeros_like(dst)).long()
         deg = (a_crow[1:][d] - a_crow[:-1][d]) * ok if a_rows > 0 else torch.zeros_like(d)
         cap = int(deg.sum())
+    elif replace:
+        cap = num_dst * fanout             # draws may repeat: not bounded by nnz
     else:
         cap = min(num_dst * fanout, nnz)   # at most one kept entry per non-zero of A
     blk_crow = torch.empty(num_dst + 1, dtype=torch.int32, device=dev)
     blk_col = torch.empty(cap, dtype=torch.int32, device=dev)
     blk_val = torch.empty(cap, dtype=a_val.dtype, device=dev) if a_val is not None else None
+    blk_eid = torch.empty(cap, dtype=idt, device=dev) if return_eid else None
     src_nodes = torch.empty(num_dst + cap, dtype=idt, device=dev)
     counts = torch.empty(3, dtype=torch.int64, device=dev)
+    flags = (_lib.SAMPLE_REPLACE if replace else 0) | (_lib.SAMPLE_EDGE_IDS if return_eid else 0)
+    sopts = _lib.SampleOptsStruct(flags, _DENSE[prob.dtype] if prob is not None else 0, _ptr(prob))
+    opts = ctypes.byref(sopts) if flags or prob is not None else None
     L = _lib.lib()
     with torch.cuda.device(dev):
         A = _csr_struct(a_crow, a_col, a_val, a_rows, a_cols)
-        nbytes = L.ofspmm_sample_neighbors_workspace_bytes(num_dst, cap, _INDEX[idt])
+        nbytes = L.ofspmm_sample_neighbors_ex_workspace_bytes(num_dst, cap, _INDEX[idt], opts)
         ws, wsp = _workspace(nbytes, dev)
-        check(L.ofspmm_sample_neighbors(ctypes.byref(A), _ptr(dst), num_dst, fanout, rng_seed & (2 ** 64 - 1), cap,
-                                        _ptr(blk_crow), _ptr(blk_col), _ptr(blk_val), _ptr(src_nodes),
-                                        counts.data_ptr(), wsp, nbytes, _stream_ptr(dst)), "sample_neighbors")
+        check(L.ofspmm_sample_neighbors_ex(ctypes.byref(A), opts, _ptr(dst), num_dst, fanout, rng_seed & (2 ** 64 - 1),
+                                           cap, _ptr(blk_crow), _ptr(blk_col), _ptr(blk_val), _ptr(blk_eid),
+                                           _ptr(src_nodes), counts.data_ptr(), wsp, nbytes, _stream_ptr(dst)),
+              "sample_neighbors")
     nnz_blk, num_src, bad = counts.tolist()
     _chk(bad == 0, f"sample_neighbors: {bad} destination ids are out of range [0, {a_rows}) or repeated")
-    return (blk_crow, blk_col[:nnz_blk], blk_val[:nnz_blk] if blk_val is not None else None, src_nodes[:num_src])
+    out = (blk_crow, blk_col[:nnz_blk], blk_val[:nnz_blk] if blk_val is not None else None, src_nodes[:num_src])
+    return out + (blk_eid[:nnz_blk],) if return_eid else out
 
 
 def spmm_csr_grad_b_transient_compute(a_crow, a_col, a_val, dy, a_rows: int, a_cols: int,

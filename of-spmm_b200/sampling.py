@@ -14,7 +14,7 @@ on the device by ``ofspmm_sample_neighbors``.  A block's adjacency is an ordinar
 from __future__ import annotations
 
 from dataclasses import dataclass
-from typing import List, Sequence
+from typing import List, Optional, Sequence
 
 import torch
 
@@ -44,28 +44,38 @@ def hop_seed(rng_seed: int, hop: int) -> int:
 class Block:
     """One sampled layer: ``adj`` is ``num_dst x num_src`` (int32 CSR, ``val`` None for a pattern
     matrix), its columns index ``src_nodes`` (global ids, A's index dtype), and
-    ``src_nodes[:adj.rows]`` are the destination nodes themselves."""
+    ``src_nodes[:adj.rows]`` are the destination nodes themselves.  ``eid`` (with ``edge_ids=True``)
+    is the position in A of every entry of ``adj``, so ``w[eid]`` are the block's weights for
+    per-edge parameters ``w`` of the full graph, with gradients flowing back to ``w``."""
     adj: CsrMatrix
     src_nodes: torch.Tensor
+    eid: Optional[torch.Tensor] = None
 
     @property
     def dst_nodes(self) -> torch.Tensor:
         return self.src_nodes[:self.adj.rows]
 
 
-def sample_blocks(A: CsrMatrix, seeds: torch.Tensor, fanouts: Sequence[int], rng_seed: int) -> List[Block]:
+def sample_blocks(A: CsrMatrix, seeds: torch.Tensor, fanouts: Sequence[int], rng_seed: int, *,
+                  prob: Optional[torch.Tensor] = None, replace: bool = False, edge_ids: bool = False) -> List[Block]:
     """Samples ``len(fanouts)`` hops from ``seeds`` (distinct node ids of the square CSR ``A``, on
     its device).  Hop h starts from the previous hop's ``src_nodes`` and samples at most
     ``fanouts[h]`` neighbours per node (-1: all) with seed ``hop_seed(rng_seed, h)``.
 
     Returns the blocks input layer first: ``blocks[0]`` consumes ``X[blocks[0].src_nodes]`` and
     ``blocks[-1].src_nodes[:len(seeds)] == seeds``.  Deterministic in (A, seeds, fanouts, rng_seed).
-    A's values, if any, are carried into the blocks; ``A.val`` None samples the pattern."""
+    A's values, if any, are carried into the blocks; ``A.val`` None samples the pattern.
+
+    ``prob`` (nnz weights, e.g. ``A.val``): weighted sampling without replacement; ``replace``:
+    ``fanouts[h]`` uniform draws per node with repeats kept; ``edge_ids``: every block carries
+    ``eid`` (see ``ops.sample_neighbors``)."""
     blocks = []
     nodes = seeds
     for hop, fanout in enumerate(fanouts):
-        crow, col, val, src = ops.sample_neighbors(A.crow, A.col, A.val, A.rows, A.cols, nodes, int(fanout),
-                                                   hop_seed(rng_seed, hop))
-        blocks.append(Block(CsrMatrix(crow, col, val, int(nodes.numel()), int(src.numel())), src))
+        crow, col, val, src, *eid = ops.sample_neighbors(A.crow, A.col, A.val, A.rows, A.cols, nodes, int(fanout),
+                                                         hop_seed(rng_seed, hop), prob=prob, replace=replace,
+                                                         return_eid=edge_ids)
+        blocks.append(Block(CsrMatrix(crow, col, val, int(nodes.numel()), int(src.numel())), src,
+                            eid[0] if edge_ids else None))
         nodes = src
     return blocks[::-1]
