@@ -434,6 +434,19 @@ OFSPMM_API int ofspmm_sample_neighbors(const ofspmm_csr* A, const void* dst, int
  * A.val[blk_eid] equals blk_val bit for bit; a gradient wrt A's edge weights flows back through it.
  * blk_eid must be non-NULL with the flag (when cap > 0) and NULL without it.
  *
+ * Edge exclusion (OFSPMM_SAMPLE_EXCLUDE), in every mode: `exclude` holds `num_exclude` strictly
+ * ascending positions in A (A's index dtype), the edges a link-prediction batch predicts and their
+ * reverses, which its blocks must not contain.  Position j of row v is eligible iff crow[v] + j is
+ * not in `exclude` (weighted: and its weight is eligible); n_e = deg - (excluded entries of the row).
+ * Uniform: k = min(n_e, fanout) eligible entries with the smallest (x, j); weighted: npos counts the
+ * eligible entries; with replacement: draw t takes the r_t-th eligible position (ascending j), r_t =
+ * mulhi64(x(s, v, t), n_e), and n_e == 0 gives no draws.  The keys are those above, so a row
+ * without an excluded entry is sampled exactly as without the flag, and num_exclude == 0 is the
+ * call without it.  An `exclude` that is not strictly ascending gives unspecified (memory-safe)
+ * blocks.  The fields are read only with the flag, so callers built against the two-field struct
+ * are unaffected; the workspace does not depend on them.  With the flag, exclude == NULL and
+ * num_exclude > 0, or num_exclude < 0, is OFSPMM_ERR_INVALID_ARG.
+ *
  * OFSPMM_ERR_INVALID_ARG also for an unknown flag bit and a prob_dtype other than FLOAT / BFLOAT16.
  * The workspace depends on (num_dst, cap, flags) only; the workspace query returns 0 for invalid
  * arguments. */
@@ -441,8 +454,10 @@ typedef struct ofspmm_sample_opts {
   uint32_t flags;      /* OFSPMM_SAMPLE_* */
   int32_t prob_dtype;  /* dtype of prob: OFSPMM_DTYPE_FLOAT or OFSPMM_DTYPE_BFLOAT16 */
   const void* prob;    /* NULL: uniform; else nnz per-entry weights (device) */
+  const void* exclude; /* OFSPMM_SAMPLE_EXCLUDE: strictly ascending positions in A (device) */
+  int64_t num_exclude; /* OFSPMM_SAMPLE_EXCLUDE: entries of exclude */
 } ofspmm_sample_opts;
-enum { OFSPMM_SAMPLE_REPLACE = 1, OFSPMM_SAMPLE_EDGE_IDS = 2 };
+enum { OFSPMM_SAMPLE_REPLACE = 1, OFSPMM_SAMPLE_EDGE_IDS = 2, OFSPMM_SAMPLE_EXCLUDE = 8 };
 OFSPMM_API size_t ofspmm_sample_neighbors_ex_workspace_bytes(int64_t num_dst, int64_t cap, int idx_dtype,
                                                              const ofspmm_sample_opts* opts);
 OFSPMM_API int ofspmm_sample_neighbors_ex(const ofspmm_csr* A, const ofspmm_sample_opts* opts, const void* dst,
@@ -450,6 +465,32 @@ OFSPMM_API int ofspmm_sample_neighbors_ex(const ofspmm_csr* A, const ofspmm_samp
                                           void* blk_crow, void* blk_col, void* blk_val, void* blk_eid, void* src_nodes,
                                           int64_t* counts, void* workspace, size_t workspace_bytes,
                                           ofspmm_stream_t stream);
+
+/* ---- Link prediction: edge lookup and negative sampling on A (rows x cols, any shape unless
+ * stated).  Both need the columns of every row in ascending order (the project's CSR convention);
+ * on an unsorted row the result is unspecified but memory-safe.  Neither takes a workspace; both
+ * are CUDA-graph capturable.
+ *
+ * Edge lookup (DGL's g.edge_ids(u, v)): for i < n, eid[i] = crow[u] + lower_bound(col[crow[u] :
+ * crow[u+1]], v[i]) if that entry equals v[i] (the first of repeated columns), else -1; a u[i]
+ * outside [0, rows) gives -1.  u, v and eid have A's index dtype.
+ *
+ * Negative sampling (DGL's negative_sampler.Uniform with rejection): for source i, u = src[i], and
+ * draw t in [0, k), tries r = 0 .. max_trials-1 propose
+ *     c = mulhi64(mix(mix(s ^ i) + r*k + t), cols)        (s = rng_seed, mix as above)
+ * and the first proposal accepted goes to neg_dst[i*k + t] (A's index dtype), -1 if none is.  A
+ * proposal is rejected with OFSPMM_NEG_EXCLUDE_SELF when c == u, and with OFSPMM_NEG_EXCLUDE_EDGES
+ * when c is a column of row u (the lookup above).  The draws are keyed by the position i, not by the
+ * node: positive edges that share a source get different negatives.  A u outside [0, rows) gives k
+ * entries of -1.  counts (device int64[2]): [0] = slots holding -1 (those of invalid sources
+ * included), [1] = invalid sources.  OFSPMM_ERR_INVALID_ARG for k < 0, max_trials < 1, an unknown
+ * flag, and EXCLUDE_SELF with rows != cols. */
+enum { OFSPMM_NEG_EXCLUDE_EDGES = 1, OFSPMM_NEG_EXCLUDE_SELF = 2 };
+OFSPMM_API int ofspmm_edge_ids(const ofspmm_csr* A, const void* u, const void* v, int64_t n, void* eid,
+                               ofspmm_stream_t stream);
+OFSPMM_API int ofspmm_negative_sample(const ofspmm_csr* A, const void* src, int64_t num_src, int64_t k,
+                                      uint64_t rng_seed, uint32_t flags, int32_t max_trials, void* neg_dst,
+                                      int64_t* counts, ofspmm_stream_t stream);
 
 /* ---- Host-buffer convenience entry (what a CPU-tensor caller / the e2e benchmark uses): copies
  * the CSR arrays and B from HOST memory (pinned recommended) to device staging carved from

@@ -10,8 +10,8 @@ __version__ = "0.1.0"
 
 from . import graphs  # noqa: F401
 from ._lib import LIB_PATH, OfspmmError, OfspmmLibraryError, launch_count  # noqa: F401
-from .functional import SpmmOpKernelState, sddmm_csr, spmm_csr, spmm_csr_grad_b  # noqa: F401
-from .ops import (OpInferError, csr_transpose, merge_path_partition, merge_path_partition_host,  # noqa: F401
-                  row_blocks, row_hist, sample_neighbors)
-from .sampling import Block, sample_blocks  # noqa: F401
+from .functional import SpmmOpKernelState, edge_score, sddmm_csr, spmm_csr, spmm_csr_grad_b  # noqa: F401
+from .ops import (OpInferError, csr_transpose, edge_ids, merge_path_partition, merge_path_partition_host,  # noqa: F401
+                  negative_sample, row_blocks, row_hist, sample_neighbors)
+from .sampling import Block, LinkBatch, link_pairs, sample_blocks, sample_link_batch  # noqa: F401
 from . import formats  # noqa: E402,F401

@@ -30,7 +30,8 @@ EXPORTS = (
     "ofspmm_cast_from_f32", "ofspmm_coo_to_csr_workspace_bytes", "ofspmm_coo_to_csr", "ofspmm_csr_expand_rows",
     "ofspmm_csr_normalize", "ofspmm_signal_peers", "ofspmm_pull_rows_multi", "ofspmm_combine_rows_multi",
     "ofspmm_sample_neighbors_workspace_bytes", "ofspmm_sample_neighbors",
-    "ofspmm_sample_neighbors_ex_workspace_bytes", "ofspmm_sample_neighbors_ex",
+    "ofspmm_sample_neighbors_ex_workspace_bytes", "ofspmm_sample_neighbors_ex", "ofspmm_edge_ids",
+    "ofspmm_negative_sample",
 )
 
 # ofspmm_opts.flags / variant codes (include/ofspmm.h)
@@ -38,7 +39,9 @@ FWD_ACCUMULATE, FWD_BIAS, FWD_RELU, ORDER_DYNAMIC, ORDER_STATIC, FWD_ACC32_IN, F
 FWD_MEAN = 128
 VARIANT_AUTO, VARIANT_ITEMS64, VARIANT_ROWPAR, VARIANT_ROWS, VARIANT_EXPLICIT = 0, 1, 2, 4, 0x100
 # ofspmm_sample_opts.flags
-SAMPLE_REPLACE, SAMPLE_EDGE_IDS = 1, 2
+SAMPLE_REPLACE, SAMPLE_EDGE_IDS, SAMPLE_EXCLUDE = 1, 2, 8
+# ofspmm_negative_sample flags
+NEG_EXCLUDE_EDGES, NEG_EXCLUDE_SELF = 1, 2
 
 
 class OfspmmLibraryError(ImportError):
@@ -79,7 +82,8 @@ class OptsStruct(ctypes.Structure):
 
 class SampleOptsStruct(ctypes.Structure):
     """struct ofspmm_sample_opts (include/ofspmm.h)."""
-    _fields_ = [("flags", ctypes.c_uint32), ("prob_dtype", ctypes.c_int32), ("prob", ctypes.c_void_p)]
+    _fields_ = [("flags", ctypes.c_uint32), ("prob_dtype", ctypes.c_int32), ("prob", ctypes.c_void_p),
+                ("exclude", ctypes.c_void_p), ("num_exclude", ctypes.c_int64)]
 
 
 _LIB = None
@@ -190,6 +194,10 @@ def lib() -> ctypes.CDLL:
     L.ofspmm_sample_neighbors_ex.argtypes = [csr_p, sopts_p, vp, i64, i64, ctypes.c_uint64, i64, vp, vp, vp, vp, vp, vp,
                                              vp, sz, vp]
     L.ofspmm_sample_neighbors_ex.restype = i32
+    L.ofspmm_edge_ids.argtypes = [csr_p, vp, vp, i64, vp, vp]
+    L.ofspmm_edge_ids.restype = i32
+    L.ofspmm_negative_sample.argtypes = [csr_p, vp, i64, i64, ctypes.c_uint64, ctypes.c_uint32, ctypes.c_int32, vp, vp, vp]
+    L.ofspmm_negative_sample.restype = i32
     _LIB = L
     return L
 

@@ -113,11 +113,14 @@ int begin_bwd(const ofspmm_csr* A, const void* dY, void* dB, int64_t n, int dens
 }
 
 // Checks of the sampling options (NULL: none): known flags only; weights of a dense dtype, and not
-// with replacement.
+// with replacement; an exclusion list of a non-negative size, present unless empty.
 int check_sample_opts(const ofspmm_sample_opts* o) {
   if (o == nullptr) return OFSPMM_OK;
-  if (o->flags & ~static_cast<uint32_t>(OFSPMM_SAMPLE_REPLACE | OFSPMM_SAMPLE_EDGE_IDS)) return OFSPMM_ERR_INVALID_ARG;
+  if (o->flags & ~static_cast<uint32_t>(OFSPMM_SAMPLE_REPLACE | OFSPMM_SAMPLE_EDGE_IDS | OFSPMM_SAMPLE_EXCLUDE))
+    return OFSPMM_ERR_INVALID_ARG;
   if (o->prob != nullptr && ((o->flags & OFSPMM_SAMPLE_REPLACE) || !dense_ok(o->prob_dtype))) return OFSPMM_ERR_INVALID_ARG;
+  if ((o->flags & OFSPMM_SAMPLE_EXCLUDE) && (o->num_exclude < 0 || (o->num_exclude > 0 && o->exclude == nullptr)))
+    return OFSPMM_ERR_INVALID_ARG;
   return OFSPMM_OK;
 }
 bool sample_edge_ids(const ofspmm_sample_opts* o) { return o != nullptr && (o->flags & OFSPMM_SAMPLE_EDGE_IDS); }
@@ -507,6 +510,24 @@ int ofspmm_sample_neighbors_ex(const ofspmm_csr* A, const ofspmm_sample_opts* op
   return launch_sample_neighbors(A, opts, dst, num_dst, fanout, rng_seed, cap, blk_crow, blk_col, blk_val,
                                  eid ? blk_eid : nullptr, src_nodes, counts, workspace,
                                  reinterpret_cast<cudaStream_t>(stream));
+}
+
+int ofspmm_edge_ids(const ofspmm_csr* A, const void* u, const void* v, int64_t n, void* eid, ofspmm_stream_t stream) {
+  if (int rc = check_csr(A, false)) return rc;
+  if (n < 0 || (n > 0 && (u == nullptr || v == nullptr || eid == nullptr))) return OFSPMM_ERR_INVALID_ARG;
+  return launch_edge_ids(A, u, v, n, eid, reinterpret_cast<cudaStream_t>(stream));
+}
+
+int ofspmm_negative_sample(const ofspmm_csr* A, const void* src, int64_t num_src, int64_t k, uint64_t rng_seed,
+                           uint32_t flags, int32_t max_trials, void* neg_dst, int64_t* counts, ofspmm_stream_t stream) {
+  if (int rc = check_csr(A, false)) return rc;
+  if (num_src < 0 || k < 0 || max_trials < 1 || counts == nullptr) return OFSPMM_ERR_INVALID_ARG;
+  if (flags & ~static_cast<uint32_t>(OFSPMM_NEG_EXCLUDE_EDGES | OFSPMM_NEG_EXCLUDE_SELF)) return OFSPMM_ERR_INVALID_ARG;
+  if ((flags & OFSPMM_NEG_EXCLUDE_SELF) && A->rows != A->cols) return OFSPMM_ERR_INVALID_ARG;
+  if (k > 0 && num_src > INT64_MAX / k) return OFSPMM_ERR_TOO_LARGE;   // num_src * k slots must be addressable
+  if (num_src > 0 && (src == nullptr || (k > 0 && neg_dst == nullptr))) return OFSPMM_ERR_INVALID_ARG;
+  return launch_negative_sample(A, src, num_src, k, rng_seed, flags, max_trials, neg_dst, counts,
+                                reinterpret_cast<cudaStream_t>(stream));
 }
 
 int ofspmm_csr_expand_rows(const void* crow, int idx_dtype, int64_t rows, int64_t* row_of_nnz, ofspmm_stream_t stream) {

@@ -185,6 +185,10 @@ size_t sample_neighbors_workspace_bytes(int64_t num_dst, int64_t cap, bool edge_
 int launch_sample_neighbors(const ofspmm_csr* A, const ofspmm_sample_opts* opts, const void* dst, int64_t num_dst,
                             int64_t fanout, uint64_t seed, int64_t cap, void* blk_crow, void* blk_col, void* blk_val,
                             void* blk_eid, void* src_nodes, int64_t* counts, void* ws, cudaStream_t stream);
+int launch_edge_ids(const ofspmm_csr* A, const void* u, const void* v, int64_t n, void* eid, cudaStream_t stream);
+// flags: validated OFSPMM_NEG_* bits; counts: device int64[2], zeroed here.
+int launch_negative_sample(const ofspmm_csr* A, const void* src, int64_t num_src, int64_t k, uint64_t seed,
+                           uint32_t flags, int max_trials, void* neg_dst, int64_t* counts, cudaStream_t stream);
 int launch_expand_rows(const void* crow, int idx_dtype, int64_t rows, int64_t* out, cudaStream_t stream);
 int launch_csr_normalize(const void* crow, const void* col, float* val, int idx_dtype, int64_t rows, int64_t cols, int mode,
                          float* dinv, cudaStream_t stream);

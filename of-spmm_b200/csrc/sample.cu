@@ -4,6 +4,9 @@
 // ascending order).  Uniform: k = min(deg, fanout), key = x = mix(mix(seed ^ v) + j) (splitmix64);
 // weighted: k = min(npos, fanout), key = bits(neglog(U(x)) / w_j), all ones for an ineligible weight
 // (sample_key.h); with replacement: k = fanout independent draws j_t = mulhi(x(seed, v, t), deg).
+// Edge exclusion (OFSPMM_SAMPLE_EXCLUDE) makes the excluded positions ineligible: the count, npos,
+// select and draw kernels take the list as a trailing argument `ex...`, empty without the flag, so
+// that the kernels of the calls without it are unchanged.
 //   count   one thread per destination: validity (range, repeats found in the sorted ids), k, and a
 //           list of the rows long enough for a whole CTA;
 //   npos    weighted only: eligible entries per row, one warp per row (one CTA per long row);
@@ -21,6 +24,7 @@
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 
+#include "bsearch.cuh"
 #include "launch.cuh"
 #include "sample_key.h"
 
@@ -43,6 +47,7 @@ struct UniformKey {
   __device__ __forceinline__ unsigned long long operator()(long long j) const {
     return sk_mix64(h0 + static_cast<unsigned long long>(j));
   }
+  __device__ __forceinline__ bool excluded(long long) const { return false; }
 };
 
 // A weight widened exactly to fp64: fp32 bits, or bf16 bits (the high half of an fp32).
@@ -59,23 +64,85 @@ struct WeightedKey {
   __device__ __forceinline__ unsigned long long operator()(long long j) const {
     return sk_weighted_key(sk_mix64(h0 + static_cast<unsigned long long>(j)), widen(p[j]));
   }
+  __device__ __forceinline__ bool excluded(long long) const { return false; }
 };
+
+// OFSPMM_SAMPLE_EXCLUDE: `n` strictly ascending positions in A.
+template <typename IdxT>
+struct ExcludeList {
+  const IdxT* pos;
+  long long n;
+};
+
+// The excluded positions of one row: none without an exclusion list (every member folds away).
+struct NoExcludedRow {
+  __device__ __forceinline__ long long count() const { return 0; }
+  __device__ __forceinline__ bool has(long long) const { return false; }
+};
+
+// pos[0, cnt): the excluded positions inside the row [b, b + deg) of A, ascending.
+template <typename IdxT>
+struct ExcludedRow {
+  const IdxT* pos;
+  long long cnt, b, deg;
+  // Excluded entries of the row, at most deg (a list with repeats is not strictly ascending: the
+  // blocks are unspecified, but no row takes more than it has).
+  __device__ __forceinline__ long long count() const { return cnt < deg ? cnt : deg; }
+  // Position e of A is excluded: a search of a usually empty range.
+  __device__ __forceinline__ bool has(long long e) const {
+    const long long q = lower_bound(pos, cnt, static_cast<IdxT>(e));
+    return q < cnt && static_cast<long long>(pos[q]) == e;
+  }
+  // Offset in the row of its r-th eligible entry (ascending): r plus the excluded positions passed.
+  __device__ __forceinline__ long long position(long long r) const {
+    long long j = r;
+    for (long long q = 0; q < cnt && static_cast<long long>(pos[q]) <= b + j; ++q) ++j;
+    return j;
+  }
+};
+
+__device__ __forceinline__ NoExcludedRow excluded_row(long long, long long) { return {}; }
+
+template <typename IdxT>
+__device__ __forceinline__ ExcludedRow<IdxT> excluded_row(long long b, long long deg, const ExcludeList<IdxT>& ex) {
+  const long long lo = lower_bound(ex.pos, ex.n, static_cast<IdxT>(b));
+  const long long hi = lower_bound(ex.pos, ex.n, static_cast<IdxT>(b + deg));
+  return {ex.pos + lo, hi - lo, b, deg};
+}
+
+// A selection key whose excluded entries get the key all ones and no place in the tie rank.
+template <typename Key, typename IdxT>
+struct ExcludedKey {
+  Key key;
+  ExcludedRow<IdxT> row;
+  __device__ __forceinline__ unsigned long long operator()(long long j) const { return excluded(j) ? ~0ull : key(j); }
+  __device__ __forceinline__ bool excluded(long long j) const { return row.cnt != 0 && row.has(row.b + j); }
+};
+
+// Offset in the row of the draw x: mulhi(x, deg); with an exclusion list the mulhi(x, n_e)-th
+// eligible entry.
+__device__ __forceinline__ long long draw_offset(unsigned long long x, long long deg, const NoExcludedRow&) {
+  return static_cast<long long>(__umul64hi(x, static_cast<unsigned long long>(deg)));
+}
+
+template <typename IdxT>
+__device__ __forceinline__ long long draw_offset(unsigned long long x, long long deg, const ExcludedRow<IdxT>& row) {
+  return row.position(static_cast<long long>(__umul64hi(x, static_cast<unsigned long long>(deg - row.count()))));
+}
+
+template <typename Key>
+__device__ __forceinline__ Key with_exclusion(const Key& key, const NoExcludedRow&) { return key; }
+
+template <typename Key, typename IdxT>
+__device__ __forceinline__ ExcludedKey<Key, IdxT> with_exclusion(const Key& key, const ExcludedRow<IdxT>& row) {
+  return {key, row};
+}
 
 // Bits of a sort key that holds ids in [0, rows] (rows itself is the "no id" sentinel).
 int id_bits(long long rows) {
   int b = 1;
   while (b < 32 && (1ll << b) <= rows) ++b;
   return b;
-}
-
-template <typename T>
-__device__ __forceinline__ long long lower_bound(const T* a, long long n, T x) {
-  long long lo = 0, hi = n;
-  while (lo < hi) {
-    const long long mid = (lo + hi) >> 1;
-    if (a[mid] < x) lo = mid + 1; else hi = mid;
-  }
-  return lo;
 }
 
 // dkey[i] = dst[i] when it is a row of A, else the sentinel `rows`; didx[i] = i.
@@ -92,12 +159,13 @@ __global__ void sample_dst_keys_kernel(const IdxT* __restrict__ dst, long long n
 
 // kcnt[i] = k of destination i (0 for an invalid one: out of range, or an id that occurs more than
 // once); kcnt[num_dst] = 0 so that the exclusive scan ends in the total.  Weighted: k from deg is
-// only an upper bound, which sample_npos / sample_npos_long turn into min(npos, fanout).
-template <typename IdxT>
+// only an upper bound, which sample_npos / sample_npos_long turn into min(npos, fanout).  With an
+// exclusion list the row's excluded entries are not counted: k from n_e = deg - excluded.
+template <typename IdxT, typename... Ex>
 __global__ void sample_count_kernel(const IdxT* __restrict__ crow, const IdxT* __restrict__ dst, long long num_dst,
                                     long long rows, long long fanout, int mode, const unsigned* __restrict__ dkey_sorted,
                                     long long* __restrict__ kcnt, int* __restrict__ longs, unsigned* __restrict__ nlong,
-                                    long long* __restrict__ counts) {
+                                    long long* __restrict__ counts, Ex... ex) {
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i > num_dst) return;
   if (i == num_dst) { kcnt[i] = 0; return; }
@@ -111,10 +179,11 @@ __global__ void sample_count_kernel(const IdxT* __restrict__ crow, const IdxT* _
   long long k = 0;
   if (valid) {
     const long long deg = static_cast<long long>(crow[v + 1]) - static_cast<long long>(crow[v]);
+    const long long ne = deg - excluded_row(static_cast<long long>(crow[v]), deg, ex...).count();
     if (mode == kReplace) {
-      k = deg > 0 ? fanout : 0;   // fanout >= 0: draws need no selection, hence no long-row list
+      k = ne > 0 ? fanout : 0;   // fanout >= 0: draws need no selection, hence no long-row list
     } else {
-      k = fanout < 0 ? deg : (deg < fanout ? deg : fanout);
+      k = fanout < 0 ? ne : (ne < fanout ? ne : fanout);
       if (k > 0 && deg > kLongRow) longs[atomicAdd(nlong, 1u)] = static_cast<int>(i);
     }
   } else {
@@ -125,11 +194,11 @@ __global__ void sample_count_kernel(const IdxT* __restrict__ crow, const IdxT* _
 
 // Weighted: kcnt[i] = min(npos, fanout) (npos for fanout -1) of the listed long rows, one CTA per
 // row, as their selection runs.
-template <typename IdxT, typename PT>
+template <typename IdxT, typename PT, typename... Ex>
 __global__ void __launch_bounds__(kLongThreads)
 sample_npos_long_kernel(const IdxT* __restrict__ crow, const IdxT* __restrict__ dst, long long fanout,
                         const PT* __restrict__ prob, const int* __restrict__ longs, const unsigned* __restrict__ nlong,
-                        long long* __restrict__ kcnt) {
+                        long long* __restrict__ kcnt, Ex... ex) {
   __shared__ unsigned warp_cnt[kLongThreads / 32];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const unsigned n = *nlong;
@@ -137,8 +206,10 @@ sample_npos_long_kernel(const IdxT* __restrict__ crow, const IdxT* __restrict__ 
     const long long i = longs[r];
     const long long v = static_cast<long long>(dst[i]);
     const long long b = static_cast<long long>(crow[v]), deg = static_cast<long long>(crow[v + 1]) - b;
+    const auto xr = excluded_row(b, deg, ex...);
     unsigned c = 0;
-    for (long long j = threadIdx.x; j < deg; j += kLongThreads) c += sk_eligible(widen(prob[b + j])) ? 1u : 0u;
+    for (long long j = threadIdx.x; j < deg; j += kLongThreads)
+      c += sk_eligible(widen(prob[b + j])) && !xr.has(b + j) ? 1u : 0u;
     c = __reduce_add_sync(kFull, c);
     if (lane == 0) warp_cnt[warp] = c;
     __syncthreads();
@@ -154,10 +225,10 @@ sample_npos_long_kernel(const IdxT* __restrict__ crow, const IdxT* __restrict__ 
 
 // Weighted: kcnt[i] = min(npos, fanout) (npos for fanout -1), one warp per destination of at most
 // kLongRow entries; the longer ones are sample_npos_long's.
-template <typename IdxT, typename PT>
+template <typename IdxT, typename PT, typename... Ex>
 __global__ void __launch_bounds__(kSampleWarps * 32)
 sample_npos_kernel(const IdxT* __restrict__ crow, const IdxT* __restrict__ dst, long long num_dst, long long fanout,
-                   const PT* __restrict__ prob, long long* __restrict__ kcnt) {
+                   const PT* __restrict__ prob, long long* __restrict__ kcnt, Ex... ex) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const long long step = static_cast<long long>(gridDim.x) * kSampleWarps;
   for (long long i = static_cast<long long>(blockIdx.x) * kSampleWarps + warp; i < num_dst; i += step) {
@@ -165,8 +236,9 @@ sample_npos_kernel(const IdxT* __restrict__ crow, const IdxT* __restrict__ dst, 
     const long long v = static_cast<long long>(dst[i]);
     const long long b = static_cast<long long>(crow[v]), deg = static_cast<long long>(crow[v + 1]) - b;
     if (deg > kLongRow) continue;
+    const auto xr = excluded_row(b, deg, ex...);
     unsigned c = 0;
-    for (long long j = lane; j < deg; j += 32) c += sk_eligible(widen(prob[b + j])) ? 1u : 0u;
+    for (long long j = lane; j < deg; j += 32) c += sk_eligible(widen(prob[b + j])) && !xr.has(b + j) ? 1u : 0u;
     const long long npos = __reduce_add_sync(kFull, c);
     if (lane == 0) kcnt[i] = fanout >= 0 && npos > fanout ? fanout : npos;
   }
@@ -215,7 +287,8 @@ __device__ __forceinline__ long long group_prefix(int* slots, int warp, int lane
 
 // Samples row v (entries [b, b + deg) of A) into stage slots [off, off + k), in ascending j, by the
 // keys key(j).  Uniform over the group: every thread calls it with the same arguments except `tid`.
-// stage_eid (may be null) receives the positions b + j in A.
+// stage_eid (may be null) receives the positions b + j in A.  An entry key_of.excluded(j) is never
+// selected: k counts eligible entries only, its key is all ones, and it takes no place in the ties.
 template <int G, typename IdxT, typename VT, typename Key>
 __device__ void sample_row(RowShared<G>& sh, int tid, const IdxT* __restrict__ col, const VT* __restrict__ val,
                            long long b, long long deg, long long k, const Key& key_of, long long cols,
@@ -280,7 +353,7 @@ __device__ void sample_row(RowShared<G>& sh, int tid, const IdxT* __restrict__ c
     bool sel = in;
     if (!all) {
       const unsigned long long key = in ? key_of(j) : 0ull;
-      const bool eq = in && key == thr;
+      const bool eq = in && key == thr && !key_of.excluded(j);
       const unsigned eqm = __ballot_sync(kFull, eq);
       long long eq_rank = eq_before + __popc(eqm & lt_mask), eq_total = __popc(eqm);
       if constexpr (G > 32) eq_rank += group_prefix<G>(sh.warp_eq, warp, lane, __popc(eqm), &eq_total);
@@ -301,13 +374,13 @@ __device__ void sample_row(RowShared<G>& sh, int tid, const IdxT* __restrict__ c
   }
 }
 
-template <typename IdxT, typename VT, typename Key>
+template <typename IdxT, typename VT, typename Key, typename... Ex>
 __global__ void __launch_bounds__(kSampleWarps * 32)
 sample_rows_warp_kernel(const IdxT* __restrict__ crow, const IdxT* __restrict__ col, const VT* __restrict__ val,
                         long long cols, const IdxT* __restrict__ dst, long long num_dst,
                         const long long* __restrict__ slot, long long cap, unsigned long long seed,
                         const void* __restrict__ prob, unsigned* __restrict__ stage_col, VT* __restrict__ stage_val,
-                        long long* __restrict__ stage_eid) {
+                        long long* __restrict__ stage_eid, Ex... ex) {
   __shared__ RowShared<32> sh[kSampleWarps];
   if (slot[num_dst] > cap) return;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -318,18 +391,19 @@ sample_rows_warp_kernel(const IdxT* __restrict__ crow, const IdxT* __restrict__ 
     const long long v = static_cast<long long>(dst[i]);
     const long long b = static_cast<long long>(crow[v]), deg = static_cast<long long>(crow[v + 1]) - b;
     if (deg > kLongRow) continue;
-    sample_row<32>(sh[warp], lane, col, val, b, deg, k, Key(seed, v, b, prob), cols, off, stage_col, stage_val,
-                   stage_eid);
+    sample_row<32>(sh[warp], lane, col, val, b, deg, k, with_exclusion(Key(seed, v, b, prob), excluded_row(b, deg, ex...)),
+                   cols, off, stage_col, stage_val, stage_eid);
   }
 }
 
-template <typename IdxT, typename VT, typename Key>
+template <typename IdxT, typename VT, typename Key, typename... Ex>
 __global__ void __launch_bounds__(kLongThreads)
 sample_long_rows_kernel(const IdxT* __restrict__ crow, const IdxT* __restrict__ col, const VT* __restrict__ val,
                         long long cols, const IdxT* __restrict__ dst, long long num_dst,
                         const long long* __restrict__ slot, long long cap, unsigned long long seed,
                         const void* __restrict__ prob, const int* __restrict__ longs, const unsigned* __restrict__ nlong,
-                        unsigned* __restrict__ stage_col, VT* __restrict__ stage_val, long long* __restrict__ stage_eid) {
+                        unsigned* __restrict__ stage_col, VT* __restrict__ stage_val, long long* __restrict__ stage_eid,
+                        Ex... ex) {
   __shared__ RowShared<kLongThreads> sh;
   if (slot[num_dst] > cap) return;
   const unsigned n = *nlong;
@@ -339,19 +413,21 @@ sample_long_rows_kernel(const IdxT* __restrict__ crow, const IdxT* __restrict__ 
     if (k == 0) continue;   // weighted: no eligible entry
     const long long v = static_cast<long long>(dst[i]);
     const long long b = static_cast<long long>(crow[v]), deg = static_cast<long long>(crow[v + 1]) - b;
-    sample_row<kLongThreads>(sh, threadIdx.x, col, val, b, deg, k, Key(seed, v, b, prob), cols, off, stage_col,
+    sample_row<kLongThreads>(sh, threadIdx.x, col, val, b, deg, k,
+                             with_exclusion(Key(seed, v, b, prob), excluded_row(b, deg, ex...)), cols, off, stage_col,
                              stage_val, stage_eid);
   }
 }
 
 // With replacement: draw t of destination v takes position j_t = mulhi(x(seed, v, t), deg) into
-// slot off + t; one warp per destination, col / val read at the drawn positions only.
-template <typename IdxT, typename VT>
+// slot off + t; one warp per destination, col / val read at the drawn positions only.  With an
+// exclusion list: the r_t-th eligible position, r_t = mulhi(x(seed, v, t), n_e).
+template <typename IdxT, typename VT, typename... Ex>
 __global__ void __launch_bounds__(kSampleWarps * 32)
 sample_draw_kernel(const IdxT* __restrict__ crow, const IdxT* __restrict__ col, const VT* __restrict__ val,
                    long long cols, const IdxT* __restrict__ dst, long long num_dst, const long long* __restrict__ slot,
                    long long cap, unsigned long long seed, unsigned* __restrict__ stage_col,
-                   VT* __restrict__ stage_val, long long* __restrict__ stage_eid) {
+                   VT* __restrict__ stage_val, long long* __restrict__ stage_eid, Ex... ex) {
   if (slot[num_dst] > cap) return;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const long long step = static_cast<long long>(gridDim.x) * kSampleWarps;
@@ -361,8 +437,9 @@ sample_draw_kernel(const IdxT* __restrict__ crow, const IdxT* __restrict__ col, 
     const long long v = static_cast<long long>(dst[i]);
     const long long b = static_cast<long long>(crow[v]), deg = static_cast<long long>(crow[v + 1]) - b;
     const UniformKey x(seed, v, b, nullptr);
+    const auto xr = excluded_row(b, deg, ex...);
     for (long long t = lane; t < k; t += 32) {
-      const long long e = b + static_cast<long long>(__umul64hi(x(t), static_cast<unsigned long long>(deg)));
+      const long long e = b + draw_offset(x(t), deg, xr);
       const long long c = static_cast<long long>(col[e]);
       stage_col[off + t] = static_cast<unsigned>(c >= 0 && c < cols ? c : cols);
       if (val != nullptr) stage_val[off + t] = val[e];
@@ -475,17 +552,21 @@ SampleLayout sample_layout(int64_t num_dst, int64_t cap, bool edge_ids) {
   return L;
 }
 
-// The sampling mode of a call and its weights (validated options; NULL options: uniform).
+// The sampling mode of a call, its weights and its exclusion list (validated options; NULL
+// options: uniform, nothing excluded).
 struct SampleCall {
   int mode;
   const void* prob;
   int prob_dtype;
+  const void* exclude;
+  int64_t num_exclude;
 };
 
-template <typename IdxT, typename VT>
+// ex...: an ExcludeList<IdxT> for a call with a non-empty exclusion list, else nothing.
+template <typename IdxT, typename VT, typename... Ex>
 int sample_impl(const ofspmm_csr* A, const SampleCall& m, const void* dst_v, int64_t num_dst, int64_t fanout,
                 uint64_t seed, int64_t cap, void* blk_crow, void* blk_col, void* blk_val, void* blk_eid,
-                void* src_nodes, int64_t* counts, void* ws, cudaStream_t stream) {
+                void* src_nodes, int64_t* counts, void* ws, cudaStream_t stream, Ex... ex) {
   const SampleLayout L = sample_layout(num_dst, cap, blk_eid != nullptr);
   unsigned char* w = static_cast<unsigned char*>(ws);
   unsigned* nlong = reinterpret_cast<unsigned*>(w + L.hdr);
@@ -527,8 +608,8 @@ int sample_impl(const ofspmm_csr* A, const SampleCall& m, const void* dst_v, int
                                                    bits, stream));
     count_launch(4);
   }
-  sample_count_kernel<IdxT><<<static_cast<unsigned>((num_dst + 1 + 255) / 256), 256, 0, stream>>>(
-      crow, dst, num_dst, rows, fanout, m.mode, dkey, kcnt, longs, nlong, reinterpret_cast<long long*>(counts));
+  sample_count_kernel<IdxT, Ex...><<<static_cast<unsigned>((num_dst + 1 + 255) / 256), 256, 0, stream>>>(
+      crow, dst, num_dst, rows, fanout, m.mode, dkey, kcnt, longs, nlong, reinterpret_cast<long long*>(counts), ex...);
   count_launch();
   // f(Tag<PT>{}) for the weights' bit type: fp32 or bf16 words
   auto by_prob = [&](auto&& f) { m.prob_dtype == OFSPMM_DTYPE_FLOAT ? f(Tag<uint32_t>{}) : f(Tag<uint16_t>{}); };
@@ -537,19 +618,21 @@ int sample_impl(const ofspmm_csr* A, const SampleCall& m, const void* dst_v, int
       using PT = typename decltype(pt)::type;
       const PT* prob = static_cast<const PT*>(m.prob);
       const long long lgrid = num_dst < dev.sms * 2 ? num_dst : dev.sms * 2;
-      sample_npos_long_kernel<IdxT, PT><<<static_cast<unsigned>(lgrid), kLongThreads, 0, stream>>>(
-          crow, dst, fanout, prob, longs, nlong, kcnt);
-      sample_npos_kernel<IdxT, PT><<<wgrid, kSampleWarps * 32, 0, stream>>>(crow, dst, num_dst, fanout, prob, kcnt);
+      sample_npos_long_kernel<IdxT, PT, Ex...><<<static_cast<unsigned>(lgrid), kLongThreads, 0, stream>>>(
+          crow, dst, fanout, prob, longs, nlong, kcnt, ex...);
+      sample_npos_kernel<IdxT, PT, Ex...><<<wgrid, kSampleWarps * 32, 0, stream>>>(crow, dst, num_dst, fanout, prob, kcnt,
+                                                                           ex...);
       count_launch(2);
     });
   }
   auto select = [&](auto key) {
     using Key = typename decltype(key)::type;
-    sample_rows_warp_kernel<IdxT, VT, Key><<<wgrid, kSampleWarps * 32, 0, stream>>>(
-        crow, col, val, A->cols, dst, num_dst, slot, cap, seed, m.prob, stage_col, stage_val, stage_eid);
+    sample_rows_warp_kernel<IdxT, VT, Key, Ex...><<<wgrid, kSampleWarps * 32, 0, stream>>>(
+        crow, col, val, A->cols, dst, num_dst, slot, cap, seed, m.prob, stage_col, stage_val, stage_eid, ex...);
     const long long lgrid = num_dst < dev.sms * 2 ? num_dst : dev.sms * 2;
-    sample_long_rows_kernel<IdxT, VT, Key><<<static_cast<unsigned>(lgrid), kLongThreads, 0, stream>>>(
-        crow, col, val, A->cols, dst, num_dst, slot, cap, seed, m.prob, longs, nlong, stage_col, stage_val, stage_eid);
+    sample_long_rows_kernel<IdxT, VT, Key, Ex...><<<static_cast<unsigned>(lgrid), kLongThreads, 0, stream>>>(
+        crow, col, val, A->cols, dst, num_dst, slot, cap, seed, m.prob, longs, nlong, stage_col, stage_val, stage_eid,
+        ex...);
     count_launch(2);
   };
   cub_bytes = L.cub_bytes;
@@ -562,8 +645,8 @@ int sample_impl(const ofspmm_csr* A, const SampleCall& m, const void* dst_v, int
   }
   if (num_dst > 0) {
     if (m.mode == kReplace) {
-      sample_draw_kernel<IdxT, VT><<<wgrid, kSampleWarps * 32, 0, stream>>>(
-          crow, col, val, A->cols, dst, num_dst, slot, cap, seed, stage_col, stage_val, stage_eid);
+      sample_draw_kernel<IdxT, VT, Ex...><<<wgrid, kSampleWarps * 32, 0, stream>>>(
+          crow, col, val, A->cols, dst, num_dst, slot, cap, seed, stage_col, stage_val, stage_eid, ex...);
       count_launch();
     } else if (m.mode == kWeighted) {
       by_prob([&](auto pt) { select(Tag<WeightedKey<typename decltype(pt)::type>>{}); });
@@ -599,20 +682,30 @@ size_t sample_neighbors_workspace_bytes(int64_t num_dst, int64_t cap, bool edge_
 int launch_sample_neighbors(const ofspmm_csr* A, const ofspmm_sample_opts* opts, const void* dst, int64_t num_dst,
                             int64_t fanout, uint64_t seed, int64_t cap, void* blk_crow, void* blk_col, void* blk_val,
                             void* blk_eid, void* src_nodes, int64_t* counts, void* ws, cudaStream_t stream) {
-  SampleCall m{kUniform, nullptr, 0};
-  if (opts != nullptr && opts->prob != nullptr) m = {kWeighted, opts->prob, opts->prob_dtype};
+  SampleCall m{kUniform, nullptr, 0, nullptr, 0};
+  if (opts != nullptr && opts->prob != nullptr) m = {kWeighted, opts->prob, opts->prob_dtype, nullptr, 0};
   // fanout -1 with replacement is every entry once: the same block as without replacement
   else if (opts != nullptr && (opts->flags & OFSPMM_SAMPLE_REPLACE) && fanout >= 0) m.mode = kReplace;
+  if (opts != nullptr && (opts->flags & OFSPMM_SAMPLE_EXCLUDE)) {
+    m.exclude = opts->exclude;
+    m.num_exclude = opts->num_exclude;
+  }
   return dispatch_idx(A->idx_dtype, [&](auto idx) {
     using IdxT = typename decltype(idx)::type;
+    // an empty exclusion list is the call without one: the same kernels
+    auto run = [&](auto vt, void* bval, auto... ex) {
+      return sample_impl<IdxT, typename decltype(vt)::type>(A, m, dst, num_dst, fanout, seed, cap, blk_crow, blk_col,
+                                                            bval, blk_eid, src_nodes, counts, ws, stream, ex...);
+    };
+    auto run_ex = [&](auto vt, void* bval) {
+      return m.num_exclude > 0 ? run(vt, bval, ExcludeList<IdxT>{static_cast<const IdxT*>(m.exclude), m.num_exclude})
+                               : run(vt, bval);
+    };
     // values are copied bit for bit: fp32 as 32-bit, bf16 as 16-bit words; a pattern matrix has none
-    if (A->val_dtype == OFSPMM_VAL_UNIT)
-      return sample_impl<IdxT, uint8_t>(A, m, dst, num_dst, fanout, seed, cap, blk_crow, blk_col, nullptr, blk_eid,
-                                        src_nodes, counts, ws, stream);
+    if (A->val_dtype == OFSPMM_VAL_UNIT) return run_ex(Tag<uint8_t>{}, nullptr);
     return dispatch_dense(A->val_dtype, [&](auto vt) {
       using VT = std::conditional_t<sizeof(typename decltype(vt)::type) == 4, uint32_t, uint16_t>;
-      return sample_impl<IdxT, VT>(A, m, dst, num_dst, fanout, seed, cap, blk_crow, blk_col, blk_val, blk_eid,
-                                   src_nodes, counts, ws, stream);
+      return run_ex(Tag<VT>{}, blk_val);
     });
   });
 }

@@ -199,3 +199,49 @@ def spmm_csr_bias_act(a_crow: torch.Tensor, a_col: torch.Tensor, a_val: Optional
     if bias is not None and (bias.dim() != 1 or bias.shape[0] != b.shape[1] or bias.dtype != b.dtype):
         raise ops.OpInferError(f"bias must be a 1-D tensor of {b.shape[1]} elements of dtype {b.dtype}")
     return _SpmmCsrEpilogueFn.apply(a_crow, a_col, a_val, b, bias, a_rows, a_cols, bool(relu), state, kernels, reduce)
+
+
+# ---------------------------------------------------------------------------------------------
+# link prediction: dot-product scores of node pairs
+
+class _EdgeScoreFn(torch.autograd.Function):
+    """score[p] = <h_row[row(p)], h_col[col[p]]> over the entries p of the pair matrix S (the SDDMM);
+    backward: d h_row = S·h_col and d h_col = Sᵀ·h_row with the values dscore (the forward SpMM and
+    Aᵀ·dY)."""
+
+    @staticmethod
+    def forward(ctx, p_crow, p_col, h_row, h_col, rows, cols, kernels):
+        score = kernels.sddmm(p_crow, p_col, h_row.detach(), h_col.detach(), rows, cols, h_row.dtype, None)
+        ctx.need = (h_row.requires_grad, h_col.requires_grad)
+        ctx.rows, ctx.cols, ctx.kernels = rows, cols, kernels
+        ctx.save_for_backward(p_crow, p_col, h_row if ctx.need[1] else None, h_col if ctx.need[0] else None)
+        ctx.mark_non_differentiable(p_crow, p_col)
+        return score
+
+    @staticmethod
+    def backward(ctx, dscore):
+        p_crow, p_col, h_row, h_col = ctx.saved_tensors
+        dscore = dscore.contiguous()
+        d_row = d_col = None
+        if ctx.need[0]:
+            d_row = ctx.kernels.fwd(p_crow, p_col, dscore, _detach(h_col), ctx.rows, ctx.cols, None, False, None)
+        if ctx.need[1]:
+            d_col = ctx.kernels.grad_b(p_crow, p_col, dscore, _detach(h_row).contiguous(), ctx.rows, ctx.cols, None)
+        return None, None, d_row, d_col, None, None, None
+
+
+def edge_score(p_crow: torch.Tensor, p_col: torch.Tensor, h_row: torch.Tensor, h_col: torch.Tensor, rows: int,
+               cols: int, kernels=None) -> torch.Tensor:
+    """Dot-product scores of node pairs: ``score[p] = <h_row[i], h_col[p_col[p]]>`` for every entry p
+    of row i of the ``rows x cols`` pattern CSR (p_crow, p_col), e.g. ``LinkBatch.pair``.  fp32 or
+    bf16 (the score has ``h``'s dtype); differentiable wrt ``h_row`` and ``h_col``.  Repeated pairs
+    each get their score and their gradient share."""
+    kernels = kernels or OpsKernels()
+    if h_row.dim() != 2 or h_col.dim() != 2 or h_row.shape[1] != h_col.shape[1] or h_row.dtype != h_col.dtype:
+        raise ops.OpInferError("h_row and h_col must be 2-D with one width and one dtype")
+    if h_row.shape[0] != rows:
+        raise ops.OpInferError(f"h_row has {h_row.shape[0]} rows, the pair matrix {rows}")
+    if isinstance(kernels, OpsKernels):
+        ops._check_device(p_crow, p_col, h_row, h_col)
+        ops.infer_spmm_csr(p_crow, p_col, None, h_col, rows, cols)
+    return _EdgeScoreFn.apply(p_crow, p_col, h_row.contiguous(), h_col.contiguous(), rows, cols, kernels)

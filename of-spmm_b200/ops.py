@@ -486,7 +486,7 @@ def csr_transpose(a_crow, a_col, a_val, a_rows: int, a_cols: int, want_perm: boo
 
 def sample_neighbors(a_crow, a_col, a_val, a_rows: int, a_cols: int, dst: torch.Tensor, fanout: int,
                      rng_seed: int, *, prob: Optional[torch.Tensor] = None, replace: bool = False,
-                     return_eid: bool = False):
+                     return_eid: bool = False, exclude_eid: Optional[torch.Tensor] = None):
     """One fan-out-sampled bipartite block of the square CSR A (``ofspmm_sample_neighbors_ex``): for
     each destination ``dst[i]``, at most ``fanout`` of its entries (all of them for -1), chosen by
     the keys of include/ofspmm.h — uniform without replacement, a pure function of
@@ -500,12 +500,16 @@ def sample_neighbors(a_crow, a_col, a_val, a_rows: int, a_cols: int, dst: torch.
     entries whose weight is not positive and finite are never picked.  ``replace=True``: exactly
     ``fanout`` uniform draws per non-empty row, in draw order, repeats kept (multi-edges); not with
     ``prob``.  ``return_eid=True`` appends ``eid``, the position in A (A's index dtype) of every
-    block entry: ``a_col[eid] == src_nodes[blk_col]`` and ``a_val[eid] == blk_val``."""
+    block entry: ``a_col[eid] == src_nodes[blk_col]`` and ``a_val[eid] == blk_val``.
+
+    ``exclude_eid``: positions in A (any order, repeats allowed) that no block entry may be, e.g. the
+    edges a link-prediction batch predicts; the other entries are sampled as without it, and a row
+    without an excluded entry exactly so."""
     if prob is not None:
         _chk(not replace, "weighted sampling with replacement is not supported (prob with replace=True)")
         _chk(prob.dim() == 1 and prob.numel() == a_col.numel() and prob.dtype in _DENSE,
              "prob must hold nnz float32 / bfloat16 weights")
-    _check_device(a_crow, a_col, a_val, dst, prob)
+    _check_device(a_crow, a_col, a_val, dst, prob, exclude_eid)
     _chk(a_crow.dim() == 1 and a_col.dim() == 1 and dst.dim() == 1, "a_crow, a_col and dst must be 1-D")
     _chk(a_crow.dtype in _INDEX and a_col.dtype == a_crow.dtype, "a_crow / a_col must share an index dtype (int32/int64)")
     _chk(a_rows == a_cols, f"neighbour sampling needs a square matrix, got {a_rows} x {a_cols}")
@@ -535,7 +539,12 @@ def sample_neighbors(a_crow, a_col, a_val, a_rows: int, a_cols: int, dst: torch.
     src_nodes = torch.empty(num_dst + cap, dtype=idt, device=dev)
     counts = torch.empty(3, dtype=torch.int64, device=dev)
     flags = (_lib.SAMPLE_REPLACE if replace else 0) | (_lib.SAMPLE_EDGE_IDS if return_eid else 0)
-    sopts = _lib.SampleOptsStruct(flags, _DENSE[prob.dtype] if prob is not None else 0, _ptr(prob))
+    if exclude_eid is not None:
+        _chk(exclude_eid.dim() == 1 and not exclude_eid.is_floating_point(), "exclude_eid must be a 1-D tensor of edge ids")
+        exclude_eid = torch.unique(exclude_eid.to(idt))   # sorted, distinct: the strictly ascending list
+        flags |= _lib.SAMPLE_EXCLUDE
+    sopts = _lib.SampleOptsStruct(flags, _DENSE[prob.dtype] if prob is not None else 0, _ptr(prob),
+                                  _ptr(exclude_eid), int(exclude_eid.numel()) if exclude_eid is not None else 0)
     opts = ctypes.byref(sopts) if flags or prob is not None else None
     L = _lib.lib()
     with torch.cuda.device(dev):
@@ -550,6 +559,57 @@ def sample_neighbors(a_crow, a_col, a_val, a_rows: int, a_cols: int, dst: torch.
     _chk(bad == 0, f"sample_neighbors: {bad} destination ids are out of range [0, {a_rows}) or repeated")
     out = (blk_crow, blk_col[:nnz_blk], blk_val[:nnz_blk] if blk_val is not None else None, src_nodes[:num_src])
     return out + (blk_eid[:nnz_blk],) if return_eid else out
+
+
+def _check_link_args(a_crow, a_col, a_rows: int, a_cols: int, *ids) -> None:
+    _check_device(a_crow, a_col, *ids)
+    _chk(a_crow.dim() == 1 and a_col.dim() == 1, "a_crow and a_col must be 1-D")
+    _chk(a_crow.dtype in _INDEX and a_col.dtype == a_crow.dtype, "a_crow / a_col must share an index dtype (int32/int64)")
+    _chk(a_rows >= 0 and a_cols >= 0 and a_crow.numel() == a_rows + 1, f"a_crow must have a_rows+1 = {a_rows + 1} entries")
+    for t in ids:
+        _chk(t.dim() == 1 and not t.is_floating_point() and not t.is_complex(), f"node ids must be 1-D integers, got {t.dtype}")
+
+
+def edge_ids(a_crow, a_col, a_rows: int, a_cols: int, u: torch.Tensor, v: torch.Tensor) -> torch.Tensor:
+    """Position in A of the entry (u[i], v[i]) (``ofspmm_edge_ids``; DGL's ``g.edge_ids(u, v)``), -1
+    where A has no such entry or u[i] is out of range.  Columns must ascend within each row (the
+    first of repeated columns is found).  Returns A's index dtype; no host synchronisation."""
+    _check_link_args(a_crow, a_col, a_rows, a_cols, u, v)
+    _chk(u.numel() == v.numel(), "u and v must have one entry per pair")
+    dev, idt = a_crow.device, a_crow.dtype
+    u, v = u.to(idt).contiguous(), v.to(idt).contiguous()
+    eid = torch.empty(u.numel(), dtype=idt, device=dev)
+    with torch.cuda.device(dev):
+        A = _csr_struct(a_crow, a_col, None, a_rows, a_cols)
+        check(_lib.lib().ofspmm_edge_ids(ctypes.byref(A), _ptr(u), _ptr(v), u.numel(), _ptr(eid), _stream_ptr(eid)),
+              "edge_ids")
+    return eid
+
+
+def negative_sample(a_crow, a_col, a_rows: int, a_cols: int, src: torch.Tensor, k: int, rng_seed: int, *,
+                    exclude_edges: bool = True, exclude_self: bool = True, max_trials: int = 8):
+    """``k`` corrupted destinations per source (``ofspmm_negative_sample``; DGL's
+    ``negative_sampler.Uniform`` with rejection): column c uniform over [0, a_cols), redrawn up to
+    ``max_trials`` times while (src[i], c) is an entry of A (``exclude_edges``) or c == src[i]
+    (``exclude_self``, square A only).  Draws are keyed by the position i, so repeated sources get
+    different negatives.  Returns ``(neg, counts)``: neg (len(src) x k, A's index dtype) with -1 for
+    a draw whose every trial was rejected (and for an out-of-range source), and the device int64
+    ``counts`` = [-1 slots, invalid sources]; no host synchronisation."""
+    _check_link_args(a_crow, a_col, a_rows, a_cols, src)
+    _chk(k >= 0, f"k must be >= 0, got {k}")
+    _chk(max_trials >= 1, f"max_trials must be >= 1, got {max_trials}")
+    _chk(not exclude_self or a_rows == a_cols, "exclude_self needs a square matrix")
+    dev, idt = a_crow.device, a_crow.dtype
+    src = src.to(idt).contiguous()
+    neg = torch.empty((src.numel(), k), dtype=idt, device=dev)
+    counts = torch.empty(2, dtype=torch.int64, device=dev)
+    flags = (_lib.NEG_EXCLUDE_EDGES if exclude_edges else 0) | (_lib.NEG_EXCLUDE_SELF if exclude_self else 0)
+    with torch.cuda.device(dev):
+        A = _csr_struct(a_crow, a_col, None, a_rows, a_cols)
+        check(_lib.lib().ofspmm_negative_sample(ctypes.byref(A), _ptr(src), src.numel(), k, rng_seed & (2 ** 64 - 1),
+                                                flags, max_trials, _ptr(neg), counts.data_ptr(), _stream_ptr(counts)),
+              "negative_sample")
+    return neg, counts
 
 
 def spmm_csr_grad_b_transient_compute(a_crow, a_col, a_val, dy, a_rows: int, a_cols: int,

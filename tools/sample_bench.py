@@ -99,10 +99,11 @@ def _device_info():
 
 
 class AbiCall:
-    """One preallocated ofspmm_sample_neighbors call (what the kernel timing launches)."""
+    """One preallocated ofspmm_sample_neighbors call (what the kernel timing launches); ``exclude``:
+    a sorted, distinct list of positions in A (OFSPMM_SAMPLE_EXCLUDE)."""
 
-    def __init__(self, A, dst, fanout, seed, prob=None, replace=False, edge_ids=False):
-        self.keep = (A, dst, prob)
+    def __init__(self, A, dst, fanout, seed, prob=None, replace=False, edge_ids=False, exclude=None):
+        self.keep = (A, dst, prob, exclude)
         self.A = ops._csr_struct(A.crow, A.col, A.val, A.rows, A.cols)
         n = dst.numel()
         cap = n * fanout if replace else min(n * fanout, A.nnz)
@@ -112,10 +113,13 @@ class AbiCall:
                      torch.empty(n + cap, dtype=A.crow.dtype, device=DEV), torch.empty(3, dtype=torch.int64, device=DEV),
                      torch.empty(cap, dtype=A.crow.dtype, device=DEV) if edge_ids else None]
         L = _lib.lib()
-        self.plain = prob is None and not replace and not edge_ids
-        flags = (_lib.SAMPLE_REPLACE if replace else 0) | (_lib.SAMPLE_EDGE_IDS if edge_ids else 0)
+        self.plain = prob is None and not replace and not edge_ids and exclude is None
+        flags = (_lib.SAMPLE_REPLACE if replace else 0) | (_lib.SAMPLE_EDGE_IDS if edge_ids else 0) | \
+                (_lib.SAMPLE_EXCLUDE if exclude is not None else 0)
         self.sopts = _lib.SampleOptsStruct(flags, ops._DENSE[prob.dtype] if prob is not None else 0,
-                                           None if prob is None else prob.data_ptr())
+                                           None if prob is None else prob.data_ptr(),
+                                           None if exclude is None else exclude.data_ptr(),
+                                           0 if exclude is None else exclude.numel())
         if self.plain:
             self.ws_bytes = L.ofspmm_sample_neighbors_workspace_bytes(n, cap, ops._INDEX[A.crow.dtype])
         else:

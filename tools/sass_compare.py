@@ -2,7 +2,9 @@
 addresses and immediates masked) and ptxas registers / spills (the *.ptxas.log files the Makefile
 writes next to the objects).  Kernels are matched by demangled name; a template argument a later
 build added is removed before matching (the partition entry type `int2` of the narrow kernels, the
-key type of the transpose kernels).
+key type of the transpose kernels), and `> >` is matched with `>>` (c++filt closes a nested template
+argument without the space when an empty trailing parameter pack follows it, as in the sampling
+kernels' exclusion pack).
 
     python tools/sass_compare.py OLD_LIB NEW_LIB [--old-build DIR --new-build DIR]
 """
@@ -49,6 +51,7 @@ def demangle(names):
 
 
 def norm(d):
+    d = d.replace("> >", ">>")
     d = d.replace(", int2>", ">").replace(", int2,", ",").replace("ofspmm::PartOf<int2>::Nz", "int")
     if "transpose_" in d:
         for a, b in (("<int, int>", "<int>"), ("<int, int, ", "<int, "), ("<long, long>", "<long>"),
